@@ -32,6 +32,7 @@ N_COUPLES, RATE, ITERS, EBN0_DB = 212, '1/3', 8, 2.0
 ACS_PER_FRAME = 320 * N_COUPLES * 2 * ITERS          # SURVEY §8(d): 1 085 440
 NOMINAL_ACS_PER_CLK_SM = 64.0                        # 1 FADD + 1 FMNMX per ACS at 128 issue slots/clk/SM
 METRIC = "turbo_info_throughput_N212_R1/3_8it"
+LLR_SEED = 20261018                                  # Philox seed of the headline frames (rank r: frames r*B ...)
 WORKLOAD = "DVB-RCS2 rate-1/3 turbo, N=212 couples, BPSK AWGN Eb/N0=2 dB, max-log-MAP 8 iterations (BASELINE configs[1])"
 
 
@@ -208,6 +209,25 @@ def run_reference(args, rank, world):
     print(json.dumps(line), file=_OUT, flush=True)
 
 
+DUMP_FRAMES = 16384            # 16384 frames x 424 bits as float32 = 27.8 MB: a dump stays small enough to keep and diff
+
+
+def dump_outputs(out_dir, bits, counters):
+    """--dump-outputs: what the headline decode handed its caller after the last timed step, for comparing two builds
+    output for output.  bits.npy: the int32 hard decisions of a fixed, seeded sample of frames (all frames when
+    there are at most DUMP_FRAMES), as float32 0/1 [S, 2N]; frame_index.npy: their rows in the batch (float64);
+    counters.npy: the in-kernel counters (bit errors, frame errors, frames, bits; float64), accumulated over the
+    timed steps as the caller's counter tensor holds them."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    B = bits.shape[0]
+    idx = np.sort(np.random.RandomState(0).choice(B, min(B, DUMP_FRAMES), replace=False))
+    sample = bits.index_select(0, torch.from_numpy(idx).to(bits.device)).cpu().numpy()
+    np.save(os.path.join(out_dir, "bits.npy"), sample.astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "counters.npy"), np.asarray(counters, np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------
 def run_ours(args, rank, world, local_rank):
     import torch
@@ -230,7 +250,7 @@ def run_ours(args, rank, world, local_rank):
     info = torch.empty((B, codec.k_info), dtype=torch.uint8, device=dev)
     coded = torch.empty((B, h.n_llr), dtype=torch.uint8, device=dev)
     llr = torch.empty((B, h.n_llr), dtype=torch.float32, device=dev)
-    h.mc_generate_bpsk(B, nv, 20261018, rank * B, info, coded, llr)
+    h.mc_generate_bpsk(B, nv, LLR_SEED, rank * B, info, coded, llr)
     del coded
     bits = torch.empty((B, codec.k_info), dtype=torch.int32, device=dev)
     counters = torch.zeros(4, dtype=torch.int64, device=dev)
@@ -291,6 +311,8 @@ def run_ours(args, rank, world, local_rank):
     frames_per_s = world * B / (ms_per_step * 1e-3)
     gbps = frames_per_s * codec.k_info / 1e9
     cnt = counters.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bits, cnt)
 
     # ---- roofline of the dominant kernel (tpf_kernel, the thread-per-frame decoder; one launch per step) ----
     sms = torch.cuda.get_device_properties(dev).multi_processor_count
@@ -619,7 +641,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=1_000_000, help="frames per GPU per step")
     ap.add_argument("--e2e-frames", type=int, default=262144, dest="e2e_frames")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy "
+                         "(bits.npy, frame_index.npy; counters.npy sums all --steps timed steps, so compare dumps "
+                         "taken with the same arguments)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.frames = max(16, (args.frames // 16) * 16)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,11 +1,14 @@
 """The reference's own scripts, UNMODIFIED, against the drop-in module (SURVEY 8(f) N3).
 
-`/root/reference/d_test.py` and `turbo_test_suite.py` import `dvb_rcs2_turbo` (names `DVB_RCS2_TurboCodec`,
+The reference's `d_test.py` and `turbo_test_suite.py` import `dvb_rcs2_turbo` (names `DVB_RCS2_TurboCodec`,
 `bcjr_decode`) and walk the facade: `.encode/.decode`, `.interleaver.{perm,inv_perm,N,interleave}`,
 `.encoder1/2.encode`, `.decoder1/2.decode`, `.k_info/.n_coded/.N/.code_rate`.  Here `sys.modules
 ['dvb_rcs2_turbo']` is pointed at `modulations_b200.dvb_rcs2_turbo` and the scripts' `main()` is run.
 
-This container has no GPU and the GPU box has no `/root/reference`, so the test exercises the HOST side of
+The scripts are not part of this repository: those two tests run when $REFERENCE_DIR (by default the same directory
+as oracle/make_golden.py's) holds a checkout of the reference project and skip otherwise.  The calls the scripts make
+on the drop-in are replayed by `test_facade_calls_of_the_scripts`, which runs everywhere.  No GPU is needed: the
+tests exercise the HOST side of
 the drop-in (names, argument handling, shapes, dtypes, the facade objects): the one class through which
 the package reaches the device (`_CodecHandle`) is replaced by a stand-in that answers with the C oracle.
 That stand-in lives here, in tests/; nothing under modulations_b200/ knows about it.  The device side of
@@ -20,9 +23,10 @@ import types
 import numpy as np
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "d_test.py")),
-                                reason="the reference tree is only present in the authoring container")
+REF = os.environ.get("REFERENCE_DIR", "/root/reference")
+needs_scripts = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "d_test.py")),
+                                   reason="the reference's scripts are not part of this repository: set $REFERENCE_DIR "
+                                          "to a checkout of the reference project")
 
 
 class _OracleHandle:
@@ -106,6 +110,7 @@ def _load(name):
     return mod
 
 
+@needs_scripts
 def test_d_test_runs_unmodified(dropin, capsys):
     mod = _load("d_test")
     assert mod.bcjr_decode is dropin.bcjr_decode
@@ -114,6 +119,7 @@ def test_d_test_runs_unmodified(dropin, capsys):
     assert "DEBUG COMPLETE" in out and "TURBO ITERATION ANALYSIS" in out
 
 
+@needs_scripts
 def test_turbo_test_suite_runs_unmodified(dropin, monkeypatch, capsys):
     mod = _load("turbo_test_suite")
     # setup(): rate 1 = '1/3', block 48, 3 blocks, SNR 0..1 dB step 1 (a negative start makes the reference's own
@@ -125,3 +131,35 @@ def test_turbo_test_suite_runs_unmodified(dropin, monkeypatch, capsys):
     out = capsys.readouterr().out
     assert "Test completed" in out
     assert tester.codec.k_info == 96 and tester.codec.n_coded == 288 and abs(tester.codec.code_rate - 1 / 3) < 1e-12
+
+
+def test_facade_calls_of_the_scripts(dropin):
+    """The calls d_test.py and turbo_test_suite.py make on the drop-in (the two names they import, the facade's
+    attributes, encode / decode, the interleaver, both constituent encoders and SISO decoders; INTEGRATION.md), at the
+    scripts' own configuration (N=48, rate 1/3, 2 iterations), each checked against the C oracle."""
+    from oracle import oracle
+    from tests import vectors
+    N = 48
+    c = dropin.DVB_RCS2_TurboCodec(block_length=N, code_rate='1/3', n_iterations=2)
+    assert (c.k_info, c.n_coded, c.N, c.interleaver.N) == (96, 288, N, N) and abs(c.code_rate - 1 / 3) < 1e-12
+    o = oracle.OracleTurbo(N, '1/3', 2, perm=c.interleaver.perm, inv_perm=c.interleaver.inv_perm)
+    rs = np.random.RandomState(5)
+    info = rs.randint(0, 2, c.k_info)
+    coded = c.encode(info)
+    assert np.array_equal(coded, o.encode(info))
+    A, B = info[0::2], info[1::2]
+    Ai, Bi = c.interleaver.interleave(A, B)
+    assert np.array_equal(Ai, A[o.perm]) and np.array_equal(Bi, B[o.perm])
+    full = np.asarray(coded).reshape(N, 6)                  # rate 1/3: A, B, W1, Y1, W2, Y2 per couple
+    for enc, a, b, cols in ((c.encoder1, A, B, (2, 3)), (c.encoder2, Ai, Bi, (4, 5))):
+        W, Y = enc.encode(a, b)
+        assert np.array_equal(W, full[:, cols[0]]) and np.array_equal(Y, full[:, cols[1]])
+    llr = vectors.awgn_llr(rs, np.asarray(coded), '1/3', 2.0)
+    Lc = vectors.depuncture(llr, N, o.punct)
+    La = vectors.siso_apriori(N)
+    for dec, w, y in ((c.decoder1, Lc[2], Lc[3]), (c.decoder2, Lc[4], Lc[5])):
+        got, want = dec.decode(Lc[0], Lc[1], w, y, *La), o.siso(Lc[0], Lc[1], w, y, *La, 0.7)
+        assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
+    got, want = dropin.bcjr_decode(Lc[0], Lc[1], Lc[2], Lc[3], *La, 1.0), o.siso(Lc[0], Lc[1], Lc[2], Lc[3], *La, 1.0)
+    assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
+    assert np.array_equal(c.decode(llr), o.decode(llr))

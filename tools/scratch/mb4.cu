@@ -1,6 +1,6 @@
 // prep-chain throughput: cycles per make_record for one warp per SM sub-partition, P independent positions per iteration
 #include <cstdio>
-#include "/root/repo/modulations_b200/csrc/tpf_core.cuh"
+#include "../../modulations_b200/csrc/tpf_core.cuh"
 using namespace b200dvb::tpf;
 template <int P, int MODE>
 __global__ void __launch_bounds__(128) prep_probe(int iters, float seed, long long *cyc, float *sink)
