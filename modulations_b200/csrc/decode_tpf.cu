@@ -2,9 +2,10 @@
 // reference (dvb_rcs2_turbo.py:116-281 bcjr_max_log_map, :464-537 decode).
 //
 // Why (DESIGN.md §4.1): a thread that holds all 16 state metrics of one frame and one
-// direction needs no shuffle and no shared-memory exchange — a trellis step is 32 FADD +
-// 16 FMNMX + 16 FSUB of straight-line code with 16-way instruction-level parallelism, so ONE
-// warp per SM sub-partition saturates the FP32 pipe (measured: 61.7 cycles per step).  What
+// direction needs no shuffle and no shared-memory exchange — a trellis step is 32 adds +
+// 16 FMNMX + 15 subtractions of straight-line code with 16-way instruction-level parallelism,
+// issued as 24 packed FADD2 (two lanes per instruction, tpf_core.cuh) + 16 FMNMX, so ONE warp per
+// SM sub-partition keeps the issue port busy (measured: 62.5 cycles per step, 77.6 unpacked).  What
 // kept this mapping out of reach was storage: 32 B of branch metrics per step per frame,
 // 64 frames per SM to feed four warps = 434 KB.  Here the SM's two on-chip memories are
 // pooled: tensor memory (256 KB, otherwise idle — the decoder has no MMA) holds the records
@@ -119,11 +120,22 @@ template <int KIND> __device__ __forceinline__ void pf_complete(const Ctx &c, Bu
     for (int i = 0; i < 8; ++i) g[i] = (KIND == 2 && c.isb) ? B.b[i] : B.a[i];
 }
 
-__device__ __forceinline__ void ck_store(const Ctx &c, int slot, const float (&v)[16])
-{   // always in natural state order: the beta lanes hold rho4 labels during the passes
-    float n[16];
+// Vectors leave the registers in the order of the step that resumes them: beta vectors in natural state order, whose
+// neighbours (z[2t], z[2t+1]) are the pairs of the packed bwd_step; alpha vectors in pair order, position p holding
+// state apos(p) = (x0, x8, x1, x9, ...), the pairs (x[t], x[8+t]) of the packed forward steps.  Either way a 16-byte
+// access moves two register pairs and the out phase needs no moves to rebuild them.
+__device__ __forceinline__ constexpr int apos(int p) { return (p >> 1) | ((p & 1) << 3); }
+// the vector of an "in" pass in its stored order: the beta lanes hold rho4 labels during the passes, and
+// rho4(2t + 1) == rho4(2t) + 8, so both half-warps store the same kind of pair (v[t], v[8+t])
+__device__ __forceinline__ void pass_out(const Ctx &c, const float (&v)[16], float (&n)[16])
+{
 #pragma unroll
-    for (int s = 0; s < 16; ++s) n[s] = c.isb ? v[rho4(s)] : v[s];
+    for (int p = 0; p < 16; ++p) n[p] = c.isb ? v[rho4(p)] : v[apos(p)];
+}
+__device__ __forceinline__ void ck_store(const Ctx &c, int slot, const float (&v)[16])
+{
+    float n[16];
+    pass_out(c, v, n);
 #pragma unroll
     for (int q = 0; q < 4; ++q)
         st_ws(c.CK + (slot * 4 + q) * 32 + c.lane, make_float4(n[4 * q], n[4 * q + 1], n[4 * q + 2], n[4 * q + 3]));
@@ -179,18 +191,27 @@ __device__ __forceinline__ void issue_ckpt(const Ctx &c, int slot)
 #pragma unroll
     for (int q = 0; q < 4; ++q) cpa16(dst + q * 32, c.CK + (slot * 4 + q) * 32 + c.lane, c.one);
 }
+// ALPHA: the slot holds an alpha vector (stored order apos), else a beta vector (natural order)
+template <bool ALPHA = false>
 __device__ __forceinline__ void slot_get(const float4 *slot, int lane, float (&v)[16])
 {
+    constexpr int P[4] = {ALPHA ? apos(0) : 0, ALPHA ? apos(1) : 1, ALPHA ? apos(2) : 2, ALPHA ? apos(3) : 3};
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         const float4 t = slot[q * 32 + lane];
-        v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
+        const int b = ALPHA ? 2 * q : 4 * q;                        // apos(4q + i) == 2q + apos(i)
+        v[b + P[0]] = t.x; v[b + P[1]] = t.y; v[b + P[2]] = t.z; v[b + P[3]] = t.w;
     }
 }
+template <bool ALPHA = false>
 __device__ __forceinline__ void slot_put(float4 *slot, int lane, const float (&v)[16])
 {
+    constexpr int P[4] = {ALPHA ? apos(0) : 0, ALPHA ? apos(1) : 1, ALPHA ? apos(2) : 2, ALPHA ? apos(3) : 3};
 #pragma unroll
-    for (int q = 0; q < 4; ++q) slot[q * 32 + lane] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+    for (int q = 0; q < 4; ++q) {
+        const int b = ALPHA ? 2 * q : 4 * q;
+        slot[q * 32 + lane] = make_float4(v[b + P[0]], v[b + P[1]], v[b + P[2]], v[b + P[3]]);
+    }
 }
 
 // Y = Lc + La travels in 32-byte entries: the two steps of a pair, in ascending k, per lane.  256-bit global
@@ -296,7 +317,7 @@ __device__ __forceinline__ void window(const Ctx &c, int wa, int w0, int len, do
         if (!c.isb) slot_put(c.slotZ(), c.lane, Z);                 // running beta of the alpha lane
     }
     float X[16];
-    slot_get(c.slotX(), c.lane, X);
+    slot_get<true>(c.slotX(), c.lane, X);
     if (nslot >= 0) issue_ckpt(c, nslot);
     cpa_commit();
     float yr[4], yn[4], uvp[4], zs[16];
@@ -324,7 +345,7 @@ __device__ __forceinline__ void window(const Ctx &c, int wa, int w0, int len, do
 #pragma unroll
     for (int i = 0; i < 4; ++i) { pend.uv[i] = uvp[i]; pend.y[i] = yr[i]; }
     pend.idx = w0 + len - 1;
-    if (c.isb) slot_put(c.slotX(), c.lane, X);                      // running alpha of the beta lane
+    if (c.isb) slot_put<true>(c.slotX(), c.lane, X);                // running alpha of the beta lane
     if (nlen) yq_park(c, nq, nw0, nlen, nslot - 1);
 }
 
@@ -523,8 +544,7 @@ __device__ __forceinline__ void siso(const Ctx &c, bool second, bool first, bool
     //      drops its vector into the PARTNER's slot -------------------------------------------
     {
         float n[16];
-#pragma unroll
-        for (int s = 0; s < 16; ++s) n[s] = c.isb ? v[rho4(s)] : v[s];
+        pass_out(c, v, n);
         slot_put(c.isb ? c.slotZ() : c.slotX(), lane ^ 16, n);
     }
     const int n_inner = (M - T) / kW;            // windows whose records are in shared memory
