@@ -132,6 +132,14 @@ int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr
                    int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                    unsigned long long *counters, void *workspace, size_t workspace_bytes,
                    void *stream);
+/* b200dvb_decode with IEEE binary16 channel LLRs: llr = uint16 bit patterns [B][llr_stride] (elements), 2-byte aligned.
+ * Every value is widened exactly to float32 and decoded as b200dvb_decode decodes it: for the same codec, options and
+ * batch, the outputs (bits, packed, counters) equal b200dvb_decode's on the float32 widening, bit for bit, in every
+ * decoder mode and for every kernel choice.  NaN / Inf inputs are undefined, as for float32.  Half the input bytes of
+ * b200dvb_decode; the workspace is the same (b200dvb_decode_workspace_bytes). */
+int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride,
+                       int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                       unsigned long long *counters, void *workspace, size_t workspace_bytes, void *stream);
 
 /* Tail-biting encoder for B frames.  Replaces DVBRCS2_Turbo.encode
  * (dvb_rcs2_turbo.py:431-462) including _encode_component (:404-429) and the

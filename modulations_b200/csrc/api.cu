@@ -291,23 +291,43 @@ int b200dvb_codec_set_option(b200dvb_codec_t codec, int option, int value)
     }
 }
 
+// b200dvb_decode / b200dvb_decode_f16: the kernel choice does not depend on the element format
+static int decode_any(b200dvb_codec_t codec, int B, const void *llr, bool f16, long long llr_stride,
+                      int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                      unsigned long long *counters, void *workspace, size_t workspace_bytes,
+                      void *stream)
+{
+    if (!codec || B < 0 || !llr || (B && !workspace)) return B200DVB_EINVAL;
+    if (llr_stride < codec->c.n_llr) return B200DVB_EINVAL;
+    if (codec->c.opt_mode != B200DVB_MODE_PARITY)
+        return nii_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters,
+                                 workspace, workspace_bytes, (cudaStream_t)stream);
+    if (use_lat(codec->c, B))
+        return lat_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters, (cudaStream_t)stream);
+    if (use_tpf(codec->c, B))
+        return tpf_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters,
+                                 workspace, workspace_bytes, (cudaStream_t)stream);
+    return launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters, workspace,
+                         workspace_bytes, (cudaStream_t)stream);
+}
+
 int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr_stride,
                    int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                    unsigned long long *counters, void *workspace, size_t workspace_bytes,
                    void *stream)
 {
-    if (!codec || B < 0 || !llr || (B && !workspace)) return B200DVB_EINVAL;
-    if (llr_stride < codec->c.n_llr) return B200DVB_EINVAL;
-    if (codec->c.opt_mode != B200DVB_MODE_PARITY)
-        return nii_launch_decode(codec->c, B, llr, llr_stride, bits, packed, ref_bits, counters,
-                                 workspace, workspace_bytes, (cudaStream_t)stream);
-    if (use_lat(codec->c, B))
-        return lat_launch_decode(codec->c, B, llr, llr_stride, bits, packed, ref_bits, counters, (cudaStream_t)stream);
-    if (use_tpf(codec->c, B))
-        return tpf_launch_decode(codec->c, B, llr, llr_stride, bits, packed, ref_bits, counters,
-                                 workspace, workspace_bytes, (cudaStream_t)stream);
-    return launch_decode(codec->c, B, llr, llr_stride, bits, packed, ref_bits, counters, workspace,
-                         workspace_bytes, (cudaStream_t)stream);
+    return decode_any(codec, B, llr, false, llr_stride, bits, packed, ref_bits, counters, workspace,
+                      workspace_bytes, stream);
+}
+
+int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride,
+                       int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                       unsigned long long *counters, void *workspace, size_t workspace_bytes,
+                       void *stream)
+{
+    if (reinterpret_cast<uintptr_t>(llr) & 1) return B200DVB_EINVAL;
+    return decode_any(codec, B, llr, true, llr_stride, bits, packed, ref_bits, counters, workspace,
+                      workspace_bytes, stream);
 }
 
 int b200dvb_encode(b200dvb_codec_t codec, int B, const uint8_t *info, uint8_t *coded,

@@ -1,11 +1,37 @@
 // common.cuh — shared declarations for libb200dvb.so (sm_100a only).
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stddef.h>
 #include "../../include/b200dvb.h"
 
 namespace b200dvb {
+
+// ---- channel LLR element format ------------------------------------------------
+// Channel LLRs arrive as float32 (b200dvb_decode) or IEEE binary16 (b200dvb_decode_f16).  The decode kernels take
+// the element type LlrT as a template parameter and read channel LLRs only through these helpers, which widen binary16
+// exactly to float32 where the value is consumed: everything after the load is the float32 kernel's, fed the same
+// float32 values.
+__device__ __forceinline__ float llr_f32(float x) { return x; }
+__device__ __forceinline__ float llr_f32(__half x) { return __half2float(x); }
+template <class L> __device__ __forceinline__ float llr_ldg(const L *p) { return llr_f32(__ldg(p)); }
+// two adjacent elements; p is aligned to two elements
+__device__ __forceinline__ float2 llr_ldg2(const float *p) { return __ldg(reinterpret_cast<const float2 *>(p)); }
+__device__ __forceinline__ float2 llr_ldg2(const __half *p) { return __half22float2(__ldg(reinterpret_cast<const __half2 *>(p))); }
+// float4 (16-byte) units of an LLR row of n elements, as the bulk-copy transpositions stage it
+template <class L> __host__ __device__ __forceinline__ int llr_row_q(int n) { return sizeof(L) == 4 ? (n + 3) / 4 : (n + 7) / 8; }
+// CTAs per SM that both element-format instances of a kernel reach: one geometry (frames per wave, grid) serves
+// float32 and binary16 input, so it must fit the one with the larger footprint
+template <class K32, class K16>
+inline cudaError_t occupancy_both_formats(int *occ, K32 k32, K16 k16, int threads, size_t smem)
+{
+    int a = 0, b = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k32, threads, smem);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k16, threads, smem);
+    *occ = a < b ? a : b;
+    return e;
+}
 
 // ---- error plumbing --------------------------------------------------------
 void set_cuda_error(cudaError_t e, const char *where);
@@ -102,7 +128,8 @@ struct Modem {
 };
 
 // launchers (each returns a B200DVB_* code)
-int launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+// llr: float32 elements, or binary16 when f16 (llr_stride in elements either way)
+int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                   uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                   void *ws, size_t ws_bytes, cudaStream_t s);
 int launch_siso(const Codec &c, int B, const float *Lc_A, const float *Lc_B, const float *Lc_W,
@@ -112,16 +139,16 @@ size_t decode_workspace_bytes(const Codec &c, int B);
 size_t siso_workspace_bytes(const Codec &c, int B);
 int quad_configure(Codec &c);
 int tpf_configure(Codec &c);
-int tpf_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s);
 size_t tpf_workspace_bytes(const Codec &c, int B);
 int tpf_read_phase_cycles(double *out_h, int reset);
 int lat_configure(Codec &c);
-int lat_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits, uint32_t *packed,
+int lat_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits, uint32_t *packed,
                       const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s);
 int nii_configure(Codec &c);
-int nii_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s);
 size_t nii_workspace_bytes(const Codec &c, int B);

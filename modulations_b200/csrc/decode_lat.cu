@@ -35,7 +35,7 @@ struct LatArgs {
     int N, B, iterations, n_llr, num_sms, warm;
     double sf_inner, sf_last;
     const int16_t *tab;             // [7][N]: perm, inv_perm, offA, offW1, offY1, offW2, offY2
-    const float *llr;
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
@@ -205,7 +205,7 @@ __device__ unsigned long long g_lat_cycles[8];
 // (thread k reads the 64-byte cell and the 32-byte record of step k with LDS.128) are free of bank conflicts: with
 // strides of 16 / 8 words eight lanes hit two / four bank groups and P2 ran at 3 700 cycles per SISO instead of 1 500
 // (ncu: its samples sit on the adds behind those loads).  Costs 48 bytes per couple: frames beyond N ~ 780 use PAD = false.
-template <bool TIMED, bool PAD>
+template <bool TIMED, bool PAD, class LlrT>
 __global__ void __launch_bounds__(kLatThreads, 2)
 lat_kernel(const LatArgs A)
 {
@@ -233,7 +233,7 @@ lat_kernel(const LatArgs A)
     for (int frame = blockIdx.x; frame < A.B; frame += gridDim.x) {
         __syncthreads();
         long long tA = TIMED ? clock64() : 0;
-        const float *row = A.llr + (size_t)frame * A.llr_stride;
+        const LlrT *row = static_cast<const LlrT *>(A.llr) + (size_t)frame * A.llr_stride;
         for (int i = tid; i < 2 * N; i += kLatThreads) perm[i] = A.tab[i];
         if (tid < 2) s_err[tid] = 0;
         for (int i = tid; i < (2 * N + 31) / 32; i += kLatThreads) words[i] = 0u;
@@ -243,8 +243,8 @@ lat_kernel(const LatArgs A)
         for (int k = tid; k < N; k += kLatThreads) {
             const int oa = g_off[k], op = g_off[perm[k]];
             const int o0 = g_off[N + k], o1 = g_off[2 * N + k], o2 = g_off[3 * N + k], o3 = g_off[4 * N + k];
-            L1[k] = make_float4(__ldg(row + oa), __ldg(row + oa + 1), o0 >= 0 ? __ldg(row + o0) : 0.f, o1 >= 0 ? __ldg(row + o1) : 0.f);
-            L2[k] = make_float4(__ldg(row + op), __ldg(row + op + 1), o2 >= 0 ? __ldg(row + o2) : 0.f, o3 >= 0 ? __ldg(row + o3) : 0.f);
+            L1[k] = make_float4(llr_ldg(row + oa), llr_ldg(row + oa + 1), o0 >= 0 ? llr_ldg(row + o0) : 0.f, o1 >= 0 ? llr_ldg(row + o1) : 0.f);
+            L2[k] = make_float4(llr_ldg(row + op), llr_ldg(row + op + 1), o2 >= 0 ? llr_ldg(row + o2) : 0.f, o3 >= 0 ? llr_ldg(row + o3) : 0.f);
         }
         __syncthreads();
         if (TIMED) { const long long t = clock64(); ph[0] += t - tA; tA = t; }
@@ -352,7 +352,7 @@ static size_t lat_cap()
     cudaDeviceProp prop;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaGetDeviceProperties(&prop, dev) != cudaSuccess) return 0;
     cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, lat_kernel<false, false>) != cudaSuccess) return 0;
+    if (cudaFuncGetAttributes(&fa, lat_kernel<false, false, float>) != cudaSuccess) return 0;   // every instance has the same static words
     return (size_t)prop.sharedMemPerBlockOptin - fa.sharedSizeBytes;   // the static words count against the limit
 }
 
@@ -367,20 +367,35 @@ int lat_configure(Codec &c)
     if (lat_smem(c.N, false) > cap) return B200DVB_OK;
     c.lat_pad = lat_smem(c.N, true) <= cap;
     const size_t need = lat_smem(c.N, c.lat_pad != 0);
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     int occ = 0;
-    if (c.lat_pad) B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lat_kernel<false, true>, kLatThreads, need));
-    else           B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lat_kernel<false, false>, kLatThreads, need));
+    if (c.lat_pad) B2_CUDA(occupancy_both_formats(&occ, lat_kernel<false, true, float>, lat_kernel<false, true, __half>, kLatThreads, need));
+    else           B2_CUDA(occupancy_both_formats(&occ, lat_kernel<false, false, float>, lat_kernel<false, false, __half>, kLatThreads, need));
     if (occ < 1) return B200DVB_OK;
     c.lat_enabled = 1;
     c.lat_frames_per_wave = (occ < 2 ? occ : 2) * prop.multiProcessorCount;   // at most two CTAs per SM
     return B200DVB_OK;
 }
 
-int lat_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits, uint32_t *packed,
+template <class LlrT> static void lat_start(const LatArgs &A, bool pad, bool timed, int grid, size_t smem, cudaStream_t s)
+{
+    if (pad) {
+        if (timed) lat_kernel<true, true, LlrT><<<grid, kLatThreads, smem, s>>>(A);
+        else       lat_kernel<false, true, LlrT><<<grid, kLatThreads, smem, s>>>(A);
+    } else {
+        if (timed) lat_kernel<true, false, LlrT><<<grid, kLatThreads, smem, s>>>(A);
+        else       lat_kernel<false, false, LlrT><<<grid, kLatThreads, smem, s>>>(A);
+    }
+}
+
+int lat_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits, uint32_t *packed,
                       const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s)
 {
     if (B == 0) return B200DVB_OK;
@@ -390,13 +405,8 @@ int lat_launch_decode(const Codec &c, int B, const float *llr, long long llr_str
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed; A.ref_bits = ref_bits; A.counters = counters;
     const int grid = B < c.lat_frames_per_wave ? B : c.lat_frames_per_wave;
     const size_t smem = lat_smem(c.N, c.lat_pad != 0);
-    if (c.lat_pad) {
-        if (c.opt_phase_timers) lat_kernel<true, true><<<grid, kLatThreads, smem, s>>>(A);
-        else                    lat_kernel<false, true><<<grid, kLatThreads, smem, s>>>(A);
-    } else {
-        if (c.opt_phase_timers) lat_kernel<true, false><<<grid, kLatThreads, smem, s>>>(A);
-        else                    lat_kernel<false, false><<<grid, kLatThreads, smem, s>>>(A);
-    }
+    if (f16) lat_start<__half>(A, c.lat_pad != 0, c.opt_phase_timers != 0, grid, smem, s);
+    else     lat_start<float>(A, c.lat_pad != 0, c.opt_phase_timers != 0, grid, smem, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

@@ -115,7 +115,7 @@ struct NiiArgs {
     float sf_inner, sf_last;
     int sf_inner_q, sf_last_q;       // the same in Q6 for the fixed-point mode
     const int16_t *tab;
-    const float *llr;
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
@@ -639,7 +639,7 @@ __device__ __forceinline__ void siso(const Ctx &c, bool second, bool first, bool
     if (TIMED) { const long long t = clock64(); ph[2] += t - tA; tA = t; }
 }
 
-template <class AR, bool TIMED>
+template <class AR, bool TIMED, class LlrT>
 __global__ void __launch_bounds__(kTpfWarps * 32, 1)
 nii_kernel(const NiiArgs A)
 {
@@ -710,7 +710,7 @@ nii_kernel(const NiiArgs A)
         const long long t0 = TIMED ? clock64() : 0;
         // ---- de-puncture + transpose the 16 frames' LLRs into [j][lane] (as decode_tpf.cu) ------------------
         if (A.vec4) {
-            const int nq = (A.n_llr + 3) / 4;                       // float4 per row (row pitch is a multiple of 16 B)
+            const int nq = llr_row_q<LlrT>(A.n_llr);                // float4 per row (row pitch is a multiple of 16 B)
             const int pitch4 = ((nq + 6) & ~7) + 1;                 // row pitch = 4 (mod 32) words: rows land in different banks
             const int rec_bytes = g.mid * 2 * 16 * (int)sizeof(float4);
             const bool in_rec = rec_bytes > kStageBytes;
@@ -739,7 +739,7 @@ nii_kernel(const NiiArgs A)
                     mbar_expect_tx(mbar, (unsigned)(live_rows * nq * 16));
                     for (int r = 0; r < G; ++r)
                         if (row_frame(g0, r) < A.B)
-                            bulk_g2s_stream(rowbuf + r * pitch4, A.llr + row_frame(g0, r) * A.llr_stride, (unsigned)(nq * 16), mbar, c.pol);
+                            bulk_g2s_stream(rowbuf + r * pitch4, static_cast<const LlrT *>(A.llr) + row_frame(g0, r) * A.llr_stride, (unsigned)(nq * 16), mbar, c.pol);
                 }
             };
             pull(0);
@@ -749,14 +749,14 @@ nii_kernel(const NiiArgs A)
                 for (int i = lane; i < lines; i += 32)
                     if ((long long)i * 128 < nb) asm volatile("prefetch.global.L2 [%0];" ::"l"(A.ref_bits + frame0 * 2 * N + i * 128));
             }
-            const float *row = reinterpret_cast<const float *>(rowbuf + fr * pitch4);
-            const float *rowh = reinterpret_cast<const float *>(rowbuf + (GL + fr) * pitch4);   // sub-frame 1 (kFpl == 2)
+            const LlrT *row = reinterpret_cast<const LlrT *>(rowbuf + fr * pitch4);
+            const LlrT *rowh = reinterpret_cast<const LlrT *>(rowbuf + (GL + fr) * pitch4);   // sub-frame 1 (kFpl == 2)
             for (int g0 = 0; g0 < kTpfFrames; g0 += GL) {
                 mbar_wait(mbar, mphase);
                 mphase ^= 1u;
                 const bool livef = frame0 + g0 + fr < A.B;
                 const bool liveh = kFpl == 2 && frame0 + kTpfFrames + g0 + fr < A.B;
-                auto val = [&](int o) { return AR::chan(livef ? row[o] : 0.f, liveh ? rowh[o] : 0.f); };
+                auto val = [&](int o) { return AR::chan(livef ? llr_f32(row[o]) : 0.f, liveh ? llr_f32(rowh[o]) : 0.f); };
 #pragma unroll 4
                 for (int k0 = 0; k0 < N; k0 += KQ) {
                     const int k = k0 + kq;
@@ -786,8 +786,9 @@ nii_kernel(const NiiArgs A)
             for (int fr = 0; fr < kTpfFrames; ++fr) {
                 const long long fl_ = frame0 + fr, fh_ = frame0 + kTpfFrames + fr;
                 const bool livef = fl_ < A.B, liveh = kFpl == 2 && fh_ < A.B;
-                const float *Lf = A.llr + (livef ? fl_ : 0) * A.llr_stride, *Lh = A.llr + (liveh ? fh_ : 0) * A.llr_stride;
-                auto val = [&](int o) { return AR::chan(livef ? __ldg(Lf + o) : 0.f, liveh ? __ldg(Lh + o) : 0.f); };
+                const LlrT *Lf = static_cast<const LlrT *>(A.llr) + (livef ? fl_ : 0) * A.llr_stride;
+                const LlrT *Lh = static_cast<const LlrT *>(A.llr) + (liveh ? fh_ : 0) * A.llr_stride;
+                auto val = [&](int o) { return AR::chan(livef ? llr_ldg(Lf + o) : 0.f, liveh ? llr_ldg(Lh + o) : 0.f); };
                 const float zero = AR::chan(0.f, 0.f);
                 float4 x1 = make_float4(zero, zero, zero, zero), x2 = x1;
                 x1.x = val(oa); x1.y = val(oa + 1); x2.x = val(op); x2.y = val(op + 1);
@@ -958,10 +959,15 @@ int nii_configure(Codec &c)
     g.off_ck = take((size_t)g.nslots * 4 * 32 * sizeof(float4));
     g.off_init = take((size_t)2 * 4 * 32 * sizeof(float4));
     g.ws_per_warp = off;
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    const int smax = (int)prop.sharedMemPerBlockOptin;
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
     g.enabled = 1;
     return B200DVB_OK;
 }
@@ -991,7 +997,18 @@ size_t nii_workspace_bytes(const Codec &c, int B)
     return (size_t)nii_grid(c, B) * kTpfWarps * c.nii.ws_per_warp + 256;
 }
 
-int nii_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+template <class LlrT> static void nii_start(const NiiArgs &A, bool fixed, bool timed, int grid, size_t smem, cudaStream_t s)
+{
+    if (fixed) {
+        if (timed) nii_kernel<ArS16, true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+        else       nii_kernel<ArS16, false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+    } else {
+        if (timed) nii_kernel<ArF32, true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+        else       nii_kernel<ArF32, false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+    }
+}
+
+int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -1003,10 +1020,11 @@ int nii_launch_decode(const Codec &c, int B, const float *llr, long long llr_str
     const int tile = fixed ? 2 * kTpfFrames : kTpfFrames;
     A.n_tiles = (B + tile - 1) / tile;
     A.n_llr = c.n_llr;
-    A.vec4 = (c.N <= 256) && (llr_stride % 4 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && ((c.n_llr + 3) / 4 * 4 <= kRowFloats) &&
+    const int nq = f16 ? llr_row_q<__half>(c.n_llr) : llr_row_q<float>(c.n_llr);
+    A.vec4 = (c.N <= 256) && ((llr_stride * (f16 ? 2 : 4)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
              !c.opt_no_row_staging;
     if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
-        const int nq = (c.n_llr + 3) / 4, pitch4 = ((nq + 6) & ~7) + 1;
+        const int pitch4 = ((nq + 6) & ~7) + 1;
         const int rec_bytes = c.nii.mid * 2 * 16 * (int)sizeof(float4);
         const int avail = rec_bytes > kStageBytes ? rec_bytes : kStageBytes - c.N * 16;
         if (avail / (pitch4 * 16) < 2) A.vec4 = 0;
@@ -1017,13 +1035,8 @@ int nii_launch_decode(const Codec &c, int B, const float *llr, long long llr_str
     A.ref_bits = ref_bits; A.counters = counters;
     A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
     const int grid = nii_grid(c, B);
-    if (fixed) {
-        if (c.opt_phase_timers) nii_kernel<ArS16, true><<<grid, kTpfWarps * 32, c.nii.smem_bytes, s>>>(A);
-        else                    nii_kernel<ArS16, false><<<grid, kTpfWarps * 32, c.nii.smem_bytes, s>>>(A);
-    } else {
-        if (c.opt_phase_timers) nii_kernel<ArF32, true><<<grid, kTpfWarps * 32, c.nii.smem_bytes, s>>>(A);
-        else                    nii_kernel<ArF32, false><<<grid, kTpfWarps * 32, c.nii.smem_bytes, s>>>(A);
-    }
+    if (f16) nii_start<__half>(A, fixed, c.opt_phase_timers != 0, grid, c.nii.smem_bytes, s);
+    else     nii_start<float>(A, fixed, c.opt_phase_timers != 0, grid, c.nii.smem_bytes, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

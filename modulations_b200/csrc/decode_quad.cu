@@ -39,7 +39,7 @@ struct QuadArgs {
     double sf_inner, sf_last;
     const int16_t *tab;
     // full decode
-    const float *llr;
+    const void *llr;      // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
@@ -50,7 +50,7 @@ struct QuadArgs {
     const double *LaA, *LaB;
     double *LeA, *LeB;
     double siso_sf;
-    int vec_ab, vec_wy;   // 8-byte loads of (A,B) / (W,Y) pairs are legal for this codec + stride
+    int vec_ab, vec_wy;   // two-element loads of (A,B) / (W,Y) pairs are legal for this codec + stride
     int timed;            // development: add this launch's per-phase cycles to g_phase_cycles
     // workspace
     double2 *Le1, *Le2, *Y;
@@ -634,7 +634,7 @@ __device__ __forceinline__ double2 make_extrinsic(const float4 uv, double YA, do
     return make_double2(ea, eb);
 }
 
-template <bool SISO_ONLY, bool TMEM, bool GREC = false>
+template <bool SISO_ONLY, bool TMEM, bool GREC = false, class LlrT = float>
 __global__ void __launch_bounds__(kMaxCtaThreads)
 quad_kernel(const QuadArgs A)
 {
@@ -744,22 +744,22 @@ quad_kernel(const QuadArgs A)
                             if (A.LaA) La[u].x = __ldg(A.LaA + e);
                             if (A.LaB) La[u].y = __ldg(A.LaB + e);
                         } else {
-                            const float *Lf = A.llr + frame * A.llr_stride;
+                            const LlrT *Lf = static_cast<const LlrT *>(A.llr) + frame * A.llr_stride;
                             const int src = second ? t_perm[k] : k;
                             const int oa = t_offA[src];
                             if (A.vec_ab) {
-                                const float2 v = __ldg(reinterpret_cast<const float2 *>(Lf + oa));
+                                const float2 v = llr_ldg2(Lf + oa);
                                 sA[u] = v.x; sB[u] = v.y;
                             } else {
-                                sA[u] = __ldg(Lf + oa); sB[u] = __ldg(Lf + oa + 1);
+                                sA[u] = llr_ldg(Lf + oa); sB[u] = llr_ldg(Lf + oa + 1);
                             }
                             const int ow = t_oW[k], oy = t_oY[k];
-                            if (A.vec_wy) {          // both parities present, adjacent and 8-byte aligned
-                                const float2 v = __ldg(reinterpret_cast<const float2 *>(Lf + ow));
+                            if (A.vec_wy) {          // both parities present, adjacent and aligned to two elements
+                                const float2 v = llr_ldg2(Lf + ow);
                                 pW[u] = v.x; pY[u] = v.y;
                             } else {
-                                if (ow >= 0) pW[u] = __ldg(Lf + ow);
-                                if (oy >= 0) pY[u] = __ldg(Lf + oy);
+                                if (ow >= 0) pW[u] = llr_ldg(Lf + ow);
+                                if (oy >= 0) pY[u] = llr_ldg(Lf + oy);
                             }
                             if (!first) La[u] = __ldcg(LePrev + (size_t)f * N + (second ? src : (int)t_inv[k]));
                         }
@@ -855,11 +855,11 @@ quad_kernel(const QuadArgs A)
                 const long long frame = frame0 + f;
                 La[u] = e1[u] = make_double2(0.0, 0.0); sA[u] = sB[u] = 0.f; rb[u] = make_uchar2(0, 0);
                 if (i < P && frame < A.B) {
-                    const float *Lf = A.llr + frame * A.llr_stride;
+                    const LlrT *Lf = static_cast<const LlrT *>(A.llr) + frame * A.llr_stride;
                     const int oa = t_offA[j];
                     La[u] = __ldcg(Le2 + (size_t)f * N + t_inv[j]);
                     e1[u] = __ldcg(Le1 + (size_t)f * N + j);
-                    sA[u] = __ldg(Lf + oa); sB[u] = __ldg(Lf + oa + 1);
+                    sA[u] = llr_ldg(Lf + oa); sB[u] = llr_ldg(Lf + oa + 1);
                     if (A.ref_bits)
                         rb[u] = *reinterpret_cast<const uchar2 *>(A.ref_bits + (size_t)frame * 2 * N + 2 * j);
                 }
@@ -1019,13 +1019,15 @@ int quad_configure(Codec &c)
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     int occ = 0;
     if (g.use_tmem) {
-        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, quad_kernel<false, true>, g.threads, g.smem_bytes));
+        B2_CUDA(occupancy_both_formats(&occ, quad_kernel<false, true>, quad_kernel<false, true, false, __half>, g.threads, g.smem_bytes));
         if (occ > 1 && g.tmem_cols > 256) occ = 1;      // two CTAs must both get their TMEM columns
         if (occ > 512 / g.tmem_cols) occ = 512 / g.tmem_cols;
     } else {
-        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, quad_kernel<false, false>, g.threads, g.smem_bytes));
+        B2_CUDA(occupancy_both_formats(&occ, quad_kernel<false, false>, quad_kernel<false, false, false, __half>, g.threads, g.smem_bytes));
     }
     if (occ < 1) return B200DVB_ENOSPEC;
     g.ctas_per_sm = occ;
@@ -1040,12 +1042,14 @@ int quad_configure(Codec &c)
         t.tmem_cols = 32;
         while (t.tmem_cols < 4 * (t.nckA + t.nckB)) t.tmem_cols *= 2;
         t.smem_bytes = quad_smem_bytes(t);
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
         // the shared memory this geometry leaves unused is worth more as L1 for the records
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                     (int)((t.smem_bytes * 100 + cap - 1) / cap) + 4));
+        const int carve = (int)((t.smem_bytes * 100 + cap - 1) / cap) + 4;
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
         int og = 0;
-        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&og, quad_kernel<false, true, true>, t.threads, t.smem_bytes));
+        B2_CUDA(occupancy_both_formats(&og, quad_kernel<false, true, true>, quad_kernel<false, true, true, __half>, t.threads, t.smem_bytes));
         if (og > 512 / t.tmem_cols) og = 512 / t.tmem_cols;
         if (og > 1) og = 1;
         if (og >= 1) { t.ctas_per_sm = og; c.geom_g = t; }
@@ -1096,7 +1100,14 @@ static inline unsigned char *align256(void *p)
     return reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(p) + 255) & ~(uintptr_t)255);
 }
 
-int launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+template <class LlrT> static void quad_start(const QuadArgs &A, const QuadGeom &G, int grid, cudaStream_t s)
+{
+    if (G.grec)          quad_kernel<false, true, true, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
+    else if (G.use_tmem) quad_kernel<false, true, false, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
+    else                 quad_kernel<false, false, false, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
+}
+
+int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                   uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                   void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -1111,16 +1122,16 @@ int launch_decode(const Codec &c, int B, const float *llr, long long llr_stride,
     A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
     A.ref_bits = ref_bits; A.counters = counters;
-    const bool even = (llr_stride % 2 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 7) == 0);
+    const uintptr_t pair_bytes = f16 ? 4 : 8;
+    const bool even = (llr_stride % 2 == 0) && ((reinterpret_cast<uintptr_t>(llr) & (pair_bytes - 1)) == 0);
     A.vec_ab = even && c.vec_ab;
     A.vec_wy = even && c.vec_wy;
     A.timed = c.opt_phase_timers;
     A.Le1 = reinterpret_cast<double2 *>(align256(ws));
     A.Le2 = A.Le1 + per; A.Y = A.Le2 + per;
     A.grec = reinterpret_cast<float *>(align256(A.Y + per));
-    if (G.grec)          quad_kernel<false, true, true><<<grid, G.threads, G.smem_bytes, s>>>(A);
-    else if (G.use_tmem) quad_kernel<false, true><<<grid, G.threads, G.smem_bytes, s>>>(A);
-    else                 quad_kernel<false, false><<<grid, G.threads, G.smem_bytes, s>>>(A);
+    if (f16) quad_start<__half>(A, G, grid, s);
+    else     quad_start<float>(A, G, grid, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

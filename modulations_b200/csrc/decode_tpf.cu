@@ -53,7 +53,7 @@ struct TpfArgs {
     int B, iterations, n_tiles, n_llr, vec4;
     double sf_inner, sf_last;
     const int16_t *tab;
-    const float *llr;
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
@@ -571,7 +571,7 @@ __device__ __forceinline__ void siso(const Ctx &c, bool second, bool first, bool
     if (TIMED) { const long long t = clock64(); ph[5] += t - tA; tA = t; }
 }
 
-template <bool TIMED>
+template <bool TIMED, class LlrT>
 __global__ void __launch_bounds__(kTpfWarps * 32, 1)
 tpf_kernel(const TpfArgs A)
 {
@@ -640,7 +640,7 @@ tpf_kernel(const TpfArgs A)
             // shared-memory areas is larger (the record area is dead between tiles).  Lane = (couple kq, frame fr)
             // with fr the minor index: one store instruction then writes 32/G couples x G frames x 16 B, i.e. FULL
             // 128-byte lines (G = 8) of the [j][lane] layout, instead of 32 partial lines.
-            const int nq = (A.n_llr + 3) / 4;                       // float4 per row (row pitch is a multiple of 16 B)
+            const int nq = llr_row_q<LlrT>(A.n_llr);                // float4 per row (row pitch is a multiple of 16 B)
             const int pitch4 = ((nq + 6) & ~7) + 1;                 // row pitch = 4 (mod 32) words: rows land in different banks
             const int rec_bytes = g.mid * 2 * 16 * (int)sizeof(float4);
             const bool in_rec = rec_bytes > kStageBytes;
@@ -666,7 +666,7 @@ tpf_kernel(const TpfArgs A)
                     fence_proxy_async();                            // the row buffer was read (or held records) before
                     mbar_expect_tx(mbar, (unsigned)(live_rows * nq * 16));
                     for (int r = 0; r < live_rows; ++r)
-                        bulk_g2s_stream(rowbuf + r * pitch4, A.llr + (frame0 + g0 + r) * A.llr_stride, (unsigned)(nq * 16), mbar, c.pol);
+                        bulk_g2s_stream(rowbuf + r * pitch4, static_cast<const LlrT *>(A.llr) + (frame0 + g0 + r) * A.llr_stride, (unsigned)(nq * 16), mbar, c.pol);
                 }
             };
             pull(0);
@@ -676,7 +676,7 @@ tpf_kernel(const TpfArgs A)
                 for (int i = lane; i < lines; i += 32)
                     if ((long long)i * 128 < nb) asm volatile("prefetch.global.L2 [%0];" ::"l"(A.ref_bits + frame0 * 2 * N + i * 128));
             }
-            const float *row = reinterpret_cast<const float *>(rowbuf + fr * pitch4);
+            const LlrT *row = reinterpret_cast<const LlrT *>(rowbuf + fr * pitch4);
             for (int g0 = 0; g0 < kTpfFrames; g0 += G) {
                 mbar_wait(mbar, mphase);
                 mphase ^= 1u;
@@ -689,11 +689,11 @@ tpf_kernel(const TpfArgs A)
                     const int o2 = (short)(e.z & 0xffff), o3 = e.z >> 16;
                     float4 x1 = make_float4(0.f, 0.f, 0.f, 0.f), x2 = x1;
                     if (livef) {
-                        x1.x = row[oa]; x1.y = row[oa + 1]; x2.x = row[op]; x2.y = row[op + 1];
-                        if (o0 >= 0) x1.z = row[o0];
-                        if (o1 >= 0) x1.w = row[o1];
-                        if (o2 >= 0) x2.z = row[o2];
-                        if (o3 >= 0) x2.w = row[o3];
+                        x1.x = llr_f32(row[oa]); x1.y = llr_f32(row[oa + 1]); x2.x = llr_f32(row[op]); x2.y = llr_f32(row[op + 1]);
+                        if (o0 >= 0) x1.z = llr_f32(row[o0]);
+                        if (o1 >= 0) x1.w = llr_f32(row[o1]);
+                        if (o2 >= 0) x2.z = llr_f32(row[o2]);
+                        if (o3 >= 0) x2.w = llr_f32(row[o3]);
                     }
                     if (k < N) {
                         st_ws(c.L1A + lpos(c, k, g0 + fr), x1);
@@ -714,15 +714,15 @@ tpf_kernel(const TpfArgs A)
 #pragma unroll
                 for (int fr = 0; fr < 8; ++fr) {
                     const long long frame = frame0 + f0 + fr;
-                    const float *Lf = A.llr + frame * A.llr_stride;
+                    const LlrT *Lf = static_cast<const LlrT *>(A.llr) + frame * A.llr_stride;
                     x1[fr] = make_float4(0.f, 0.f, 0.f, 0.f); x2[fr] = x1[fr];
                     if (frame < A.B) {
-                        x1[fr].x = __ldg(Lf + oa); x1[fr].y = __ldg(Lf + oa + 1);
-                        x2[fr].x = __ldg(Lf + op); x2[fr].y = __ldg(Lf + op + 1);
-                        if (o0 >= 0) x1[fr].z = __ldg(Lf + o0);
-                        if (o1 >= 0) x1[fr].w = __ldg(Lf + o1);
-                        if (o2 >= 0) x2[fr].z = __ldg(Lf + o2);
-                        if (o3 >= 0) x2[fr].w = __ldg(Lf + o3);
+                        x1[fr].x = llr_ldg(Lf + oa); x1[fr].y = llr_ldg(Lf + oa + 1);
+                        x2[fr].x = llr_ldg(Lf + op); x2[fr].y = llr_ldg(Lf + op + 1);
+                        if (o0 >= 0) x1[fr].z = llr_ldg(Lf + o0);
+                        if (o1 >= 0) x1[fr].w = llr_ldg(Lf + o1);
+                        if (o2 >= 0) x2[fr].z = llr_ldg(Lf + o2);
+                        if (o3 >= 0) x2[fr].w = llr_ldg(Lf + o3);
                     }
                 }
 #pragma unroll
@@ -877,8 +877,10 @@ int tpf_configure(Codec &c)
     g.off_ck = take((size_t)g.nslots * 4 * 32 * sizeof(float4));
     g.ws_per_warp = off;
     // the device's maximum, not this codec's need: the attribute is per function and device, and codecs of several N coexist
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     g.enabled = 1;
     return B200DVB_OK;
 }
@@ -907,7 +909,14 @@ size_t tpf_workspace_bytes(const Codec &c, int B)
     return (size_t)tpf_grid(c, B) * kTpfWarps * c.tpf.ws_per_warp + 256;
 }
 
-int tpf_launch_decode(const Codec &c, int B, const float *llr, long long llr_stride, int32_t *bits,
+// B200DVB_OPT_PHASE_TIMERS (development): the instance with per-phase clock64() accounting, read by b200dvb_debug_tpf_cycles
+template <class LlrT> static void tpf_start(const TpfArgs &A, bool timed, int grid, size_t smem, cudaStream_t s)
+{
+    if (timed) tpf_kernel<true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+    else       tpf_kernel<false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+}
+
+int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -917,11 +926,12 @@ int tpf_launch_decode(const Codec &c, int B, const float *llr, long long llr_str
     A.g = c.tpf; A.B = B; A.iterations = c.iterations;
     A.n_tiles = (B + kTpfFrames - 1) / kTpfFrames;
     A.n_llr = c.n_llr;
-    // whole rows by 16-byte cp.async: pitch and base 16-byte aligned, row fits half the staging area
-    A.vec4 = (c.N <= 256) && (llr_stride % 4 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && ((c.n_llr + 3) / 4 * 4 <= kRowFloats) &&
+    // whole rows by bulk copy: pitch and base 16-byte aligned, row fits half the staging area
+    const int nq = f16 ? llr_row_q<__half>(c.n_llr) : llr_row_q<float>(c.n_llr);
+    A.vec4 = (c.N <= 256) && ((llr_stride * (f16 ? 2 : 4)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
              !c.opt_no_row_staging;
     if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
-        const int nq = (c.n_llr + 3) / 4, pitch4 = ((nq + 6) & ~7) + 1;
+        const int pitch4 = ((nq + 6) & ~7) + 1;
         const int rec_bytes = c.tpf.mid * 2 * 16 * (int)sizeof(float4);
         const int avail = rec_bytes > kStageBytes ? rec_bytes : kStageBytes - c.N * 16;
         if (avail / (pitch4 * 16) < 2) A.vec4 = 0;
@@ -930,10 +940,8 @@ int tpf_launch_decode(const Codec &c, int B, const float *llr, long long llr_str
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
     A.ref_bits = ref_bits; A.counters = counters;
     A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-    // B200DVB_OPT_PHASE_TIMERS (development): the instance with per-phase clock64() accounting, read by b200dvb_debug_tpf_cycles
-    const bool timed = c.opt_phase_timers != 0;
-    if (timed) tpf_kernel<true><<<tpf_grid(c, B), kTpfWarps * 32, c.tpf.smem_bytes, s>>>(A);
-    else       tpf_kernel<false><<<tpf_grid(c, B), kTpfWarps * 32, c.tpf.smem_bytes, s>>>(A);
+    if (f16) tpf_start<__half>(A, c.opt_phase_timers != 0, tpf_grid(c, B), c.tpf.smem_bytes, s);
+    else     tpf_start<float>(A, c.opt_phase_timers != 0, tpf_grid(c, B), c.tpf.smem_bytes, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

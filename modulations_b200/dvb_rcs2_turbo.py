@@ -198,16 +198,18 @@ class _CodecHandle:
         return coded, circ
 
     def decode(self, x, bits=None, packed=None, ref=None, counters=None, stream=None, ws=None):
-        """x float32 CUDA [B, >= n_llr] (row stride in elements taken from the tensor)."""
+        """x float32 or float16 CUDA [B, >= n_llr] (row stride in elements taken from the tensor).  float16 goes to
+        b200dvb_decode_f16: the decode of its exact float32 widening, bit for bit."""
         torch = _lib.torch_mod()
         B = x.shape[0]
         st = stream or self.stream()
+        lib = _lib.load()
+        fn = lib.b200dvb_decode_f16 if x.dtype == torch.float16 else lib.b200dvb_decode
         with torch.cuda.device(self.device):
             buf, need = ws if ws is not None else self.workspace("decode", B, st)
             stride = x.stride(0) if B > 1 else x.shape[1]     # a length-1 axis may report stride 0
-            rc = _lib.load().b200dvb_decode(self.h, B, _lib.ptr(x), stride, _lib.ptr(bits), _lib.ptr(packed),
-                                            _lib.ptr(ref), _lib.ptr(counters), _lib.ptr(buf), need,
-                                            ctypes.c_void_p(st.cuda_stream))
+            rc = fn(self.h, B, _lib.ptr(x), stride, _lib.ptr(bits), _lib.ptr(packed), _lib.ptr(ref),
+                    _lib.ptr(counters), _lib.ptr(buf), need, ctypes.c_void_p(st.cuda_stream))
         _lib.check(rc, "decode")
 
     def siso(self, f4, d2, sf):
@@ -465,6 +467,10 @@ class DVBRCS2_Turbo:
     def decode_batch(self, llr, ref_bits=None, counters=None, out="bits"):
         """llr [B, >= n_llr] float32 (numpy or CUDA torch) -> hard decisions.
 
+        float16 input (``torch.float16`` or ``np.float16``) reaches the device as 16 bits and is decoded by the
+        binary16 path: fp16 in = decode of its exact float32 widening, bit for bit, in every mode and kernel.  Any
+        other dtype is converted to float32.
+
         out="bits": int32 [B, 2N] (reference layout); "packed": uint32 [B, ceil(2N/32)], bit i of a frame at
         word i//32, bit i%32; "none": nothing (error counting only).  ``ref_bits`` (anything reshapeable to
         uint8 [B, 2N]) and ``counters`` (CUDA int64/uint64 tensor, >= 4 elements) enable in-kernel error
@@ -475,7 +481,10 @@ class DVBRCS2_Turbo:
         if out not in ("bits", "packed", "none"):
             raise ValueError('out must be "bits", "packed" or "none"')
         is_torch = isinstance(llr, torch.Tensor)
-        x = _lib.to_device(llr, torch.float32, h.device)
+        if not is_torch:
+            llr = np.asarray(llr)
+        half = llr.dtype == (torch.float16 if is_torch else np.float16)
+        x = _lib.to_device(llr, torch.float16 if half else torch.float32, h.device)
         if x.dim() == 1:
             x = x[None, :]
         if x.dim() != 2 or x.shape[1] < h.n_llr:
@@ -506,7 +515,10 @@ class DVBRCS2_Turbo:
         return res
 
     def decode_batch_host(self, llr_host, out_host=None, chunk=None, out="bits"):
-        """End-to-end decode of HOST buffers: pinned ``llr_host`` float32 [B, >= n_llr] -> pinned ``out_host``.
+        """End-to-end decode of HOST buffers: pinned ``llr_host`` float32 or float16 [B, >= n_llr] -> pinned ``out_host``.
+
+        float16 rows cross PCIe as 16 bits (half the bytes) and are decoded by the binary16 path: fp16 in = decode of
+        its exact float32 widening, bit for bit.
 
         out="bits": int32 [B, 2N], the reference's layout (1 696 B per N=212 frame over PCIe);
         out="packed": int32 words [B, ceil(2N/32)], bit i of a frame at word i//32, bit i%32 (56 B per frame:
@@ -523,9 +535,13 @@ class DVBRCS2_Turbo:
             raise ValueError('out must be "bits", "packed" or "uint8"')
         if chunk is None:
             chunk = max(16, h.frames_per_wave)
-        x = llr_host if isinstance(llr_host, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(llr_host, np.float32))
-        if x.dim() != 2 or x.shape[1] < h.n_llr or x.dtype != torch.float32:
-            raise IndexError(f"llr needs float32 shape [B, >= {h.n_llr}]")
+        if isinstance(llr_host, torch.Tensor):
+            x = llr_host
+        else:
+            a = np.asarray(llr_host)
+            x = torch.from_numpy(np.ascontiguousarray(a, np.float16 if a.dtype == np.float16 else np.float32))
+        if x.dim() != 2 or x.shape[1] < h.n_llr or x.dtype not in (torch.float32, torch.float16):
+            raise IndexError(f"llr needs float32 or float16 shape [B, >= {h.n_llr}]")
         B, width = x.shape
         wpf = (self.k_info + 31) // 32
         oshape, odtype = {"bits": ((self.k_info,), torch.int32), "packed": ((wpf,), torch.int32),
@@ -535,11 +551,11 @@ class DVBRCS2_Turbo:
         elif tuple(out_host.shape) != (B,) + oshape or out_host.dtype != odtype:
             raise ValueError(f"out_host must be {odtype} of shape {(B,) + oshape}")
         nstage = 3
-        key = (h, chunk, width, out)
+        key = (h, chunk, width, out, x.dtype)
         if self._e2e is None or self._e2e[0] != key:
             with torch.cuda.device(h.device):
                 streams = [torch.cuda.Stream(device=h.device) for _ in range(nstage)]
-                din = [torch.empty((chunk, width), dtype=torch.float32, device=h.device) for _ in range(nstage)]
+                din = [torch.empty((chunk, width), dtype=x.dtype, device=h.device) for _ in range(nstage)]
                 dout = [torch.empty((chunk,) + oshape, dtype=odtype, device=h.device) for _ in range(nstage)]
                 dpk = [torch.empty((chunk, wpf), dtype=torch.int32, device=h.device) if out == "uint8" else None
                        for _ in range(nstage)]

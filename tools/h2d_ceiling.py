@@ -4,14 +4,15 @@
 plain cudaMemcpyAsync on two streams and NO kernel, all ranks at once.  The aggregate is the most any
 host-buffer decode can reach on this box: e2e Gbit/s <= frames/s at the ceiling x 2N.
 
-    python tools/h2d_ceiling.py                       (1 GPU)
+    python tools/h2d_ceiling.py [FRAMES] [--llr-bytes 4|2]     (1 GPU)
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/h2d_ceiling.py
 
-Prints one JSON line per run (rank 0): per-direction GB/s per rank (min/max) and summed.
+--llr-bytes 2: the LLRs cross as float16 (decode_batch_host with a float16 buffer), half the H2D bytes; the default
+is float32.  Prints one JSON line per run (rank 0): per-direction GB/s per rank (min/max) and summed.
 """
+import argparse
 import json
 import os
-import sys
 
 import torch
 import torch.distributed as dist
@@ -19,18 +20,11 @@ import torch.distributed as dist
 N, N_LLR = 212, 1272
 
 
-def main():
-    rank = int(os.environ.get("RANK", "0"))
-    world = int(os.environ.get("WORLD_SIZE", "1"))
-    local = int(os.environ.get("LOCAL_RANK", "0"))
-    frames = int(sys.argv[1]) if len(sys.argv) > 1 else 262144
-    torch.cuda.set_device(local)
-    dev = torch.device("cuda", local)
-    if world > 1:
-        dist.init_process_group("nccl", device_id=dev)
+def measure(frames, esz, dev, world):
+    """{layout: ceiling figures} for `frames` frames per rank and step, LLRs of `esz` bytes; all ranks at once."""
     out = {}
     for label, d2h_per_frame in (("int32_bits", 2 * N * 4), ("packed_bits", ((2 * N + 31) // 32) * 4)):
-        hin = torch.empty((frames, N_LLR), dtype=torch.float32, pin_memory=True)
+        hin = torch.empty((frames, N_LLR), dtype=torch.float32 if esz == 4 else torch.float16, pin_memory=True)
         hout = torch.empty(frames * d2h_per_frame, dtype=torch.uint8, pin_memory=True)
         din = torch.empty_like(hin, device=dev)
         dout = torch.empty_like(hout, device=dev)
@@ -65,19 +59,37 @@ def main():
         if world > 1:
             dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
         ms_max = float(tmax.item())
-        h2d = frames * N_LLR * 4
+        h2d = frames * N_LLR * esz
         d2h = frames * d2h_per_frame
         out[label] = {"ms_per_step_max_over_ranks": ms_max, "h2d_gbs_per_rank": h2d / ms_max / 1e6,
                       "d2h_gbs_per_rank": d2h / ms_max / 1e6, "h2d_gbs_total": world * h2d / ms_max / 1e6,
                       "frames_per_s_total": world * frames / (ms_max * 1e-3),
                       "info_gbit_per_s_ceiling": world * frames * 2 * N / (ms_max * 1e-3) / 1e9}
         del hin, hout, din, dout
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("frames", nargs="?", type=int, default=262144)
+    ap.add_argument("--llr-bytes", type=int, choices=(4, 2), default=4, help="bytes per LLR element: 4 float32, 2 float16")
+    args = ap.parse_args()
+    frames, esz = args.frames, args.llr_bytes
+    rank = int(os.environ.get("RANK", "0"))
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local)
+    dev = torch.device("cuda", local)
+    if world > 1:
+        dist.init_process_group("nccl", device_id=dev)
+    out = measure(frames, esz, dev, world)
     if rank == 0:
         try:
             aff = len(os.sched_getaffinity(0))
         except Exception:
             aff = None
-        print(json.dumps({"tool": "h2d_ceiling", "n_gpus": world, "frames_per_rank_per_step": frames,
+        extra = {} if esz == 4 else {"llr_bytes": esz}
+        print(json.dumps({"tool": "h2d_ceiling", "n_gpus": world, "frames_per_rank_per_step": frames, **extra,
                           "cpu_count": os.cpu_count(), "affinity": aff, **out}), flush=True)
     if world > 1:
         dist.destroy_process_group()
