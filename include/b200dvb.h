@@ -140,6 +140,17 @@ int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr
 int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride,
                        int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                        unsigned long long *counters, void *workspace, size_t workspace_bytes, void *stream);
+/* b200dvb_decode with 8-bit channel LLRs and a scale: llr = int8 [B][llr_stride] (elements = bytes), any alignment.
+ * Element q (-128 ... 127) is decoded as the float32 value q * scale, rounded as IEEE float32 multiplication rounds it
+ * (no FTZ, no fused multiply-add): for the same codec, options and batch, the outputs (bits, packed, counters) equal
+ * b200dvb_decode's on the float32 array float32(q) * scale, bit for bit, in every decoder mode and for every kernel
+ * choice.  scale must be finite and non-zero (else B200DVB_EINVAL); a negative scale flips the sign convention.
+ * In B200DVB_MODE_NII16 (LLRs in 1/4 units), int8 q = clamp(rint(4 x), -127, 127) with scale 0.25 decodes exactly as
+ * float32 x does: the mode's own quantisation of x is that q.  A quarter of the input bytes of b200dvb_decode; the
+ * workspace is the same (b200dvb_decode_workspace_bytes). */
+int b200dvb_decode_i8(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride, float scale,
+                      int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                      unsigned long long *counters, void *workspace, size_t workspace_bytes, void *stream);
 
 /* Tail-biting encoder for B frames.  Replaces DVBRCS2_Turbo.encode
  * (dvb_rcs2_turbo.py:431-462) including _encode_component (:404-429) and the

@@ -41,6 +41,7 @@ SIGNATURES = {
     "b200dvb_decode_workspace_bytes": (_c_size_t, [_c_void_p, _c_int]),
     "b200dvb_decode": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
     "b200dvb_decode_f16": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
+    "b200dvb_decode_i8": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll, _c_float] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
     "b200dvb_encode": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
     "b200dvb_mc_generate_bpsk": (_c_int, [_c_void_p, _c_int, _c_float, _c_ull, _c_ull] + [_c_void_p] * 4),
     "b200dvb_awgn_complex": (_c_int, [_c_size_t, _c_float, _c_ull, _c_ull, _c_void_p, _c_void_p]),

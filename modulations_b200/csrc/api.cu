@@ -291,8 +291,8 @@ int b200dvb_codec_set_option(b200dvb_codec_t codec, int option, int value)
     }
 }
 
-// b200dvb_decode / b200dvb_decode_f16: the kernel choice does not depend on the element format
-static int decode_any(b200dvb_codec_t codec, int B, const void *llr, bool f16, long long llr_stride,
+// b200dvb_decode / _f16 / _i8: the kernel choice does not depend on the element format
+static int decode_any(b200dvb_codec_t codec, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride,
                       int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                       unsigned long long *counters, void *workspace, size_t workspace_bytes,
                       void *stream)
@@ -300,14 +300,14 @@ static int decode_any(b200dvb_codec_t codec, int B, const void *llr, bool f16, l
     if (!codec || B < 0 || !llr || (B && !workspace)) return B200DVB_EINVAL;
     if (llr_stride < codec->c.n_llr) return B200DVB_EINVAL;
     if (codec->c.opt_mode != B200DVB_MODE_PARITY)
-        return nii_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters,
+        return nii_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters,
                                  workspace, workspace_bytes, (cudaStream_t)stream);
     if (use_lat(codec->c, B))
-        return lat_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters, (cudaStream_t)stream);
+        return lat_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, (cudaStream_t)stream);
     if (use_tpf(codec->c, B))
-        return tpf_launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters,
+        return tpf_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters,
                                  workspace, workspace_bytes, (cudaStream_t)stream);
-    return launch_decode(codec->c, B, llr, f16, llr_stride, bits, packed, ref_bits, counters, workspace,
+    return launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, workspace,
                          workspace_bytes, (cudaStream_t)stream);
 }
 
@@ -316,7 +316,7 @@ int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr
                    unsigned long long *counters, void *workspace, size_t workspace_bytes,
                    void *stream)
 {
-    return decode_any(codec, B, llr, false, llr_stride, bits, packed, ref_bits, counters, workspace,
+    return decode_any(codec, B, llr, LlrFormat::F32, 1.f, llr_stride, bits, packed, ref_bits, counters, workspace,
                       workspace_bytes, stream);
 }
 
@@ -326,7 +326,17 @@ int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long 
                        void *stream)
 {
     if (reinterpret_cast<uintptr_t>(llr) & 1) return B200DVB_EINVAL;
-    return decode_any(codec, B, llr, true, llr_stride, bits, packed, ref_bits, counters, workspace,
+    return decode_any(codec, B, llr, LlrFormat::F16, 1.f, llr_stride, bits, packed, ref_bits, counters, workspace,
+                      workspace_bytes, stream);
+}
+
+int b200dvb_decode_i8(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride, float scale,
+                      int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                      unsigned long long *counters, void *workspace, size_t workspace_bytes,
+                      void *stream)
+{
+    if (!isfinite(scale) || scale == 0.f) return B200DVB_EINVAL;
+    return decode_any(codec, B, llr, LlrFormat::I8, scale, llr_stride, bits, packed, ref_bits, counters, workspace,
                       workspace_bytes, stream);
 }
 

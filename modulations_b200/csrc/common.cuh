@@ -9,27 +9,45 @@
 namespace b200dvb {
 
 // ---- channel LLR element format ------------------------------------------------
-// Channel LLRs arrive as float32 (b200dvb_decode) or IEEE binary16 (b200dvb_decode_f16).  The decode kernels take
-// the element type LlrT as a template parameter and read channel LLRs only through these helpers, which widen binary16
-// exactly to float32 where the value is consumed: everything after the load is the float32 kernel's, fed the same
-// float32 values.
-__device__ __forceinline__ float llr_f32(float x) { return x; }
-__device__ __forceinline__ float llr_f32(__half x) { return __half2float(x); }
-template <class L> __device__ __forceinline__ float llr_ldg(const L *p) { return llr_f32(__ldg(p)); }
+// Channel LLRs arrive as float32 (b200dvb_decode), IEEE binary16 (b200dvb_decode_f16) or int8 with a float32 scale
+// (b200dvb_decode_i8).  The decode kernels take the element type LlrT as a template parameter and read channel LLRs
+// only through these helpers, which turn an element into its float32 value where the value is consumed: binary16 is
+// widened exactly, int8 q becomes the IEEE product q * scale (the library builds with --fmad=false).  Everything after
+// the load is the float32 kernel's, fed the same float32 values.  The float32 and binary16 overloads ignore the scale.
+enum class LlrFormat { F32, F16, I8 };
+inline int llr_bytes(LlrFormat f) { return f == LlrFormat::F32 ? 4 : f == LlrFormat::F16 ? 2 : 1; }
+__device__ __forceinline__ float llr_f32(float x, float) { return x; }
+__device__ __forceinline__ float llr_f32(__half x, float) { return __half2float(x); }
+__device__ __forceinline__ float llr_f32(int8_t x, float s) { return __fmul_rn((float)x, s); }
+template <class L> __device__ __forceinline__ float llr_ldg(const L *p, float s) { return llr_f32(__ldg(p), s); }
 // two adjacent elements; p is aligned to two elements
-__device__ __forceinline__ float2 llr_ldg2(const float *p) { return __ldg(reinterpret_cast<const float2 *>(p)); }
-__device__ __forceinline__ float2 llr_ldg2(const __half *p) { return __half22float2(__ldg(reinterpret_cast<const __half2 *>(p))); }
-// float4 (16-byte) units of an LLR row of n elements, as the bulk-copy transpositions stage it
-template <class L> __host__ __device__ __forceinline__ int llr_row_q(int n) { return sizeof(L) == 4 ? (n + 3) / 4 : (n + 7) / 8; }
-// CTAs per SM that both element-format instances of a kernel reach: one geometry (frames per wave, grid) serves
-// float32 and binary16 input, so it must fit the one with the larger footprint
-template <class K32, class K16>
-inline cudaError_t occupancy_both_formats(int *occ, K32 k32, K16 k16, int threads, size_t smem)
+__device__ __forceinline__ float2 llr_ldg2(const float *p, float) { return __ldg(reinterpret_cast<const float2 *>(p)); }
+__device__ __forceinline__ float2 llr_ldg2(const __half *p, float) { return __half22float2(__ldg(reinterpret_cast<const __half2 *>(p))); }
+__device__ __forceinline__ float2 llr_ldg2(const int8_t *p, float s)
 {
-    int a = 0, b = 0;
+    const char2 v = __ldg(reinterpret_cast<const char2 *>(p));
+    return make_float2(__fmul_rn((float)v.x, s), __fmul_rn((float)v.y, s));
+}
+// float4 (16-byte) units of an LLR row of n elements, as the bulk-copy transpositions stage it
+template <class L> __host__ __device__ __forceinline__ int llr_row_q(int n)
+{
+    return sizeof(L) == 4 ? (n + 3) / 4 : sizeof(L) == 2 ? (n + 7) / 8 : (n + 15) / 16;
+}
+inline int llr_row_q(LlrFormat f, int n)
+{
+    return f == LlrFormat::F32 ? llr_row_q<float>(n) : f == LlrFormat::F16 ? llr_row_q<__half>(n) : llr_row_q<int8_t>(n);
+}
+// CTAs per SM that every element-format instance of a kernel reaches: one geometry (frames per wave, grid) serves
+// float32, binary16 and int8 input, so it must fit the one with the largest footprint
+template <class K32, class K16, class K8>
+inline cudaError_t occupancy_all_formats(int *occ, K32 k32, K16 k16, K8 k8, int threads, size_t smem)
+{
+    int a = 0, b = 0, c = 0;
     cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k32, threads, smem);
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k16, threads, smem);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, k8, threads, smem);
     *occ = a < b ? a : b;
+    if (c < *occ) *occ = c;
     return e;
 }
 
@@ -128,8 +146,8 @@ struct Modem {
 };
 
 // launchers (each returns a B200DVB_* code)
-// llr: float32 elements, or binary16 when f16 (llr_stride in elements either way)
-int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+// llr: elements of format fmt (llr_stride in elements); llr_scale multiplies int8 elements and is unused otherwise
+int launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                   uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                   void *ws, size_t ws_bytes, cudaStream_t s);
 int launch_siso(const Codec &c, int B, const float *Lc_A, const float *Lc_B, const float *Lc_W,
@@ -139,16 +157,16 @@ size_t decode_workspace_bytes(const Codec &c, int B);
 size_t siso_workspace_bytes(const Codec &c, int B);
 int quad_configure(Codec &c);
 int tpf_configure(Codec &c);
-int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+int tpf_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s);
 size_t tpf_workspace_bytes(const Codec &c, int B);
 int tpf_read_phase_cycles(double *out_h, int reset);
 int lat_configure(Codec &c);
-int lat_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits, uint32_t *packed,
+int lat_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits, uint32_t *packed,
                       const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s);
 int nii_configure(Codec &c);
-int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+int nii_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s);
 size_t nii_workspace_bytes(const Codec &c, int B);

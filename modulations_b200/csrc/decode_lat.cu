@@ -35,12 +35,13 @@ struct LatArgs {
     int N, B, iterations, n_llr, num_sms, warm;
     double sf_inner, sf_last;
     const int16_t *tab;             // [7][N]: perm, inv_perm, offA, offW1, offY1, offW2, offY2
-    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32, binary16 or int8)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
     const uint8_t *ref_bits;
     unsigned long long *counters;
+    float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
 };
 
 __device__ __forceinline__ void ld16(const float *p, float (&v)[16])
@@ -243,8 +244,9 @@ lat_kernel(const LatArgs A)
         for (int k = tid; k < N; k += kLatThreads) {
             const int oa = g_off[k], op = g_off[perm[k]];
             const int o0 = g_off[N + k], o1 = g_off[2 * N + k], o2 = g_off[3 * N + k], o3 = g_off[4 * N + k];
-            L1[k] = make_float4(llr_ldg(row + oa), llr_ldg(row + oa + 1), o0 >= 0 ? llr_ldg(row + o0) : 0.f, o1 >= 0 ? llr_ldg(row + o1) : 0.f);
-            L2[k] = make_float4(llr_ldg(row + op), llr_ldg(row + op + 1), o2 >= 0 ? llr_ldg(row + o2) : 0.f, o3 >= 0 ? llr_ldg(row + o3) : 0.f);
+            const float sc = A.llr_scale;                           // int8 input only (llr_f32)
+            L1[k] = make_float4(llr_ldg(row + oa, sc), llr_ldg(row + oa + 1, sc), o0 >= 0 ? llr_ldg(row + o0, sc) : 0.f, o1 >= 0 ? llr_ldg(row + o1, sc) : 0.f);
+            L2[k] = make_float4(llr_ldg(row + op, sc), llr_ldg(row + op + 1, sc), o2 >= 0 ? llr_ldg(row + o2, sc) : 0.f, o3 >= 0 ? llr_ldg(row + o3, sc) : 0.f);
         }
         __syncthreads();
         if (TIMED) { const long long t = clock64(); ph[0] += t - tA; tA = t; }
@@ -375,9 +377,15 @@ int lat_configure(Codec &c)
     B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     int occ = 0;
-    if (c.lat_pad) B2_CUDA(occupancy_both_formats(&occ, lat_kernel<false, true, float>, lat_kernel<false, true, __half>, kLatThreads, need));
-    else           B2_CUDA(occupancy_both_formats(&occ, lat_kernel<false, false, float>, lat_kernel<false, false, __half>, kLatThreads, need));
+    if (c.lat_pad) B2_CUDA(occupancy_all_formats(&occ, lat_kernel<false, true, float>, lat_kernel<false, true, __half>,
+                                                 lat_kernel<false, true, int8_t>, kLatThreads, need));
+    else           B2_CUDA(occupancy_all_formats(&occ, lat_kernel<false, false, float>, lat_kernel<false, false, __half>,
+                                                 lat_kernel<false, false, int8_t>, kLatThreads, need));
     if (occ < 1) return B200DVB_OK;
     c.lat_enabled = 1;
     c.lat_frames_per_wave = (occ < 2 ? occ : 2) * prop.multiProcessorCount;   // at most two CTAs per SM
@@ -395,7 +403,7 @@ template <class LlrT> static void lat_start(const LatArgs &A, bool pad, bool tim
     }
 }
 
-int lat_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits, uint32_t *packed,
+int lat_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits, uint32_t *packed,
                       const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s)
 {
     if (B == 0) return B200DVB_OK;
@@ -403,10 +411,13 @@ int lat_launch_decode(const Codec &c, int B, const void *llr, bool f16, long lon
     A.N = c.N; A.B = B; A.iterations = c.iterations; A.n_llr = c.n_llr; A.num_sms = c.num_sms; A.warm = g_lat_warm > 0 ? g_lat_warm : lat_warm_for(c.N);
     A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed; A.ref_bits = ref_bits; A.counters = counters;
+    A.llr_scale = llr_scale;
     const int grid = B < c.lat_frames_per_wave ? B : c.lat_frames_per_wave;
     const size_t smem = lat_smem(c.N, c.lat_pad != 0);
-    if (f16) lat_start<__half>(A, c.lat_pad != 0, c.opt_phase_timers != 0, grid, smem, s);
-    else     lat_start<float>(A, c.lat_pad != 0, c.opt_phase_timers != 0, grid, smem, s);
+    const bool pad = c.lat_pad != 0, timed = c.opt_phase_timers != 0;
+    if (fmt == LlrFormat::F16)     lat_start<__half>(A, pad, timed, grid, smem, s);
+    else if (fmt == LlrFormat::I8) lat_start<int8_t>(A, pad, timed, grid, smem, s);
+    else                           lat_start<float>(A, pad, timed, grid, smem, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

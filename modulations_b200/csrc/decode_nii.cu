@@ -115,13 +115,14 @@ struct NiiArgs {
     float sf_inner, sf_last;
     int sf_inner_q, sf_last_q;       // the same in Q6 for the fixed-point mode
     const int16_t *tab;
-    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32, binary16 or int8)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
     const uint8_t *ref_bits;
     unsigned long long *counters;
     unsigned char *ws;
+    float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
 };
 
 struct Ctx {
@@ -708,6 +709,7 @@ nii_kernel(const NiiArgs A)
     for (int tile = wg; tile < A.n_tiles; tile += gridDim.x * kTpfWarps) {
         const long long frame0 = (long long)tile * kTile;
         const long long t0 = TIMED ? clock64() : 0;
+        const float sc = A.llr_scale;                               // int8 input only (llr_f32)
         // ---- de-puncture + transpose the 16 frames' LLRs into [j][lane] (as decode_tpf.cu) ------------------
         if (A.vec4) {
             const int nq = llr_row_q<LlrT>(A.n_llr);                // float4 per row (row pitch is a multiple of 16 B)
@@ -756,7 +758,7 @@ nii_kernel(const NiiArgs A)
                 mphase ^= 1u;
                 const bool livef = frame0 + g0 + fr < A.B;
                 const bool liveh = kFpl == 2 && frame0 + kTpfFrames + g0 + fr < A.B;
-                auto val = [&](int o) { return AR::chan(livef ? llr_f32(row[o]) : 0.f, liveh ? llr_f32(rowh[o]) : 0.f); };
+                auto val = [&](int o) { return AR::chan(livef ? llr_f32(row[o], sc) : 0.f, liveh ? llr_f32(rowh[o], sc) : 0.f); };
 #pragma unroll 4
                 for (int k0 = 0; k0 < N; k0 += KQ) {
                     const int k = k0 + kq;
@@ -788,7 +790,7 @@ nii_kernel(const NiiArgs A)
                 const bool livef = fl_ < A.B, liveh = kFpl == 2 && fh_ < A.B;
                 const LlrT *Lf = static_cast<const LlrT *>(A.llr) + (livef ? fl_ : 0) * A.llr_stride;
                 const LlrT *Lh = static_cast<const LlrT *>(A.llr) + (liveh ? fh_ : 0) * A.llr_stride;
-                auto val = [&](int o) { return AR::chan(livef ? llr_ldg(Lf + o) : 0.f, liveh ? llr_ldg(Lh + o) : 0.f); };
+                auto val = [&](int o) { return AR::chan(livef ? llr_ldg(Lf + o, sc) : 0.f, liveh ? llr_ldg(Lh + o, sc) : 0.f); };
                 const float zero = AR::chan(0.f, 0.f);
                 float4 x1 = make_float4(zero, zero, zero, zero), x2 = x1;
                 x1.x = val(oa); x1.y = val(oa + 1); x2.x = val(op); x2.y = val(op + 1);
@@ -968,6 +970,10 @@ int nii_configure(Codec &c)
     B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
     B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
     B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
+    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
     g.enabled = 1;
     return B200DVB_OK;
 }
@@ -1008,7 +1014,7 @@ template <class LlrT> static void nii_start(const NiiArgs &A, bool fixed, bool t
     }
 }
 
-int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+int nii_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -1020,8 +1026,8 @@ int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long lon
     const int tile = fixed ? 2 * kTpfFrames : kTpfFrames;
     A.n_tiles = (B + tile - 1) / tile;
     A.n_llr = c.n_llr;
-    const int nq = f16 ? llr_row_q<__half>(c.n_llr) : llr_row_q<float>(c.n_llr);
-    A.vec4 = (c.N <= 256) && ((llr_stride * (f16 ? 2 : 4)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
+    const int nq = llr_row_q(fmt, c.n_llr);
+    A.vec4 = (c.N <= 256) && ((llr_stride * llr_bytes(fmt)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
              !c.opt_no_row_staging;
     if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
         const int pitch4 = ((nq + 6) & ~7) + 1;
@@ -1032,11 +1038,13 @@ int nii_launch_decode(const Codec &c, int B, const void *llr, bool f16, long lon
     A.sf_inner = (float)c.sf_inner; A.sf_last = (float)c.sf_last; A.tab = c.d_tab;
     A.sf_inner_q = (int)lrint(c.sf_inner * 64.0); A.sf_last_q = (int)lrint(c.sf_last * 64.0);   // Q6: 45 and 64 for 0.7 / 1.0
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters;
+    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
     A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
     const int grid = nii_grid(c, B);
-    if (f16) nii_start<__half>(A, fixed, c.opt_phase_timers != 0, grid, c.nii.smem_bytes, s);
-    else     nii_start<float>(A, fixed, c.opt_phase_timers != 0, grid, c.nii.smem_bytes, s);
+    const bool timed = c.opt_phase_timers != 0;
+    if (fmt == LlrFormat::F16)     nii_start<__half>(A, fixed, timed, grid, c.nii.smem_bytes, s);
+    else if (fmt == LlrFormat::I8) nii_start<int8_t>(A, fixed, timed, grid, c.nii.smem_bytes, s);
+    else                           nii_start<float>(A, fixed, timed, grid, c.nii.smem_bytes, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

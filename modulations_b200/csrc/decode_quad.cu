@@ -39,7 +39,7 @@ struct QuadArgs {
     double sf_inner, sf_last;
     const int16_t *tab;
     // full decode
-    const void *llr;      // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
+    const void *llr;      // [B][llr_stride] elements of the kernel's LlrT (float32, binary16 or int8)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
@@ -55,6 +55,7 @@ struct QuadArgs {
     // workspace
     double2 *Le1, *Le2, *Y;
     float *grec;          // geometry `grec`: [CTA][frame slot][rec_stride] branch-metric records
+    float llr_scale;      // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
 };
 
 // phase timers (SM cycles summed over CTAs): 0 prep, 1 recursion in (pass 1 + pass 2 to the
@@ -748,18 +749,18 @@ quad_kernel(const QuadArgs A)
                             const int src = second ? t_perm[k] : k;
                             const int oa = t_offA[src];
                             if (A.vec_ab) {
-                                const float2 v = llr_ldg2(Lf + oa);
+                                const float2 v = llr_ldg2(Lf + oa, A.llr_scale);
                                 sA[u] = v.x; sB[u] = v.y;
                             } else {
-                                sA[u] = llr_ldg(Lf + oa); sB[u] = llr_ldg(Lf + oa + 1);
+                                sA[u] = llr_ldg(Lf + oa, A.llr_scale); sB[u] = llr_ldg(Lf + oa + 1, A.llr_scale);
                             }
                             const int ow = t_oW[k], oy = t_oY[k];
                             if (A.vec_wy) {          // both parities present, adjacent and aligned to two elements
-                                const float2 v = llr_ldg2(Lf + ow);
+                                const float2 v = llr_ldg2(Lf + ow, A.llr_scale);
                                 pW[u] = v.x; pY[u] = v.y;
                             } else {
-                                if (ow >= 0) pW[u] = llr_ldg(Lf + ow);
-                                if (oy >= 0) pY[u] = llr_ldg(Lf + oy);
+                                if (ow >= 0) pW[u] = llr_ldg(Lf + ow, A.llr_scale);
+                                if (oy >= 0) pY[u] = llr_ldg(Lf + oy, A.llr_scale);
                             }
                             if (!first) La[u] = __ldcg(LePrev + (size_t)f * N + (second ? src : (int)t_inv[k]));
                         }
@@ -859,7 +860,7 @@ quad_kernel(const QuadArgs A)
                     const int oa = t_offA[j];
                     La[u] = __ldcg(Le2 + (size_t)f * N + t_inv[j]);
                     e1[u] = __ldcg(Le1 + (size_t)f * N + j);
-                    sA[u] = llr_ldg(Lf + oa); sB[u] = llr_ldg(Lf + oa + 1);
+                    sA[u] = llr_ldg(Lf + oa, A.llr_scale); sB[u] = llr_ldg(Lf + oa + 1, A.llr_scale);
                     if (A.ref_bits)
                         rb[u] = *reinterpret_cast<const uchar2 *>(A.ref_bits + (size_t)frame * 2 * N + 2 * j);
                 }
@@ -1021,13 +1022,17 @@ int quad_configure(Codec &c)
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
     int occ = 0;
     if (g.use_tmem) {
-        B2_CUDA(occupancy_both_formats(&occ, quad_kernel<false, true>, quad_kernel<false, true, false, __half>, g.threads, g.smem_bytes));
+        B2_CUDA(occupancy_all_formats(&occ, quad_kernel<false, true>, quad_kernel<false, true, false, __half>,
+                                      quad_kernel<false, true, false, int8_t>, g.threads, g.smem_bytes));
         if (occ > 1 && g.tmem_cols > 256) occ = 1;      // two CTAs must both get their TMEM columns
         if (occ > 512 / g.tmem_cols) occ = 512 / g.tmem_cols;
     } else {
-        B2_CUDA(occupancy_both_formats(&occ, quad_kernel<false, false>, quad_kernel<false, false, false, __half>, g.threads, g.smem_bytes));
+        B2_CUDA(occupancy_all_formats(&occ, quad_kernel<false, false>, quad_kernel<false, false, false, __half>,
+                                      quad_kernel<false, false, false, int8_t>, g.threads, g.smem_bytes));
     }
     if (occ < 1) return B200DVB_ENOSPEC;
     g.ctas_per_sm = occ;
@@ -1048,8 +1053,11 @@ int quad_configure(Codec &c)
         B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
         B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
         B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, int8_t>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
         int og = 0;
-        B2_CUDA(occupancy_both_formats(&og, quad_kernel<false, true, true>, quad_kernel<false, true, true, __half>, t.threads, t.smem_bytes));
+        B2_CUDA(occupancy_all_formats(&og, quad_kernel<false, true, true>, quad_kernel<false, true, true, __half>,
+                                      quad_kernel<false, true, true, int8_t>, t.threads, t.smem_bytes));
         if (og > 512 / t.tmem_cols) og = 512 / t.tmem_cols;
         if (og > 1) og = 1;
         if (og >= 1) { t.ctas_per_sm = og; c.geom_g = t; }
@@ -1107,7 +1115,7 @@ template <class LlrT> static void quad_start(const QuadArgs &A, const QuadGeom &
     else                 quad_kernel<false, false, false, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
 }
 
-int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+int launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                   uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                   void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -1121,8 +1129,8 @@ int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long ll
     A.n_groups = (B + G.frames - 1) / G.frames;
     A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters;
-    const uintptr_t pair_bytes = f16 ? 4 : 8;
+    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
+    const uintptr_t pair_bytes = 2 * llr_bytes(fmt);
     const bool even = (llr_stride % 2 == 0) && ((reinterpret_cast<uintptr_t>(llr) & (pair_bytes - 1)) == 0);
     A.vec_ab = even && c.vec_ab;
     A.vec_wy = even && c.vec_wy;
@@ -1130,8 +1138,9 @@ int launch_decode(const Codec &c, int B, const void *llr, bool f16, long long ll
     A.Le1 = reinterpret_cast<double2 *>(align256(ws));
     A.Le2 = A.Le1 + per; A.Y = A.Le2 + per;
     A.grec = reinterpret_cast<float *>(align256(A.Y + per));
-    if (f16) quad_start<__half>(A, G, grid, s);
-    else     quad_start<float>(A, G, grid, s);
+    if (fmt == LlrFormat::F16)     quad_start<__half>(A, G, grid, s);
+    else if (fmt == LlrFormat::I8) quad_start<int8_t>(A, G, grid, s);
+    else                           quad_start<float>(A, G, grid, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

@@ -53,13 +53,14 @@ struct TpfArgs {
     int B, iterations, n_tiles, n_llr, vec4;
     double sf_inner, sf_last;
     const int16_t *tab;
-    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32 or binary16)
+    const void *llr;                 // [B][llr_stride] elements of the kernel's LlrT (float32, binary16 or int8)
     long long llr_stride;
     int32_t *bits;
     uint32_t *packed;
     const uint8_t *ref_bits;
     unsigned long long *counters;
     unsigned char *ws;
+    float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
 };
 
 constexpr int kRingPairs = 4;        // pass-1 prefetch ring depth in step pairs (2 KB each: the whole beta-vector area)
@@ -631,6 +632,7 @@ tpf_kernel(const TpfArgs A)
     for (int tile = wg; tile < A.n_tiles; tile += gridDim.x * kTpfWarps) {
         const long long frame0 = (long long)tile * kTpfFrames;
         const long long t0 = TIMED ? clock64() : 0;
+        const float sc = A.llr_scale;                               // int8 input only (llr_f32)
         // ---- de-puncture + transpose the 16 frames' LLRs into [k][frame] (:466-487, :507-512).
         //      Each frame's row is pulled into the staging area with coalesced 16-byte loads
         //      (every line of the input is read exactly once), two frames in flight; the lanes
@@ -689,11 +691,11 @@ tpf_kernel(const TpfArgs A)
                     const int o2 = (short)(e.z & 0xffff), o3 = e.z >> 16;
                     float4 x1 = make_float4(0.f, 0.f, 0.f, 0.f), x2 = x1;
                     if (livef) {
-                        x1.x = llr_f32(row[oa]); x1.y = llr_f32(row[oa + 1]); x2.x = llr_f32(row[op]); x2.y = llr_f32(row[op + 1]);
-                        if (o0 >= 0) x1.z = llr_f32(row[o0]);
-                        if (o1 >= 0) x1.w = llr_f32(row[o1]);
-                        if (o2 >= 0) x2.z = llr_f32(row[o2]);
-                        if (o3 >= 0) x2.w = llr_f32(row[o3]);
+                        x1.x = llr_f32(row[oa], sc); x1.y = llr_f32(row[oa + 1], sc); x2.x = llr_f32(row[op], sc); x2.y = llr_f32(row[op + 1], sc);
+                        if (o0 >= 0) x1.z = llr_f32(row[o0], sc);
+                        if (o1 >= 0) x1.w = llr_f32(row[o1], sc);
+                        if (o2 >= 0) x2.z = llr_f32(row[o2], sc);
+                        if (o3 >= 0) x2.w = llr_f32(row[o3], sc);
                     }
                     if (k < N) {
                         st_ws(c.L1A + lpos(c, k, g0 + fr), x1);
@@ -717,12 +719,12 @@ tpf_kernel(const TpfArgs A)
                     const LlrT *Lf = static_cast<const LlrT *>(A.llr) + frame * A.llr_stride;
                     x1[fr] = make_float4(0.f, 0.f, 0.f, 0.f); x2[fr] = x1[fr];
                     if (frame < A.B) {
-                        x1[fr].x = llr_ldg(Lf + oa); x1[fr].y = llr_ldg(Lf + oa + 1);
-                        x2[fr].x = llr_ldg(Lf + op); x2[fr].y = llr_ldg(Lf + op + 1);
-                        if (o0 >= 0) x1[fr].z = llr_ldg(Lf + o0);
-                        if (o1 >= 0) x1[fr].w = llr_ldg(Lf + o1);
-                        if (o2 >= 0) x2[fr].z = llr_ldg(Lf + o2);
-                        if (o3 >= 0) x2[fr].w = llr_ldg(Lf + o3);
+                        x1[fr].x = llr_ldg(Lf + oa, sc); x1[fr].y = llr_ldg(Lf + oa + 1, sc);
+                        x2[fr].x = llr_ldg(Lf + op, sc); x2[fr].y = llr_ldg(Lf + op + 1, sc);
+                        if (o0 >= 0) x1[fr].z = llr_ldg(Lf + o0, sc);
+                        if (o1 >= 0) x1[fr].w = llr_ldg(Lf + o1, sc);
+                        if (o2 >= 0) x2[fr].z = llr_ldg(Lf + o2, sc);
+                        if (o3 >= 0) x2[fr].w = llr_ldg(Lf + o3, sc);
                     }
                 }
 #pragma unroll
@@ -881,6 +883,8 @@ int tpf_configure(Codec &c)
     B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     g.enabled = 1;
     return B200DVB_OK;
 }
@@ -916,7 +920,7 @@ template <class LlrT> static void tpf_start(const TpfArgs &A, bool timed, int gr
     else       tpf_kernel<false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
 }
 
-int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long long llr_stride, int32_t *bits,
+int tpf_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
                       uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
                       void *ws, size_t ws_bytes, cudaStream_t s)
 {
@@ -927,8 +931,8 @@ int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long lon
     A.n_tiles = (B + kTpfFrames - 1) / kTpfFrames;
     A.n_llr = c.n_llr;
     // whole rows by bulk copy: pitch and base 16-byte aligned, row fits half the staging area
-    const int nq = f16 ? llr_row_q<__half>(c.n_llr) : llr_row_q<float>(c.n_llr);
-    A.vec4 = (c.N <= 256) && ((llr_stride * (f16 ? 2 : 4)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
+    const int nq = llr_row_q(fmt, c.n_llr);
+    A.vec4 = (c.N <= 256) && ((llr_stride * llr_bytes(fmt)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
              !c.opt_no_row_staging;
     if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
         const int pitch4 = ((nq + 6) & ~7) + 1;
@@ -938,10 +942,12 @@ int tpf_launch_decode(const Codec &c, int B, const void *llr, bool f16, long lon
     }
     A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
     A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters;
+    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
     A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-    if (f16) tpf_start<__half>(A, c.opt_phase_timers != 0, tpf_grid(c, B), c.tpf.smem_bytes, s);
-    else     tpf_start<float>(A, c.opt_phase_timers != 0, tpf_grid(c, B), c.tpf.smem_bytes, s);
+    const bool timed = c.opt_phase_timers != 0;
+    if (fmt == LlrFormat::F16)     tpf_start<__half>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
+    else if (fmt == LlrFormat::I8) tpf_start<int8_t>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
+    else                           tpf_start<float>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

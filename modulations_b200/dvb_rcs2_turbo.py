@@ -197,18 +197,23 @@ class _CodecHandle:
         _lib.check(rc, "encode")
         return coded, circ
 
-    def decode(self, x, bits=None, packed=None, ref=None, counters=None, stream=None, ws=None):
-        """x float32 or float16 CUDA [B, >= n_llr] (row stride in elements taken from the tensor).  float16 goes to
-        b200dvb_decode_f16: the decode of its exact float32 widening, bit for bit."""
+    def decode(self, x, bits=None, packed=None, ref=None, counters=None, stream=None, ws=None, llr_scale=1.0):
+        """x float32, float16 or int8 CUDA [B, >= n_llr] (row stride in elements taken from the tensor).  float16 goes
+        to b200dvb_decode_f16: the decode of its exact float32 widening, bit for bit.  int8 goes to b200dvb_decode_i8:
+        the decode of float32(q) * float32(llr_scale), bit for bit; ``llr_scale`` is not read for other dtypes."""
         torch = _lib.torch_mod()
         B = x.shape[0]
         st = stream or self.stream()
         lib = _lib.load()
-        fn = lib.b200dvb_decode_f16 if x.dtype == torch.float16 else lib.b200dvb_decode
+        fn, scale = lib.b200dvb_decode, ()
+        if x.dtype == torch.float16:
+            fn = lib.b200dvb_decode_f16
+        elif x.dtype == torch.int8:
+            fn, scale = lib.b200dvb_decode_i8, (float(llr_scale),)
         with torch.cuda.device(self.device):
             buf, need = ws if ws is not None else self.workspace("decode", B, st)
             stride = x.stride(0) if B > 1 else x.shape[1]     # a length-1 axis may report stride 0
-            rc = fn(self.h, B, _lib.ptr(x), stride, _lib.ptr(bits), _lib.ptr(packed), _lib.ptr(ref),
+            rc = fn(self.h, B, _lib.ptr(x), stride, *scale, _lib.ptr(bits), _lib.ptr(packed), _lib.ptr(ref),
                     _lib.ptr(counters), _lib.ptr(buf), need, ctypes.c_void_p(st.cuda_stream))
         _lib.check(rc, "decode")
 
@@ -464,12 +469,14 @@ class DVBRCS2_Turbo:
         return self.encode_batch(bits[None, :self.k_info])[0].astype(np.int32)
 
     # -- decoder ------------------------------------------------------------
-    def decode_batch(self, llr, ref_bits=None, counters=None, out="bits"):
+    def decode_batch(self, llr, ref_bits=None, counters=None, out="bits", llr_scale=None):
         """llr [B, >= n_llr] float32 (numpy or CUDA torch) -> hard decisions.
 
         float16 input (``torch.float16`` or ``np.float16``) reaches the device as 16 bits and is decoded by the
-        binary16 path: fp16 in = decode of its exact float32 widening, bit for bit, in every mode and kernel.  Any
-        other dtype is converted to float32.
+        binary16 path: fp16 in = decode of its exact float32 widening, bit for bit, in every mode and kernel.
+        int8 input (``torch.int8`` or ``np.int8``) reaches the device as 8 bits: q is decoded as the float32 LLR
+        float32(q) * float32(llr_scale), bit for bit (``llr_scale`` defaults to 1.0; it must be finite and non-zero,
+        and is an error with any other dtype).  Any other dtype is converted to float32.
 
         out="bits": int32 [B, 2N] (reference layout); "packed": uint32 [B, ceil(2N/32)], bit i of a frame at
         word i//32, bit i%32; "none": nothing (error counting only).  ``ref_bits`` (anything reshapeable to
@@ -484,7 +491,9 @@ class DVBRCS2_Turbo:
         if not is_torch:
             llr = np.asarray(llr)
         half = llr.dtype == (torch.float16 if is_torch else np.float16)
-        x = _lib.to_device(llr, torch.float16 if half else torch.float32, h.device)
+        i8 = llr.dtype == (torch.int8 if is_torch else np.int8)
+        kw = _scale_kw(llr_scale, i8)
+        x = _lib.to_device(llr, torch.float16 if half else torch.int8 if i8 else torch.float32, h.device)
         if x.dim() == 1:
             x = x[None, :]
         if x.dim() != 2 or x.shape[1] < h.n_llr:
@@ -508,17 +517,19 @@ class DVBRCS2_Turbo:
                                          and counters.numel() >= 4 and counters.is_contiguous()
                                          and counters.device == h.device):
             raise ValueError("counters must be a contiguous CUDA int64/uint64 tensor with >= 4 elements on the codec's device")
-        h.decode(x, bits=bits, packed=packed, ref=ref, counters=counters)
+        h.decode(x, bits=bits, packed=packed, ref=ref, counters=counters, **kw)
         res = bits if out == "bits" else packed
         if res is not None and not is_torch:
             res = res.cpu().numpy()
         return res
 
-    def decode_batch_host(self, llr_host, out_host=None, chunk=None, out="bits"):
-        """End-to-end decode of HOST buffers: pinned ``llr_host`` float32 or float16 [B, >= n_llr] -> pinned ``out_host``.
+    def decode_batch_host(self, llr_host, out_host=None, chunk=None, out="bits", llr_scale=None):
+        """End-to-end decode of HOST buffers: pinned ``llr_host`` float32, float16 or int8 [B, >= n_llr] -> pinned
+        ``out_host``.
 
         float16 rows cross PCIe as 16 bits (half the bytes) and are decoded by the binary16 path: fp16 in = decode of
-        its exact float32 widening, bit for bit.
+        its exact float32 widening, bit for bit.  int8 rows cross as 8 bits (a quarter of the bytes) and q is decoded
+        as float32(q) * float32(llr_scale), bit for bit, as in ``decode_batch``.
 
         out="bits": int32 [B, 2N], the reference's layout (1 696 B per N=212 frame over PCIe);
         out="packed": int32 words [B, ceil(2N/32)], bit i of a frame at word i//32, bit i%32 (56 B per frame:
@@ -539,9 +550,10 @@ class DVBRCS2_Turbo:
             x = llr_host
         else:
             a = np.asarray(llr_host)
-            x = torch.from_numpy(np.ascontiguousarray(a, np.float16 if a.dtype == np.float16 else np.float32))
-        if x.dim() != 2 or x.shape[1] < h.n_llr or x.dtype not in (torch.float32, torch.float16):
-            raise IndexError(f"llr needs float32 or float16 shape [B, >= {h.n_llr}]")
+            x = torch.from_numpy(np.ascontiguousarray(a, a.dtype if a.dtype in (np.float16, np.int8) else np.float32))
+        kw = _scale_kw(llr_scale, x.dtype == torch.int8)
+        if x.dim() != 2 or x.shape[1] < h.n_llr or x.dtype not in (torch.float32, torch.float16, torch.int8):
+            raise IndexError(f"llr needs float32, float16 or int8 shape [B, >= {h.n_llr}]")
         B, width = x.shape
         wpf = (self.k_info + 31) // 32
         oshape, odtype = {"bits": ((self.k_info,), torch.int32), "packed": ((wpf,), torch.int32),
@@ -572,11 +584,11 @@ class DVBRCS2_Turbo:
             with torch.cuda.stream(streams[j]):
                 din[j][:n].copy_(x[lo:lo + n], non_blocking=True)
                 if out == "bits":
-                    h.decode(din[j][:n], bits=dout[j], stream=streams[j], ws=wss[j])
+                    h.decode(din[j][:n], bits=dout[j], stream=streams[j], ws=wss[j], **kw)
                 elif out == "packed":
-                    h.decode(din[j][:n], packed=dout[j], stream=streams[j], ws=wss[j])
+                    h.decode(din[j][:n], packed=dout[j], stream=streams[j], ws=wss[j], **kw)
                 else:
-                    h.decode(din[j][:n], packed=dpk[j], stream=streams[j], ws=wss[j])
+                    h.decode(din[j][:n], packed=dpk[j], stream=streams[j], ws=wss[j], **kw)
                     _unpack_bits_device(dpk[j][:n], dout[j][:n], self.k_info)
                 out_host[lo:lo + n].copy_(dout[j][:n], non_blocking=True)
                 done[j].record(streams[j])
@@ -615,6 +627,16 @@ class DVBRCS2_Turbo:
             hout.copy_(dbits, non_blocking=True)
             st.synchronize()
         return hout_np[0].copy()
+
+
+def _scale_kw(llr_scale, is_int8):
+    """_CodecHandle.decode keywords for the LLR dtype: int8 takes its scale (1.0 when not given); a scale given with
+    any other dtype is an error, not silently ignored."""
+    if not is_int8:
+        if llr_scale is not None:
+            raise ValueError("llr_scale applies to int8 LLRs only")
+        return {}
+    return {"llr_scale": 1.0 if llr_scale is None else float(llr_scale)}
 
 
 def _unpack_bits_device(packed, out_u8, k_info):

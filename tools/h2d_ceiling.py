@@ -4,11 +4,11 @@
 plain cudaMemcpyAsync on two streams and NO kernel, all ranks at once.  The aggregate is the most any
 host-buffer decode can reach on this box: e2e Gbit/s <= frames/s at the ceiling x 2N.
 
-    python tools/h2d_ceiling.py [FRAMES] [--llr-bytes 4|2]     (1 GPU)
+    python tools/h2d_ceiling.py [FRAMES] [--llr-bytes 4|2|1]   (1 GPU)
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/h2d_ceiling.py
 
---llr-bytes 2: the LLRs cross as float16 (decode_batch_host with a float16 buffer), half the H2D bytes; the default
-is float32.  Prints one JSON line per run (rank 0): per-direction GB/s per rank (min/max) and summed.
+--llr-bytes 2: the LLRs cross as float16 (decode_batch_host with a float16 buffer), half the H2D bytes; --llr-bytes 1:
+as int8 (an int8 buffer with llr_scale), a quarter; the default is float32.  Prints one JSON line per run (rank 0): per-direction GB/s per rank (min/max) and summed.
 """
 import argparse
 import json
@@ -24,7 +24,7 @@ def measure(frames, esz, dev, world):
     """{layout: ceiling figures} for `frames` frames per rank and step, LLRs of `esz` bytes; all ranks at once."""
     out = {}
     for label, d2h_per_frame in (("int32_bits", 2 * N * 4), ("packed_bits", ((2 * N + 31) // 32) * 4)):
-        hin = torch.empty((frames, N_LLR), dtype=torch.float32 if esz == 4 else torch.float16, pin_memory=True)
+        hin = torch.empty((frames, N_LLR), dtype={4: torch.float32, 2: torch.float16, 1: torch.int8}[esz], pin_memory=True)
         hout = torch.empty(frames * d2h_per_frame, dtype=torch.uint8, pin_memory=True)
         din = torch.empty_like(hin, device=dev)
         dout = torch.empty_like(hout, device=dev)
@@ -72,7 +72,8 @@ def measure(frames, esz, dev, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("frames", nargs="?", type=int, default=262144)
-    ap.add_argument("--llr-bytes", type=int, choices=(4, 2), default=4, help="bytes per LLR element: 4 float32, 2 float16")
+    ap.add_argument("--llr-bytes", type=int, choices=(4, 2, 1), default=4,
+                    help="bytes per LLR element: 4 float32, 2 float16, 1 int8")
     args = ap.parse_args()
     frames, esz = args.frames, args.llr_bytes
     rank = int(os.environ.get("RANK", "0"))
