@@ -151,13 +151,16 @@ int b200dvb_codec_create(int N, const int32_t *next_state_h, const int32_t *out_
     memcpy(c.out_W, out_W_h, sizeof c.out_W);
     memcpy(c.out_Y, out_Y_h, sizeof c.out_Y);
     circular_lut(next_state_h, N, c.circ_lut);
-    int rc = quad_configure(c);
-    if (rc != B200DVB_OK) { delete h; return rc; }
-    rc = tpf_configure(c);
-    if (rc != B200DVB_OK) { delete h; return rc; }
-    rc = nii_configure(c);
-    if (rc != B200DVB_OK) { delete h; return rc; }
-    rc = lat_configure(c);
+    // the device's SM count and shared-memory limit, read once for every decoder's geometry
+    int dev = 0, smem_optin = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&c.num_sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e != cudaSuccess) { set_cuda_error(e, "codec_create device attributes"); delete h; return B200DVB_ECUDA; }
+    int rc = quad_configure(c, smem_optin);
+    if (rc == B200DVB_OK) rc = tpf_configure(c, smem_optin);
+    if (rc == B200DVB_OK) rc = nii_configure(c, smem_optin);
+    if (rc == B200DVB_OK) rc = lat_configure(c, smem_optin);
     if (rc != B200DVB_OK) { delete h; return rc; }
     // stream offsets (depuncture order of dvb_rcs2_turbo.py:476-487)
     c.h_tab = (int16_t *)malloc(sizeof(int16_t) * 7 * N);
@@ -181,7 +184,7 @@ int b200dvb_codec_create(int N, const int32_t *next_state_h, const int32_t *out_
         }
     }
     if (idx > 32767) { free(c.h_tab); delete h; return B200DVB_ENOSPEC; }
-    cudaError_t e = cudaMalloc(&c.d_tab, sizeof(int16_t) * 7 * N);
+    e = cudaMalloc(&c.d_tab, sizeof(int16_t) * 7 * N);
     if (e == cudaSuccess)
         e = cudaMemcpy(c.d_tab, c.h_tab, sizeof(int16_t) * 7 * N, cudaMemcpyHostToDevice);
     if (e != cudaSuccess) {
@@ -261,12 +264,25 @@ static bool use_tpf(const Codec &c, int B)
     return !(c.geom.frames <= 32 && B <= quad_wave);
 }
 
+// The one decision of which kernel decodes a batch: both the workspace query and the launch switch on it.  The
+// non-parity modes have one kernel.
+enum class Decoder { NII, LAT, TPF, QUAD };
+static Decoder decoder_for(const Codec &c, int B)
+{
+    if (c.opt_mode != B200DVB_MODE_PARITY) return Decoder::NII;
+    if (use_lat(c, B)) return Decoder::LAT;
+    return use_tpf(c, B) ? Decoder::TPF : Decoder::QUAD;
+}
+
 size_t b200dvb_decode_workspace_bytes(b200dvb_codec_t codec, int B)
 {
     if (!codec || B <= 0) return 0;
-    if (codec->c.opt_mode != B200DVB_MODE_PARITY) return nii_workspace_bytes(codec->c, B);
-    if (use_lat(codec->c, B)) return 256;                            // the whole frame lives in shared memory
-    return use_tpf(codec->c, B) ? tpf_workspace_bytes(codec->c, B) : decode_workspace_bytes(codec->c, B);
+    switch (decoder_for(codec->c, B)) {
+    case Decoder::NII: return nii_workspace_bytes(codec->c, B);
+    case Decoder::LAT: return 256;                                   // the whole frame lives in shared memory
+    case Decoder::TPF: return tpf_workspace_bytes(codec->c, B);
+    default: return quad_workspace_bytes(codec->c, B);
+    }
 }
 
 int b200dvb_codec_set_option(b200dvb_codec_t codec, int option, int value)
@@ -299,16 +315,15 @@ static int decode_any(b200dvb_codec_t codec, int B, const void *llr, LlrFormat f
 {
     if (!codec || B < 0 || !llr || (B && !workspace)) return B200DVB_EINVAL;
     if (llr_stride < codec->c.n_llr) return B200DVB_EINVAL;
-    if (codec->c.opt_mode != B200DVB_MODE_PARITY)
-        return nii_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters,
-                                 workspace, workspace_bytes, (cudaStream_t)stream);
-    if (use_lat(codec->c, B))
-        return lat_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, (cudaStream_t)stream);
-    if (use_tpf(codec->c, B))
-        return tpf_launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters,
-                                 workspace, workspace_bytes, (cudaStream_t)stream);
-    return launch_decode(codec->c, B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, workspace,
-                         workspace_bytes, (cudaStream_t)stream);
+    if (B == 0) return B200DVB_OK;
+    const DecodeIo io{B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, workspace, workspace_bytes,
+                      (cudaStream_t)stream};
+    switch (decoder_for(codec->c, B)) {
+    case Decoder::NII: return nii_launch_decode(codec->c, io);
+    case Decoder::LAT: return lat_launch_decode(codec->c, io);
+    case Decoder::TPF: return tpf_launch_decode(codec->c, io);
+    default: return quad_launch_decode(codec->c, io);
+    }
 }
 
 int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr_stride,
@@ -472,7 +487,7 @@ int b200dvb_hard_demod(b200dvb_modem_t modem, size_t n_sym, const void *iq, int 
 int b200dvb_debug_phase_cycles(double *out8_h, int reset)
 {
     if (!out8_h) return B200DVB_EINVAL;
-    return read_phase_cycles(out8_h, reset);
+    return quad_read_phase_cycles(out8_h, reset);
 }
 
 int b200dvb_debug_tpf_cycles(double *out8_h, int reset)

@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 #include <stddef.h>
+#include <type_traits>
 #include "../../include/b200dvb.h"
 
 namespace b200dvb {
@@ -15,7 +16,24 @@ namespace b200dvb {
 // widened exactly, int8 q becomes the IEEE product q * scale (the library builds with --fmad=false).  Everything after
 // the load is the float32 kernel's, fed the same float32 values.  The float32 and binary16 overloads ignore the scale.
 enum class LlrFormat { F32, F16, I8 };
-inline int llr_bytes(LlrFormat f) { return f == LlrFormat::F32 ? 4 : f == LlrFormat::F16 ? 2 : 1; }
+// f(L{}) with L the element type of format fmt: the one place that maps a format to its type
+template <class F> inline auto with_llr_type(LlrFormat fmt, F &&f)
+{
+    switch (fmt) {
+    case LlrFormat::F16: return f(__half{});
+    case LlrFormat::I8: return f(int8_t{});
+    default: return f(float{});
+    }
+}
+// f(L{}) for every element type, in turn while it returns B200DVB_OK; the first other code is the result
+template <class F> inline int for_each_llr_type(F &&f)
+{
+    int rc = f(float{});
+    if (rc == B200DVB_OK) rc = f(__half{});
+    if (rc == B200DVB_OK) rc = f(int8_t{});
+    return rc;
+}
+inline int llr_bytes(LlrFormat f) { return with_llr_type(f, [](auto t) { return (int)sizeof(t); }); }
 __device__ __forceinline__ float llr_f32(float x, float) { return x; }
 __device__ __forceinline__ float llr_f32(__half x, float) { return __half2float(x); }
 __device__ __forceinline__ float llr_f32(int8_t x, float s) { return __fmul_rn((float)x, s); }
@@ -35,20 +53,7 @@ template <class L> __host__ __device__ __forceinline__ int llr_row_q(int n)
 }
 inline int llr_row_q(LlrFormat f, int n)
 {
-    return f == LlrFormat::F32 ? llr_row_q<float>(n) : f == LlrFormat::F16 ? llr_row_q<__half>(n) : llr_row_q<int8_t>(n);
-}
-// CTAs per SM that every element-format instance of a kernel reaches: one geometry (frames per wave, grid) serves
-// float32, binary16 and int8 input, so it must fit the one with the largest footprint
-template <class K32, class K16, class K8>
-inline cudaError_t occupancy_all_formats(int *occ, K32 k32, K16 k16, K8 k8, int threads, size_t smem)
-{
-    int a = 0, b = 0, c = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k32, threads, smem);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k16, threads, smem);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, k8, threads, smem);
-    *occ = a < b ? a : b;
-    if (c < *occ) *occ = c;
-    return e;
+    return with_llr_type(f, [n](auto t) { return llr_row_q<decltype(t)>(n); });
 }
 
 // ---- error plumbing --------------------------------------------------------
@@ -61,6 +66,39 @@ void set_cuda_error(cudaError_t e, const char *where);
             return B200DVB_ECUDA;                                         \
         }                                                                 \
     } while (0)
+// a B200DVB_* code other than B200DVB_OK is returned to the caller as it is
+#define B2_CHECK(call)                                                    \
+    do {                                                                  \
+        const int rc__ = (call);                                          \
+        if (rc__ != B200DVB_OK) return rc__;                              \
+    } while (0)
+
+// CTAs per SM that every element-format instance of a kernel reaches (kernel_of(L{}) is the instance for element type
+// L): one geometry (frames per wave, grid) serves float32, binary16 and int8 input, so it must fit the one with the
+// largest footprint
+template <class K> inline int occupancy_all_formats(int *occ, K kernel_of, int threads, size_t smem)
+{
+    *occ = 1 << 30;
+    return for_each_llr_type([&](auto t) {
+        int n = 0;
+        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel_of(t), threads, smem));
+        if (n < *occ) *occ = n;
+        return B200DVB_OK;
+    });
+}
+
+// a kernel's eight per-phase cycle counters (a __device__ unsigned long long[8]) -> out_h; reset: zero them
+template <class Sym> int read_phase_cycles(const Sym &counters, double *out_h, int reset)
+{
+    unsigned long long h[8];
+    B2_CUDA(cudaMemcpyFromSymbol(h, counters, sizeof h));
+    for (int i = 0; i < 8; ++i) out_h[i] = (double)h[i];
+    if (reset) {
+        unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+        B2_CUDA(cudaMemcpyToSymbol(counters, z, sizeof z));
+    }
+    return B200DVB_OK;
+}
 
 constexpr int kMaxN = 2048;
 
@@ -94,6 +132,11 @@ struct QuadGeom {
 constexpr int kTpfFrames = 16;      // frames per warp: lanes 0-15 run alpha, lanes 16-31 beta of the same frames
 constexpr int kTpfWarps = 4;        // one warp per SM sub-partition, each with its own TMEM lane quadrant
 constexpr int kTpfWin = 4;          // checkpoint spacing / recompute window (steps)
+constexpr int kRingPairs = 4;       // prefetch ring depth of the "in" pass in step pairs (2 KB each: the whole beta-vector area)
+// per-warp staging area: [0, 8K) beta vectors of the current window, [kTpfWin][4][32] float4 (the prefetch ring of the
+// "in" pass, 6 KB, aliases it); [8K, 10K) Z slot; [10K, 12K) X slot
+constexpr int kStageBytes = 12288;
+constexpr int kRowFloats = kStageBytes / 8;   // transposition: two frame rows of up to 1536 LLRs each share the staging area
 
 struct TpfGeom {
     int enabled;      // this codec is decoded by the thread-per-frame kernel
@@ -145,34 +188,62 @@ struct Modem {
     double h_table[512];
 };
 
-// launchers (each returns a B200DVB_* code)
-// llr: elements of format fmt (llr_stride in elements); llr_scale multiplies int8 elements and is unused otherwise
-int launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                  uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                  void *ws, size_t ws_bytes, cudaStream_t s);
+// One decode call (b200dvb_decode / _f16 / _i8, B > 0): llr holds B rows of elements of format fmt, llr_stride elements
+// apart; llr_scale multiplies int8 elements and is unused otherwise.  bits, packed, ref_bits and counters may be NULL.
+struct DecodeIo {
+    int B;
+    const void *llr;
+    LlrFormat fmt;
+    float llr_scale;
+    long long llr_stride;
+    int32_t *bits;
+    uint32_t *packed;
+    const uint8_t *ref_bits;
+    unsigned long long *counters;
+    void *ws;
+    size_t ws_bytes;
+    cudaStream_t stream;
+};
+
+// the members every decode kernel's argument struct shares; sf_inner / sf_last where the struct keeps them in float64
+template <class Args> inline void fill_decode_args(Args &A, const Codec &c, const DecodeIo &io)
+{
+    A.B = io.B; A.iterations = c.iterations; A.tab = c.d_tab;
+    A.llr = io.llr; A.llr_stride = io.llr_stride; A.llr_scale = io.llr_scale;
+    A.bits = io.bits; A.packed = io.packed; A.ref_bits = io.ref_bits; A.counters = io.counters;
+    if constexpr (std::is_same<decltype(A.sf_inner), double>::value) { A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; }
+}
+
+// launchers and configuration (each returns a B200DVB_* code).  *_configure: smem_optin is the device's
+// sharedMemPerBlockOptin, and c.num_sms is set
+int quad_configure(Codec &c, size_t smem_optin);
+int quad_launch_decode(const Codec &c, const DecodeIo &io);
 int launch_siso(const Codec &c, int B, const float *Lc_A, const float *Lc_B, const float *Lc_W,
                 const float *Lc_Y, const double *La_A, const double *La_B, double sf,
                 double *Le_A, double *Le_B, void *ws, size_t ws_bytes, cudaStream_t s);
-size_t decode_workspace_bytes(const Codec &c, int B);
+size_t quad_workspace_bytes(const Codec &c, int B);
 size_t siso_workspace_bytes(const Codec &c, int B);
-int quad_configure(Codec &c);
-int tpf_configure(Codec &c);
-int tpf_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                      uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                      void *ws, size_t ws_bytes, cudaStream_t s);
+int quad_read_phase_cycles(double *out_h, int reset);
+int tpf_configure(Codec &c, size_t smem_optin);
+int tpf_launch_decode(const Codec &c, const DecodeIo &io);
 size_t tpf_workspace_bytes(const Codec &c, int B);
 int tpf_read_phase_cycles(double *out_h, int reset);
-int lat_configure(Codec &c);
-int lat_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits, uint32_t *packed,
-                      const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s);
-int nii_configure(Codec &c);
-int nii_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                      uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                      void *ws, size_t ws_bytes, cudaStream_t s);
+int nii_configure(Codec &c, size_t smem_optin);
+int nii_launch_decode(const Codec &c, const DecodeIo &io);
 size_t nii_workspace_bytes(const Codec &c, int B);
 int nii_read_phase_cycles(double *out_h, int reset);
+int lat_configure(Codec &c, size_t smem_optin);
+int lat_launch_decode(const Codec &c, const DecodeIo &io);
 int lat_read_phase_cycles(double *out_h, int reset);
-int read_phase_cycles(double *out_h, int reset);
+
+// host geometry of the thread-per-frame family (decode_tpf.cu: parity mode tpf; decode_nii.cu: nii / nii16)
+// g for N couples, left disabled (g.enabled = 0) when N does not fit.  y_cols: spare TMEM columns per lane that park the
+// window's Y; hdr_bytes: shared memory between the interleaver tables and the records; ext_bytes: bytes per frame and
+// step of each of Le, LeF and Y in the workspace; with_init: the workspace also keeps the boundary metrics (nii)
+void tpf_family_geometry(TpfGeom &g, int N, int y_cols, size_t hdr_bytes, size_t ext_bytes, bool with_init, size_t smem_optin);
+int tpf_family_grid(const Codec &c, int B, int tile);   // CTAs for B frames, `tile` frames per warp
+size_t tpf_family_workspace_bytes(const Codec &c, const TpfGeom &g, int B, int tile);
+int tpf_family_row_staging(const Codec &c, const TpfGeom &g, const DecodeIo &io);   // the kernel's `vec4`
 
 int launch_encode(const Codec &c, int B, const uint8_t *info, uint8_t *coded, uint8_t *circ,
                   cudaStream_t s);

@@ -325,17 +325,7 @@ lat_kernel(const LatArgs A)
 
 }  // namespace
 
-int lat_read_phase_cycles(double *out_h, int reset)
-{
-    unsigned long long h[8];
-    B2_CUDA(cudaMemcpyFromSymbol(h, g_lat_cycles, sizeof h));
-    for (int i = 0; i < 8; ++i) out_h[i] = (double)h[i];
-    if (reset) {
-        unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        B2_CUDA(cudaMemcpyToSymbol(g_lat_cycles, z, sizeof z));
-    }
-    return B200DVB_OK;
-}
+int lat_read_phase_cycles(double *out_h, int reset) { return read_phase_cycles(g_lat_cycles, out_h, reset); }
 
 static int g_lat_warm = 0;         // 0: lat_warm_for(N)
 void set_lat_warm(int v) { g_lat_warm = v; }
@@ -346,78 +336,56 @@ static size_t lat_smem(int N, bool pad)
     return (((size_t)4 * N + 15) / 16) * 16 + (size_t)N * (16 + 16 + 16 + 16 + 16) + (size_t)(N + 2) * rs * 4 +
            (size_t)N * cs * 4 + (size_t)(N + 1) * cs * 4 + (size_t)((2 * N + 31) / 32) * 4 + 64;
 }
-size_t lat_smem_bytes(int N) { return lat_smem(N, false); }
 
-static size_t lat_cap()
+static size_t lat_cap(size_t smem_optin)
 {
-    int dev = 0;
-    cudaDeviceProp prop;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaGetDeviceProperties(&prop, dev) != cudaSuccess) return 0;
     cudaFuncAttributes fa;
     if (cudaFuncGetAttributes(&fa, lat_kernel<false, false, float>) != cudaSuccess) return 0;   // every instance has the same static words
-    return (size_t)prop.sharedMemPerBlockOptin - fa.sharedSizeBytes;   // the static words count against the limit
+    return smem_optin - fa.sharedSizeBytes;                        // the static words count against the limit
 }
 
-int lat_configure(Codec &c)
+int lat_configure(Codec &c, size_t smem_optin)
 {
     c.lat_enabled = 0;
-    int dev = 0;
-    cudaDeviceProp prop;
-    B2_CUDA(cudaGetDevice(&dev));
-    B2_CUDA(cudaGetDeviceProperties(&prop, dev));
-    const size_t cap = lat_cap();
+    const size_t cap = lat_cap(smem_optin);
     if (lat_smem(c.N, false) > cap) return B200DVB_OK;
     c.lat_pad = lat_smem(c.N, true) <= cap;
     const size_t need = lat_smem(c.N, c.lat_pad != 0);
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CHECK(for_each_llr_type([&](auto t) {
+        using L = decltype(t);
+        B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(lat_kernel<false, true, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(lat_kernel<true, true, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        return B200DVB_OK;
+    }));
     int occ = 0;
-    if (c.lat_pad) B2_CUDA(occupancy_all_formats(&occ, lat_kernel<false, true, float>, lat_kernel<false, true, __half>,
-                                                 lat_kernel<false, true, int8_t>, kLatThreads, need));
-    else           B2_CUDA(occupancy_all_formats(&occ, lat_kernel<false, false, float>, lat_kernel<false, false, __half>,
-                                                 lat_kernel<false, false, int8_t>, kLatThreads, need));
+    if (c.lat_pad) B2_CHECK(occupancy_all_formats(&occ, [](auto t) { return lat_kernel<false, true, decltype(t)>; }, kLatThreads, need));
+    else           B2_CHECK(occupancy_all_formats(&occ, [](auto t) { return lat_kernel<false, false, decltype(t)>; }, kLatThreads, need));
     if (occ < 1) return B200DVB_OK;
     c.lat_enabled = 1;
-    c.lat_frames_per_wave = (occ < 2 ? occ : 2) * prop.multiProcessorCount;   // at most two CTAs per SM
+    c.lat_frames_per_wave = (occ < 2 ? occ : 2) * c.num_sms;     // at most two CTAs per SM
     return B200DVB_OK;
 }
 
-template <class LlrT> static void lat_start(const LatArgs &A, bool pad, bool timed, int grid, size_t smem, cudaStream_t s)
+int lat_launch_decode(const Codec &c, const DecodeIo &io)
 {
-    if (pad) {
-        if (timed) lat_kernel<true, true, LlrT><<<grid, kLatThreads, smem, s>>>(A);
-        else       lat_kernel<false, true, LlrT><<<grid, kLatThreads, smem, s>>>(A);
-    } else {
-        if (timed) lat_kernel<true, false, LlrT><<<grid, kLatThreads, smem, s>>>(A);
-        else       lat_kernel<false, false, LlrT><<<grid, kLatThreads, smem, s>>>(A);
-    }
-}
-
-int lat_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits, uint32_t *packed,
-                      const uint8_t *ref_bits, unsigned long long *counters, cudaStream_t s)
-{
-    if (B == 0) return B200DVB_OK;
     LatArgs A{};
-    A.N = c.N; A.B = B; A.iterations = c.iterations; A.n_llr = c.n_llr; A.num_sms = c.num_sms; A.warm = g_lat_warm > 0 ? g_lat_warm : lat_warm_for(c.N);
-    A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
-    A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed; A.ref_bits = ref_bits; A.counters = counters;
-    A.llr_scale = llr_scale;
-    const int grid = B < c.lat_frames_per_wave ? B : c.lat_frames_per_wave;
+    fill_decode_args(A, c, io);
+    A.N = c.N; A.n_llr = c.n_llr; A.num_sms = c.num_sms; A.warm = g_lat_warm > 0 ? g_lat_warm : lat_warm_for(c.N);
+    const int grid = io.B < c.lat_frames_per_wave ? io.B : c.lat_frames_per_wave;
     const size_t smem = lat_smem(c.N, c.lat_pad != 0);
     const bool pad = c.lat_pad != 0, timed = c.opt_phase_timers != 0;
-    if (fmt == LlrFormat::F16)     lat_start<__half>(A, pad, timed, grid, smem, s);
-    else if (fmt == LlrFormat::I8) lat_start<int8_t>(A, pad, timed, grid, smem, s);
-    else                           lat_start<float>(A, pad, timed, grid, smem, s);
+    with_llr_type(io.fmt, [&](auto t) {
+        using L = decltype(t);
+        if (pad) {
+            if (timed) lat_kernel<true, true, L><<<grid, kLatThreads, smem, io.stream>>>(A);
+            else       lat_kernel<false, true, L><<<grid, kLatThreads, smem, io.stream>>>(A);
+        } else {
+            if (timed) lat_kernel<true, false, L><<<grid, kLatThreads, smem, io.stream>>>(A);
+            else       lat_kernel<false, false, L><<<grid, kLatThreads, smem, io.stream>>>(A);
+        }
+    });
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

@@ -98,11 +98,6 @@ struct ArS16 {
 };
 
 constexpr int kW = kTpfWin;
-constexpr int kRingPairs = 4;        // prefetch ring depth of the "in" pass in step pairs (2 KB each)
-// per-warp staging area: [0, 8K) beta vectors of the current window, [kW][4][32] float4 (the prefetch ring of the
-// "in" pass aliases it); [8K, 10K) Z slot; [10K, 12K) X slot
-constexpr int kStageBytes = 12288;
-constexpr int kRowFloats = kStageBytes / 8;
 constexpr int kHdrBytes = 64 + kTpfWarps * kRingPairs * 8;   // after the tables: slots, one mbarrier per warp, kRingPairs ring mbarriers per warp
 
 // phase timers (SM cycles summed over warps): 0 transpose-in, 1 "in" pass (+prep), 2 boundary load/store + crossing,
@@ -929,122 +924,52 @@ nii_kernel(const NiiArgs A)
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-int nii_configure(Codec &c)
+int nii_configure(Codec &c, size_t smem_optin)
 {
-    TpfGeom &g = c.nii;
-    g = TpfGeom{};
-    const int N = c.N;
-    if (N < 16 || (N % 4) != 0) return B200DVB_OK;
-    const int M = N / 2;
-    int T = M < 64 ? M : 64;
-    while (T > 0 && (((M - T) % kW) != 0 || 8 * T + 2 * kW > 512)) --T;   // windows must not straddle TMEM / smem; Y columns
-    if (T < kW) return B200DVB_OK;
-    g.N = N; g.M = M; g.T = T; g.mid = N - 2 * T;
-    g.nfull = M / kW; g.rag = M % kW; g.nslots = g.nfull + (g.rag ? 1 : 0);
-    g.tmem_cols = 32;
-    while (g.tmem_cols < 8 * T + 2 * kW) g.tmem_cols *= 2;        // records + the window's Y
-    if (g.tmem_cols > 512) return B200DVB_OK;
-    const size_t tab_bytes = ((size_t)2 * N * 2 + 15) / 16 * 16;
-    g.smem_bytes = tab_bytes + kHdrBytes + (size_t)kTpfWarps * g.mid * 2 * 16 * sizeof(float4) + (size_t)kTpfWarps * kStageBytes;
-    int dev = 0;
-    cudaDeviceProp prop;
-    B2_CUDA(cudaGetDevice(&dev));
-    B2_CUDA(cudaGetDeviceProperties(&prop, dev));
-    if (g.smem_bytes > (size_t)prop.sharedMemPerBlockOptin) return B200DVB_OK;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    g.off_l1 = take((size_t)N * 16 * sizeof(float4));
-    g.off_l2 = take((size_t)N * 16 * sizeof(float4));
-    g.off_le = take((size_t)N * 16 * sizeof(float2));
-    g.off_lef = take((size_t)N * 16 * sizeof(float2));
-    g.off_y = take((size_t)(N / 2) * 16 * sizeof(float4));
-    g.off_ck = take((size_t)g.nslots * 4 * 32 * sizeof(float4));
-    g.off_init = take((size_t)2 * 4 * 32 * sizeof(float4));
-    g.ws_per_warp = off;
-    const int smax = (int)prop.sharedMemPerBlockOptin;
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax));
-    g.enabled = 1;
-    return B200DVB_OK;
+    tpf_family_geometry(c.nii, c.N, 2 * kW, kHdrBytes, sizeof(float2), true, smem_optin);
+    if (!c.nii.enabled) return B200DVB_OK;
+    return for_each_llr_type([&](auto t) {
+        using L = decltype(t);
+        B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArF32, true, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        B2_CUDA(cudaFuncSetAttribute(nii_kernel<ArS16, true, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        return B200DVB_OK;
+    });
 }
 
-int nii_read_phase_cycles(double *out_h, int reset)
-{
-    unsigned long long h[8];
-    B2_CUDA(cudaMemcpyFromSymbol(h, g_nii_cycles, sizeof h));
-    for (int i = 0; i < 8; ++i) out_h[i] = (double)h[i];
-    if (reset) {
-        unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        B2_CUDA(cudaMemcpyToSymbol(g_nii_cycles, z, sizeof z));
-    }
-    return B200DVB_OK;
-}
+int nii_read_phase_cycles(double *out_h, int reset) { return read_phase_cycles(g_nii_cycles, out_h, reset); }
 
-static int nii_grid(const Codec &c, int B)
-{
-    const int tile = c.opt_mode == B200DVB_MODE_NII16 ? 2 * kTpfFrames : kTpfFrames;
-    const int tiles = (B + tile - 1) / tile;
-    const int ctas = (tiles + kTpfWarps - 1) / kTpfWarps;
-    return ctas < c.num_sms ? ctas : c.num_sms;
-}
+static int nii_tile(const Codec &c) { return c.opt_mode == B200DVB_MODE_NII16 ? 2 * kTpfFrames : kTpfFrames; }
 
-size_t nii_workspace_bytes(const Codec &c, int B)
-{
-    return (size_t)nii_grid(c, B) * kTpfWarps * c.nii.ws_per_warp + 256;
-}
+size_t nii_workspace_bytes(const Codec &c, int B) { return tpf_family_workspace_bytes(c, c.nii, B, nii_tile(c)); }
 
-template <class LlrT> static void nii_start(const NiiArgs &A, bool fixed, bool timed, int grid, size_t smem, cudaStream_t s)
+int nii_launch_decode(const Codec &c, const DecodeIo &io)
 {
-    if (fixed) {
-        if (timed) nii_kernel<ArS16, true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
-        else       nii_kernel<ArS16, false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
-    } else {
-        if (timed) nii_kernel<ArF32, true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
-        else       nii_kernel<ArF32, false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
-    }
-}
-
-int nii_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                      uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                      void *ws, size_t ws_bytes, cudaStream_t s)
-{
-    if (B == 0) return B200DVB_OK;
-    if (ws_bytes < nii_workspace_bytes(c, B)) return B200DVB_ENOMEM;
+    if (io.ws_bytes < nii_workspace_bytes(c, io.B)) return B200DVB_ENOMEM;
     NiiArgs A{};
-    A.g = c.nii; A.B = B; A.iterations = c.iterations;
+    fill_decode_args(A, c, io);
+    A.g = c.nii;
     const bool fixed = c.opt_mode == B200DVB_MODE_NII16;
-    const int tile = fixed ? 2 * kTpfFrames : kTpfFrames;
-    A.n_tiles = (B + tile - 1) / tile;
+    A.n_tiles = (io.B + nii_tile(c) - 1) / nii_tile(c);
     A.n_llr = c.n_llr;
-    const int nq = llr_row_q(fmt, c.n_llr);
-    A.vec4 = (c.N <= 256) && ((llr_stride * llr_bytes(fmt)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
-             !c.opt_no_row_staging;
-    if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
-        const int pitch4 = ((nq + 6) & ~7) + 1;
-        const int rec_bytes = c.nii.mid * 2 * 16 * (int)sizeof(float4);
-        const int avail = rec_bytes > kStageBytes ? rec_bytes : kStageBytes - c.N * 16;
-        if (avail / (pitch4 * 16) < 2) A.vec4 = 0;
-    }
-    A.sf_inner = (float)c.sf_inner; A.sf_last = (float)c.sf_last; A.tab = c.d_tab;
+    A.vec4 = tpf_family_row_staging(c, c.nii, io);
+    A.sf_inner = (float)c.sf_inner; A.sf_last = (float)c.sf_last;
     A.sf_inner_q = (int)lrint(c.sf_inner * 64.0); A.sf_last_q = (int)lrint(c.sf_last * 64.0);   // Q6: 45 and 64 for 0.7 / 1.0
-    A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
-    A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-    const int grid = nii_grid(c, B);
+    A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(io.ws) + 255) & ~(uintptr_t)255);
+    const int grid = tpf_family_grid(c, io.B, nii_tile(c));
+    const size_t smem = c.nii.smem_bytes;
     const bool timed = c.opt_phase_timers != 0;
-    if (fmt == LlrFormat::F16)     nii_start<__half>(A, fixed, timed, grid, c.nii.smem_bytes, s);
-    else if (fmt == LlrFormat::I8) nii_start<int8_t>(A, fixed, timed, grid, c.nii.smem_bytes, s);
-    else                           nii_start<float>(A, fixed, timed, grid, c.nii.smem_bytes, s);
+    with_llr_type(io.fmt, [&](auto t) {
+        using L = decltype(t);
+        if (fixed) {
+            if (timed) nii_kernel<ArS16, true, L><<<grid, kTpfWarps * 32, smem, io.stream>>>(A);
+            else       nii_kernel<ArS16, false, L><<<grid, kTpfWarps * 32, smem, io.stream>>>(A);
+        } else {
+            if (timed) nii_kernel<ArF32, true, L><<<grid, kTpfWarps * 32, smem, io.stream>>>(A);
+            else       nii_kernel<ArF32, false, L><<<grid, kTpfWarps * 32, smem, io.stream>>>(A);
+        }
+    });
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

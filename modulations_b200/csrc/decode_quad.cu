@@ -948,7 +948,7 @@ static size_t quad_smem_bytes(const QuadGeom &g)
     return tab + fl * 4 + 68 * 4;
 }
 
-int quad_configure(Codec &c)
+int quad_configure(Codec &c, size_t smem_optin)
 {
     QuadGeom &g = c.geom;
     const int N = c.N;
@@ -964,16 +964,11 @@ int quad_configure(Codec &c)
     int ck = (g.nckA + g.nckB) * 16;
     if ((ck % 32) == 0) ck += 16;                   // == 16 (mod 32)
     g.ck_stride = ck;
-    int dev = 0;
-    cudaDeviceProp prop;
-    B2_CUDA(cudaGetDevice(&dev));
-    B2_CUDA(cudaGetDeviceProperties(&prop, dev));
-    c.num_sms = prop.multiProcessorCount;
     // One CTA per SM: `groups` pairs of (alpha warp, beta warp), 8 frames per pair, all warps
     // in the same phase so they share the instruction cache.  Two placements of the recursion
     // checkpoints are tried and the one that keeps more frames resident wins: shared memory
     // (up to 7 groups when N is small) or tensor memory (up to 4 groups: one per lane quadrant).
-    const size_t cap = (size_t)prop.sharedMemPerBlockOptin;
+    const size_t cap = smem_optin;
     const int want_groups = kMaxGroups;
     QuadGeom best{};
     best.frames = 0;
@@ -1016,23 +1011,21 @@ int quad_configure(Codec &c)
             while (g.tmem_cols < need) g.tmem_cols *= 2;
         }
     }
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));   // SISO (float32)
     B2_CUDA(cudaFuncSetAttribute(quad_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-    B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+    B2_CHECK(for_each_llr_type([&](auto t) {
+        using L = decltype(t);
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, false, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+        return B200DVB_OK;
+    }));
     int occ = 0;
     if (g.use_tmem) {
-        B2_CUDA(occupancy_all_formats(&occ, quad_kernel<false, true>, quad_kernel<false, true, false, __half>,
-                                      quad_kernel<false, true, false, int8_t>, g.threads, g.smem_bytes));
+        B2_CHECK(occupancy_all_formats(&occ, [](auto t) { return quad_kernel<false, true, false, decltype(t)>; }, g.threads, g.smem_bytes));
         if (occ > 1 && g.tmem_cols > 256) occ = 1;      // two CTAs must both get their TMEM columns
         if (occ > 512 / g.tmem_cols) occ = 512 / g.tmem_cols;
     } else {
-        B2_CUDA(occupancy_all_formats(&occ, quad_kernel<false, false>, quad_kernel<false, false, false, __half>,
-                                      quad_kernel<false, false, false, int8_t>, g.threads, g.smem_bytes));
+        B2_CHECK(occupancy_all_formats(&occ, [](auto t) { return quad_kernel<false, false, false, decltype(t)>; }, g.threads, g.smem_bytes));
     }
     if (occ < 1) return B200DVB_ENOSPEC;
     g.ctas_per_sm = occ;
@@ -1049,15 +1042,13 @@ int quad_configure(Codec &c)
         t.smem_bytes = quad_smem_bytes(t);
         // the shared memory this geometry leaves unused is worth more as L1 for the records
         const int carve = (int)((t.smem_bytes * 100 + cap - 1) / cap) + 4;
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, __half>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
-        B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, int8_t>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+        B2_CHECK(for_each_llr_type([&](auto l) {
+            B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, decltype(l)>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cap));
+            B2_CUDA(cudaFuncSetAttribute(quad_kernel<false, true, true, decltype(l)>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+            return B200DVB_OK;
+        }));
         int og = 0;
-        B2_CUDA(occupancy_all_formats(&og, quad_kernel<false, true, true>, quad_kernel<false, true, true, __half>,
-                                      quad_kernel<false, true, true, int8_t>, t.threads, t.smem_bytes));
+        B2_CHECK(occupancy_all_formats(&og, [](auto l) { return quad_kernel<false, true, true, decltype(l)>; }, t.threads, t.smem_bytes));
         if (og > 512 / t.tmem_cols) og = 512 / t.tmem_cols;
         if (og > 1) og = 1;
         if (og >= 1) { t.ctas_per_sm = og; c.geom_g = t; }
@@ -1092,7 +1083,7 @@ static size_t grec_floats(const QuadGeom &g, int grid)
     return g.grec ? (size_t)grid * areas * g.rec_stride : 0;
 }
 
-size_t decode_workspace_bytes(const Codec &c, int B)
+size_t quad_workspace_bytes(const Codec &c, int B)
 {
     const QuadGeom &g = decode_geom(c, B);
     const int grid = grid_for(c, g, B);
@@ -1108,39 +1099,30 @@ static inline unsigned char *align256(void *p)
     return reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(p) + 255) & ~(uintptr_t)255);
 }
 
-template <class LlrT> static void quad_start(const QuadArgs &A, const QuadGeom &G, int grid, cudaStream_t s)
+int quad_launch_decode(const Codec &c, const DecodeIo &io)
 {
-    if (G.grec)          quad_kernel<false, true, true, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
-    else if (G.use_tmem) quad_kernel<false, true, false, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
-    else                 quad_kernel<false, false, false, LlrT><<<grid, G.threads, G.smem_bytes, s>>>(A);
-}
-
-int launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                  uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                  void *ws, size_t ws_bytes, cudaStream_t s)
-{
-    if (B == 0) return B200DVB_OK;
-    if (ws_bytes < decode_workspace_bytes(c, B)) return B200DVB_ENOMEM;
-    const QuadGeom &G = decode_geom(c, B);
-    const int grid = grid_for(c, G, B);
+    if (io.ws_bytes < quad_workspace_bytes(c, io.B)) return B200DVB_ENOMEM;
+    const QuadGeom &G = decode_geom(c, io.B);
+    const int grid = grid_for(c, G, io.B);
     const size_t per = (size_t)grid * G.frames * c.N;
     QuadArgs A{};
-    A.g = G; A.B = B; A.iterations = c.iterations;
-    A.n_groups = (B + G.frames - 1) / G.frames;
-    A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
-    A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
-    const uintptr_t pair_bytes = 2 * llr_bytes(fmt);
-    const bool even = (llr_stride % 2 == 0) && ((reinterpret_cast<uintptr_t>(llr) & (pair_bytes - 1)) == 0);
+    fill_decode_args(A, c, io);
+    A.g = G;
+    A.n_groups = (io.B + G.frames - 1) / G.frames;
+    const uintptr_t pair_bytes = 2 * llr_bytes(io.fmt);
+    const bool even = (io.llr_stride % 2 == 0) && ((reinterpret_cast<uintptr_t>(io.llr) & (pair_bytes - 1)) == 0);
     A.vec_ab = even && c.vec_ab;
     A.vec_wy = even && c.vec_wy;
     A.timed = c.opt_phase_timers;
-    A.Le1 = reinterpret_cast<double2 *>(align256(ws));
+    A.Le1 = reinterpret_cast<double2 *>(align256(io.ws));
     A.Le2 = A.Le1 + per; A.Y = A.Le2 + per;
     A.grec = reinterpret_cast<float *>(align256(A.Y + per));
-    if (fmt == LlrFormat::F16)     quad_start<__half>(A, G, grid, s);
-    else if (fmt == LlrFormat::I8) quad_start<int8_t>(A, G, grid, s);
-    else                           quad_start<float>(A, G, grid, s);
+    with_llr_type(io.fmt, [&](auto t) {
+        using L = decltype(t);
+        if (G.grec)          quad_kernel<false, true, true, L><<<grid, G.threads, G.smem_bytes, io.stream>>>(A);
+        else if (G.use_tmem) quad_kernel<false, true, false, L><<<grid, G.threads, G.smem_bytes, io.stream>>>(A);
+        else                 quad_kernel<false, false, false, L><<<grid, G.threads, G.smem_bytes, io.stream>>>(A);
+    });
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }
@@ -1166,16 +1148,6 @@ int launch_siso(const Codec &c, int B, const float *Lc_A, const float *Lc_B, con
     return B200DVB_OK;
 }
 
-int read_phase_cycles(double *out_h, int reset)
-{
-    unsigned long long h[8];
-    B2_CUDA(cudaMemcpyFromSymbol(h, g_phase_cycles, sizeof h));
-    for (int i = 0; i < 8; ++i) out_h[i] = (double)h[i];
-    if (reset) {
-        unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        B2_CUDA(cudaMemcpyToSymbol(g_phase_cycles, z, sizeof z));
-    }
-    return B200DVB_OK;
-}
+int quad_read_phase_cycles(double *out_h, int reset) { return read_phase_cycles(g_phase_cycles, out_h, reset); }
 
 }  // namespace b200dvb

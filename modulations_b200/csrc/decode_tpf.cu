@@ -63,12 +63,6 @@ struct TpfArgs {
     float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
 };
 
-constexpr int kRingPairs = 4;        // pass-1 prefetch ring depth in step pairs (2 KB each: the whole beta-vector area)
-// per-warp staging area: [0, 8K) beta vectors of the current window, [kW][4][32] float4 (the
-// pass-1 prefetch ring, 6 KB, aliases it); [8K, 10K) Z slot; [10K, 12K) X slot
-constexpr int kStageBytes = 12288;
-constexpr int kRowFloats = kStageBytes / 8;   // transposition: two frame rows of up to 1536 LLRs each share the staging area
-
 struct Ctx {
     int N, M, T;
     int f, isb, lane;                // frame within the tile, 0 = alpha lane / 1 = beta lane
@@ -847,107 +841,98 @@ tpf_kernel(const TpfArgs A)
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-int tpf_configure(Codec &c)
+// ---- shared with decode_nii.cu, whose kernel has this kernel's mapping, record pool and transposition ----
+void tpf_family_geometry(TpfGeom &g, int N, int y_cols, size_t hdr_bytes, size_t ext_bytes, bool with_init, size_t smem_optin)
 {
-    TpfGeom &g = c.tpf;
     g = TpfGeom{};
-    const int N = c.N;
-    if (N < 16 || (N % 4) != 0) return B200DVB_OK;
+    if (N < 16 || (N % 4) != 0) return;
     const int M = N / 2;
     int T = M < 64 ? M : 64;
-    while (T > 0 && (((M - T) % kW) != 0 || 8 * T + 4 * kW > 512)) --T;   // windows must not straddle TMEM / smem; Y columns
-    if (T < kW) return B200DVB_OK;
+    while (T > 0 && (((M - T) % kW) != 0 || 8 * T + y_cols > 512)) --T;   // windows must not straddle TMEM / smem; Y columns
+    if (T < kW) return;
     g.N = N; g.M = M; g.T = T; g.mid = N - 2 * T;
     g.nfull = M / kW; g.rag = M % kW; g.nslots = g.nfull + (g.rag ? 1 : 0);
     g.tmem_cols = 32;
-    while (g.tmem_cols < 8 * T + 4 * kW) g.tmem_cols *= 2;        // records + the window's Y
-    if (g.tmem_cols > 512) return B200DVB_OK;
+    while (g.tmem_cols < 8 * T + y_cols) g.tmem_cols *= 2;        // records + the window's Y
+    if (g.tmem_cols > 512) return;
     const size_t tab_bytes = ((size_t)2 * N * 2 + 15) / 16 * 16;
-    g.smem_bytes = tab_bytes + 64 + (size_t)kTpfWarps * g.mid * 2 * 16 * sizeof(float4) + (size_t)kTpfWarps * kStageBytes;
-    int dev = 0;
-    cudaDeviceProp prop;
-    B2_CUDA(cudaGetDevice(&dev));
-    B2_CUDA(cudaGetDeviceProperties(&prop, dev));
-    if (g.smem_bytes > (size_t)prop.sharedMemPerBlockOptin) return B200DVB_OK;   // falls back to the quad kernel
+    g.smem_bytes = tab_bytes + hdr_bytes + (size_t)kTpfWarps * g.mid * 2 * 16 * sizeof(float4) + (size_t)kTpfWarps * kStageBytes;
+    if (g.smem_bytes > smem_optin) return;                        // falls back to the quad kernel
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
     g.off_l1 = take((size_t)N * 16 * sizeof(float4));
     g.off_l2 = take((size_t)N * 16 * sizeof(float4));
-    g.off_le = take((size_t)N * 16 * sizeof(double2));
-    g.off_lef = take((size_t)N * 16 * sizeof(double2));
-    g.off_y = take((size_t)N * 16 * sizeof(double2));
+    g.off_le = take((size_t)N * 16 * ext_bytes);
+    g.off_lef = take((size_t)N * 16 * ext_bytes);
+    g.off_y = take((size_t)N * 16 * ext_bytes);
     g.off_ck = take((size_t)g.nslots * 4 * 32 * sizeof(float4));
+    if (with_init) g.off_init = take((size_t)2 * 4 * 32 * sizeof(float4));
     g.ws_per_warp = off;
-    // the device's maximum, not this codec's need: the attribute is per function and device, and codecs of several N coexist
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-    B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, int8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     g.enabled = 1;
-    return B200DVB_OK;
 }
 
-int tpf_read_phase_cycles(double *out_h, int reset)
+int tpf_family_grid(const Codec &c, int B, int tile)
 {
-    unsigned long long h[8];
-    B2_CUDA(cudaMemcpyFromSymbol(h, g_tpf_cycles, sizeof h));
-    for (int i = 0; i < 8; ++i) out_h[i] = (double)h[i];
-    if (reset) {
-        unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        B2_CUDA(cudaMemcpyToSymbol(g_tpf_cycles, z, sizeof z));
-    }
-    return B200DVB_OK;
-}
-
-static int tpf_grid(const Codec &c, int B)
-{
-    const int tiles = (B + kTpfFrames - 1) / kTpfFrames;
+    const int tiles = (B + tile - 1) / tile;
     const int ctas = (tiles + kTpfWarps - 1) / kTpfWarps;
     return ctas < c.num_sms ? ctas : c.num_sms;
 }
 
-size_t tpf_workspace_bytes(const Codec &c, int B)
+size_t tpf_family_workspace_bytes(const Codec &c, const TpfGeom &g, int B, int tile)
 {
-    return (size_t)tpf_grid(c, B) * kTpfWarps * c.tpf.ws_per_warp + 256;
+    return (size_t)tpf_family_grid(c, B, tile) * kTpfWarps * g.ws_per_warp + 256;
 }
 
-// B200DVB_OPT_PHASE_TIMERS (development): the instance with per-phase clock64() accounting, read by b200dvb_debug_tpf_cycles
-template <class LlrT> static void tpf_start(const TpfArgs &A, bool timed, int grid, size_t smem, cudaStream_t s)
+// whole rows by bulk copy: pitch and base 16-byte aligned, row fits half the staging area, and the group-staged
+// transposition finds room for at least two padded rows (+ the offset table) in one of the warp's areas
+int tpf_family_row_staging(const Codec &c, const TpfGeom &g, const DecodeIo &io)
 {
-    if (timed) tpf_kernel<true, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
-    else       tpf_kernel<false, LlrT><<<grid, kTpfWarps * 32, smem, s>>>(A);
+    const int nq = llr_row_q(io.fmt, c.n_llr);
+    if (c.N > 256 || (io.llr_stride * llr_bytes(io.fmt)) % 16 != 0 || (reinterpret_cast<uintptr_t>(io.llr) & 15) != 0 ||
+        nq * 4 > kRowFloats || c.opt_no_row_staging)
+        return 0;
+    const int pitch4 = ((nq + 6) & ~7) + 1;
+    const int rec_bytes = g.mid * 2 * 16 * (int)sizeof(float4);
+    const int avail = rec_bytes > kStageBytes ? rec_bytes : kStageBytes - c.N * 16;
+    return avail / (pitch4 * 16) >= 2;
 }
 
-int tpf_launch_decode(const Codec &c, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride, int32_t *bits,
-                      uint32_t *packed, const uint8_t *ref_bits, unsigned long long *counters,
-                      void *ws, size_t ws_bytes, cudaStream_t s)
+// ---- the parity-mode kernel ----
+int tpf_configure(Codec &c, size_t smem_optin)
 {
-    if (B == 0) return B200DVB_OK;
-    if (ws_bytes < tpf_workspace_bytes(c, B)) return B200DVB_ENOMEM;
+    tpf_family_geometry(c.tpf, c.N, 4 * kW, 64, sizeof(double2), false, smem_optin);
+    if (!c.tpf.enabled) return B200DVB_OK;
+    // the device's maximum, not this codec's need: the attribute is per function and device, and codecs of several N coexist
+    return for_each_llr_type([&](auto t) {
+        using L = decltype(t);
+        B2_CUDA(cudaFuncSetAttribute(tpf_kernel<false, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        B2_CUDA(cudaFuncSetAttribute(tpf_kernel<true, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_optin));
+        return B200DVB_OK;
+    });
+}
+
+int tpf_read_phase_cycles(double *out_h, int reset) { return read_phase_cycles(g_tpf_cycles, out_h, reset); }
+
+size_t tpf_workspace_bytes(const Codec &c, int B) { return tpf_family_workspace_bytes(c, c.tpf, B, kTpfFrames); }
+
+int tpf_launch_decode(const Codec &c, const DecodeIo &io)
+{
+    if (io.ws_bytes < tpf_workspace_bytes(c, io.B)) return B200DVB_ENOMEM;
     TpfArgs A{};
-    A.g = c.tpf; A.B = B; A.iterations = c.iterations;
-    A.n_tiles = (B + kTpfFrames - 1) / kTpfFrames;
+    fill_decode_args(A, c, io);
+    A.g = c.tpf;
+    A.n_tiles = (io.B + kTpfFrames - 1) / kTpfFrames;
     A.n_llr = c.n_llr;
-    // whole rows by bulk copy: pitch and base 16-byte aligned, row fits half the staging area
-    const int nq = llr_row_q(fmt, c.n_llr);
-    A.vec4 = (c.N <= 256) && ((llr_stride * llr_bytes(fmt)) % 16 == 0) && ((reinterpret_cast<uintptr_t>(llr) & 15) == 0) && (nq * 4 <= kRowFloats) &&
-             !c.opt_no_row_staging;
-    if (A.vec4) {   // the group-staged transposition needs at least two padded rows (+ the offset table) in one of the warp's areas
-        const int pitch4 = ((nq + 6) & ~7) + 1;
-        const int rec_bytes = c.tpf.mid * 2 * 16 * (int)sizeof(float4);
-        const int avail = rec_bytes > kStageBytes ? rec_bytes : kStageBytes - c.N * 16;
-        if (avail / (pitch4 * 16) < 2) A.vec4 = 0;
-    }
-    A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; A.tab = c.d_tab;
-    A.llr = llr; A.llr_stride = llr_stride; A.bits = bits; A.packed = packed;
-    A.ref_bits = ref_bits; A.counters = counters; A.llr_scale = llr_scale;
-    A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    A.vec4 = tpf_family_row_staging(c, c.tpf, io);
+    A.ws = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(io.ws) + 255) & ~(uintptr_t)255);
+    const int grid = tpf_family_grid(c, io.B, kTpfFrames);
+    // B200DVB_OPT_PHASE_TIMERS (development): the instance with per-phase clock64() accounting, read by b200dvb_debug_tpf_cycles
     const bool timed = c.opt_phase_timers != 0;
-    if (fmt == LlrFormat::F16)     tpf_start<__half>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
-    else if (fmt == LlrFormat::I8) tpf_start<int8_t>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
-    else                           tpf_start<float>(A, timed, tpf_grid(c, B), c.tpf.smem_bytes, s);
+    with_llr_type(io.fmt, [&](auto t) {
+        using L = decltype(t);
+        if (timed) tpf_kernel<true, L><<<grid, kTpfWarps * 32, c.tpf.smem_bytes, io.stream>>>(A);
+        else       tpf_kernel<false, L><<<grid, kTpfWarps * 32, c.tpf.smem_bytes, io.stream>>>(A);
+    });
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

@@ -204,12 +204,9 @@ class _CodecHandle:
         torch = _lib.torch_mod()
         B = x.shape[0]
         st = stream or self.stream()
-        lib = _lib.load()
-        fn, scale = lib.b200dvb_decode, ()
-        if x.dtype == torch.float16:
-            fn = lib.b200dvb_decode_f16
-        elif x.dtype == torch.int8:
-            fn, scale = lib.b200dvb_decode_i8, (float(llr_scale),)
+        entry, scaled = _LLR_FORMATS[_dtype_name(x.dtype)]
+        fn = getattr(_lib.load(), entry)
+        scale = (float(llr_scale),) if scaled else ()
         with torch.cuda.device(self.device):
             buf, need = ws if ws is not None else self.workspace("decode", B, st)
             stride = x.stride(0) if B > 1 else x.shape[1]     # a length-1 axis may report stride 0
@@ -490,10 +487,8 @@ class DVBRCS2_Turbo:
         is_torch = isinstance(llr, torch.Tensor)
         if not is_torch:
             llr = np.asarray(llr)
-        half = llr.dtype == (torch.float16 if is_torch else np.float16)
-        i8 = llr.dtype == (torch.int8 if is_torch else np.int8)
-        kw = _scale_kw(llr_scale, i8)
-        x = _lib.to_device(llr, torch.float16 if half else torch.int8 if i8 else torch.float32, h.device)
+        fmt, kw = _llr_format(llr.dtype, llr_scale)
+        x = _lib.to_device(llr, getattr(torch, fmt or "float32"), h.device)
         if x.dim() == 1:
             x = x[None, :]
         if x.dim() != 2 or x.shape[1] < h.n_llr:
@@ -546,13 +541,13 @@ class DVBRCS2_Turbo:
             raise ValueError('out must be "bits", "packed" or "uint8"')
         if chunk is None:
             chunk = max(16, h.frames_per_wave)
-        if isinstance(llr_host, torch.Tensor):
-            x = llr_host
-        else:
-            a = np.asarray(llr_host)
-            x = torch.from_numpy(np.ascontiguousarray(a, a.dtype if a.dtype in (np.float16, np.int8) else np.float32))
-        kw = _scale_kw(llr_scale, x.dtype == torch.int8)
-        if x.dim() != 2 or x.shape[1] < h.n_llr or x.dtype not in (torch.float32, torch.float16, torch.int8):
+        is_torch = isinstance(llr_host, torch.Tensor)
+        x = llr_host if is_torch else np.asarray(llr_host)
+        fmt, kw = _llr_format(x.dtype, llr_scale)
+        if not is_torch:
+            fmt = fmt or "float32"
+            x = torch.from_numpy(np.ascontiguousarray(x, fmt))
+        if x.dim() != 2 or x.shape[1] < h.n_llr or fmt is None:
             raise IndexError(f"llr needs float32, float16 or int8 shape [B, >= {h.n_llr}]")
         B, width = x.shape
         wpf = (self.k_info + 31) // 32
@@ -629,14 +624,27 @@ class DVBRCS2_Turbo:
         return hout_np[0].copy()
 
 
-def _scale_kw(llr_scale, is_int8):
-    """_CodecHandle.decode keywords for the LLR dtype: int8 takes its scale (1.0 when not given); a scale given with
-    any other dtype is an error, not silently ignored."""
-    if not is_int8:
+# Channel LLR element formats the decoder takes, by dtype name (numpy's and torch's alike; the name is also the torch
+# dtype on the device): the C entry point, and whether it takes a scale (int8 q is the float32 LLR q * llr_scale).
+_LLR_FORMATS = {"float32": ("b200dvb_decode", False),
+                "float16": ("b200dvb_decode_f16", False),
+                "int8": ("b200dvb_decode_i8", True)}
+
+
+def _dtype_name(dtype):
+    return str(dtype).removeprefix("torch.")
+
+
+def _llr_format(dtype, llr_scale):
+    """-> (name in _LLR_FORMATS, or None for a dtype the decoder does not take; _CodecHandle.decode keywords).  int8
+    takes its scale (1.0 when not given); a scale given with any other dtype is an error, not silently ignored."""
+    fmt = _dtype_name(dtype)
+    fmt = fmt if fmt in _LLR_FORMATS else None
+    if fmt is None or not _LLR_FORMATS[fmt][1]:
         if llr_scale is not None:
             raise ValueError("llr_scale applies to int8 LLRs only")
-        return {}
-    return {"llr_scale": 1.0 if llr_scale is None else float(llr_scale)}
+        return fmt, {}
+    return fmt, {"llr_scale": 1.0 if llr_scale is None else float(llr_scale)}
 
 
 def _unpack_bits_device(packed, out_u8, k_info):
