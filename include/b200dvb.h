@@ -151,6 +151,26 @@ int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long 
 int b200dvb_decode_i8(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride, float scale,
                       int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                       unsigned long long *counters, void *workspace, size_t workspace_bytes, void *stream);
+/* Soft-output decode: b200dvb_decode / _f16 / _i8 (llr_format B200DVB_LLR_F32 / _F16 / _I8, with the same argument rules:
+ * F16 needs a 2-byte-aligned llr, I8 a finite non-zero llr_scale; llr_scale is ignored for F32 and F16) that also
+ * writes the a-posteriori LLR of every info bit after the last iteration:
+ *   app  float32[B][2N], required, 8-byte aligned (else B200DVB_EINVAL): app[f][2k] is bit A of couple k, app[f][2k+1]
+ *        bit B, the layout of `bits`.  Positive means bit 0, the convention of the input LLRs.
+ * The value is the one whose sign the hard decision takes (LA = (Lc + La) + Le1 of the final iteration):
+ *   B200DVB_MODE_PARITY (every kernel)  (float)LA, LA the float64 sum, rounded to nearest: float32 of the oracle's
+ *                                       Lfinal (dvb_rcs2_turbo.py:529-535), bit for bit
+ *   B200DVB_MODE_NII                    the float32 sum LA itself, bit for bit
+ *   B200DVB_MODE_NII16                  the int16 sum in 1/4-LLR units times 0.25f (exact: |LA| <= 637 units)
+ * bits, packed, ref_bits and counters are optional and hold exactly what b200dvb_decode / _f16 / _i8 give for the same
+ * input: the hard decisions are not derived from app.  fp16 and int8 input give the app of their float32 widening.
+ * The kernel choice and the workspace (b200dvb_decode_workspace_bytes) are those of b200dvb_decode. */
+#define B200DVB_LLR_F32 0
+#define B200DVB_LLR_F16 1
+#define B200DVB_LLR_I8  2
+int b200dvb_decode_app(b200dvb_codec_t codec, int B, const void *llr, int llr_format, float llr_scale,
+                       long long llr_stride, float *app, int32_t *bits, uint32_t *packed,
+                       const uint8_t *ref_bits, unsigned long long *counters,
+                       void *workspace, size_t workspace_bytes, void *stream);
 
 /* Tail-biting encoder for B frames.  Replaces DVBRCS2_Turbo.encode
  * (dvb_rcs2_turbo.py:431-462) including _encode_component (:404-429) and the

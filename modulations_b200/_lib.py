@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "libb200dvb.so")
 OK, EINVAL, ENOSPEC, ECUDA, ENOMEM, EMOD = 0, -1, -2, -3, -4, -5
 OPT_KERNEL, OPT_NO_ROW_STAGING, OPT_PHASE_TIMERS, OPT_DECODER_MODE = 1, 2, 3, 4
 MODE_PARITY, MODE_NII, MODE_NII16 = 0, 1, 2
+LLR_F32, LLR_F16, LLR_I8 = 0, 1, 2
 KERNEL_AUTO, KERNEL_QUAD, KERNEL_TPF, KERNEL_LAT = 0, 1, 2, 3
 MOD_IDS = {'BPSK': 0, 'QPSK': 1, '8PSK': 2, '16QAM': 3, '64QAM': 4, '256QAM': 5}
 BPS = {'BPSK': 1, 'QPSK': 2, '8PSK': 3, '16QAM': 4, '64QAM': 6, '256QAM': 8}
@@ -42,6 +43,8 @@ SIGNATURES = {
     "b200dvb_decode": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
     "b200dvb_decode_f16": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
     "b200dvb_decode_i8": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_ll, _c_float] + [_c_void_p] * 5 + [_c_size_t, _c_void_p]),
+    "b200dvb_decode_app": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_int, _c_float, _c_ll] + [_c_void_p] * 6
+                           + [_c_size_t, _c_void_p]),
     "b200dvb_encode": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
     "b200dvb_mc_generate_bpsk": (_c_int, [_c_void_p, _c_int, _c_float, _c_ull, _c_ull] + [_c_void_p] * 4),
     "b200dvb_awgn_complex": (_c_int, [_c_size_t, _c_float, _c_ull, _c_ull, _c_void_p, _c_void_p]),

@@ -307,17 +307,17 @@ int b200dvb_codec_set_option(b200dvb_codec_t codec, int option, int value)
     }
 }
 
-// b200dvb_decode / _f16 / _i8: the kernel choice does not depend on the element format
+// b200dvb_decode / _f16 / _i8 / _app: the kernel choice depends neither on the element format nor on the outputs
 static int decode_any(b200dvb_codec_t codec, int B, const void *llr, LlrFormat fmt, float llr_scale, long long llr_stride,
-                      int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
+                      float *app, int32_t *bits, uint32_t *packed, const uint8_t *ref_bits,
                       unsigned long long *counters, void *workspace, size_t workspace_bytes,
                       void *stream)
 {
     if (!codec || B < 0 || !llr || (B && !workspace)) return B200DVB_EINVAL;
     if (llr_stride < codec->c.n_llr) return B200DVB_EINVAL;
     if (B == 0) return B200DVB_OK;
-    const DecodeIo io{B, llr, fmt, llr_scale, llr_stride, bits, packed, ref_bits, counters, workspace, workspace_bytes,
-                      (cudaStream_t)stream};
+    const DecodeIo io{B, llr, fmt, llr_scale, llr_stride, app, bits, packed, ref_bits, counters, workspace,
+                      workspace_bytes, (cudaStream_t)stream};
     switch (decoder_for(codec->c, B)) {
     case Decoder::NII: return nii_launch_decode(codec->c, io);
     case Decoder::LAT: return lat_launch_decode(codec->c, io);
@@ -331,8 +331,8 @@ int b200dvb_decode(b200dvb_codec_t codec, int B, const float *llr, long long llr
                    unsigned long long *counters, void *workspace, size_t workspace_bytes,
                    void *stream)
 {
-    return decode_any(codec, B, llr, LlrFormat::F32, 1.f, llr_stride, bits, packed, ref_bits, counters, workspace,
-                      workspace_bytes, stream);
+    return decode_any(codec, B, llr, LlrFormat::F32, 1.f, llr_stride, nullptr, bits, packed, ref_bits, counters,
+                      workspace, workspace_bytes, stream);
 }
 
 int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride,
@@ -341,8 +341,8 @@ int b200dvb_decode_f16(b200dvb_codec_t codec, int B, const void *llr, long long 
                        void *stream)
 {
     if (reinterpret_cast<uintptr_t>(llr) & 1) return B200DVB_EINVAL;
-    return decode_any(codec, B, llr, LlrFormat::F16, 1.f, llr_stride, bits, packed, ref_bits, counters, workspace,
-                      workspace_bytes, stream);
+    return decode_any(codec, B, llr, LlrFormat::F16, 1.f, llr_stride, nullptr, bits, packed, ref_bits, counters,
+                      workspace, workspace_bytes, stream);
 }
 
 int b200dvb_decode_i8(b200dvb_codec_t codec, int B, const void *llr, long long llr_stride, float scale,
@@ -351,7 +351,30 @@ int b200dvb_decode_i8(b200dvb_codec_t codec, int B, const void *llr, long long l
                       void *stream)
 {
     if (!isfinite(scale) || scale == 0.f) return B200DVB_EINVAL;
-    return decode_any(codec, B, llr, LlrFormat::I8, scale, llr_stride, bits, packed, ref_bits, counters, workspace,
+    return decode_any(codec, B, llr, LlrFormat::I8, scale, llr_stride, nullptr, bits, packed, ref_bits, counters,
+                      workspace, workspace_bytes, stream);
+}
+
+int b200dvb_decode_app(b200dvb_codec_t codec, int B, const void *llr, int llr_format, float llr_scale,
+                       long long llr_stride, float *app, int32_t *bits, uint32_t *packed,
+                       const uint8_t *ref_bits, unsigned long long *counters,
+                       void *workspace, size_t workspace_bytes, void *stream)
+{
+    if (!app || (reinterpret_cast<uintptr_t>(app) & 7)) return B200DVB_EINVAL;   // one float2 store per couple
+    LlrFormat fmt;
+    switch (llr_format) {
+    case B200DVB_LLR_F32: fmt = LlrFormat::F32; llr_scale = 1.f; break;
+    case B200DVB_LLR_F16:
+        if (reinterpret_cast<uintptr_t>(llr) & 1) return B200DVB_EINVAL;
+        fmt = LlrFormat::F16; llr_scale = 1.f;
+        break;
+    case B200DVB_LLR_I8:
+        if (!isfinite(llr_scale) || llr_scale == 0.f) return B200DVB_EINVAL;
+        fmt = LlrFormat::I8;
+        break;
+    default: return B200DVB_EINVAL;
+    }
+    return decode_any(codec, B, llr, fmt, llr_scale, llr_stride, app, bits, packed, ref_bits, counters, workspace,
                       workspace_bytes, stream);
 }
 

@@ -188,14 +188,16 @@ struct Modem {
     double h_table[512];
 };
 
-// One decode call (b200dvb_decode / _f16 / _i8, B > 0): llr holds B rows of elements of format fmt, llr_stride elements
-// apart; llr_scale multiplies int8 elements and is unused otherwise.  bits, packed, ref_bits and counters may be NULL.
+// One decode call (b200dvb_decode / _f16 / _i8 / _app, B > 0): llr holds B rows of elements of format fmt, llr_stride
+// elements apart; llr_scale multiplies int8 elements and is unused otherwise.  app (float32 [B][2N], 8-byte aligned:
+// each couple's two values are stored as one float2), bits, packed, ref_bits and counters may be NULL.
 struct DecodeIo {
     int B;
     const void *llr;
     LlrFormat fmt;
     float llr_scale;
     long long llr_stride;
+    float *app;
     int32_t *bits;
     uint32_t *packed;
     const uint8_t *ref_bits;
@@ -210,7 +212,7 @@ template <class Args> inline void fill_decode_args(Args &A, const Codec &c, cons
 {
     A.B = io.B; A.iterations = c.iterations; A.tab = c.d_tab;
     A.llr = io.llr; A.llr_stride = io.llr_stride; A.llr_scale = io.llr_scale;
-    A.bits = io.bits; A.packed = io.packed; A.ref_bits = io.ref_bits; A.counters = io.counters;
+    A.bits = io.bits; A.packed = io.packed; A.ref_bits = io.ref_bits; A.counters = io.counters; A.app = io.app;
     if constexpr (std::is_same<decltype(A.sf_inner), double>::value) { A.sf_inner = c.sf_inner; A.sf_last = c.sf_last; }
 }
 

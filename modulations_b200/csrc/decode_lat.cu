@@ -42,6 +42,7 @@ struct LatArgs {
     const uint8_t *ref_bits;
     unsigned long long *counters;
     float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
+    float *app;                      // [B][2N] a-posteriori LLRs (float2 per couple) or NULL; last, for the same reason
 };
 
 __device__ __forceinline__ void ld16(const float *p, float (&v)[16])
@@ -297,6 +298,9 @@ lat_kernel(const LatArgs A)
             const double LB = d_add(d_add((double)ab.y, la.y), e1.y);
             const int bA = LA < 0.0, bB = LB < 0.0;
             if (A.bits) *reinterpret_cast<int2 *>(A.bits + (size_t)frame * 2 * N + 2 * k) = make_int2(bA, bB);
+            if (A.app)
+                *reinterpret_cast<float2 *>(A.app + (size_t)frame * 2 * N + 2 * k) =
+                    make_float2(__double2float_rn(LA), __double2float_rn(LB));
             atomicOr(&words[k >> 4], (unsigned)(bA | (bB << 1)) << (2 * (k & 15)));
             if (A.ref_bits) {
                 const uint8_t *r = A.ref_bits + (size_t)frame * 2 * N + 2 * k;

@@ -44,6 +44,7 @@ struct ArF32 {
     static __device__ __forceinline__ float add(float a, float b) { return f_add(a, b); }
     static __device__ __forceinline__ float chan(float lo, float) { return lo; }             // channel LLR of the lane's frame(s)
     static __device__ __forceinline__ int neg(float L, int) { return L < 0.f; }             // hard decision of sub-frame i
+    static __device__ __forceinline__ float to_llr(float L, int) { return L; }              // sub-frame i's value as an LLR
 };
 struct ArS16 {
     static constexpr int kFpl = 2;
@@ -95,6 +96,11 @@ struct ArS16 {
     static __device__ __forceinline__ float add(float a, float b) { return nii16::fl(nii16::add2(nii16::bits(a), nii16::bits(b))); }
     static __device__ __forceinline__ float chan(float lo, float hi) { return nii16::fl(nii16::pack16(nii16::quant(lo), nii16::quant(hi))); }
     static __device__ __forceinline__ int neg(float L, int i) { return (i ? nii16::hi16(nii16::bits(L)) : nii16::lo16(nii16::bits(L))) < 0; }
+    // 1/4-LLR units -> LLR: the int16 (|x| <= 637 in a decision) times 0.25 is exact in float32
+    static __device__ __forceinline__ float to_llr(float L, int i)
+    {
+        return __fmul_rn(__int2float_rn(i ? nii16::hi16(nii16::bits(L)) : nii16::lo16(nii16::bits(L))), 0.25f);
+    }
 };
 
 constexpr int kW = kTpfWin;
@@ -118,6 +124,7 @@ struct NiiArgs {
     unsigned long long *counters;
     unsigned char *ws;
     float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
+    float *app;                      // [B][2N] a-posteriori LLRs (float2 per couple) or NULL; last, for the same reason
 };
 
 struct Ctx {
@@ -866,6 +873,9 @@ nii_kernel(const NiiArgs A)
                         word[i] |= (unsigned)(bA | (bB << 1)) << (2 * (8 * (b & 1) + t));
                         if (live[i] && A.bits)
                             *reinterpret_cast<int2 *>(A.bits + (size_t)frame[i] * 2 * N + 2 * k) = make_int2(bA, bB);
+                        if (live[i] && A.app)
+                            *reinterpret_cast<float2 *>(A.app + (size_t)frame[i] * 2 * N + 2 * k) =
+                                make_float2(AR::to_llr(LA, i), AR::to_llr(LB, i));
                         if (cnt[i]) {
                             const int errs = (bA != (rb[i][t] & 0xff)) + (bB != (rb[i][t] >> 8));
                             bit_err += errs;

@@ -56,6 +56,7 @@ struct QuadArgs {
     double2 *Le1, *Le2, *Y;
     float *grec;          // geometry `grec`: [CTA][frame slot][rec_stride] branch-metric records
     float llr_scale;      // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
+    float *app;           // full decode: [B][2N] a-posteriori LLRs (float2 per couple) or NULL; last, for the same reason
 };
 
 // phase timers (SM cycles summed over CTAs): 0 prep, 1 recursion in (pass 1 + pass 2 to the
@@ -875,6 +876,9 @@ quad_kernel(const QuadArgs A)
                     const int bA = LA < 0.0, bB = LB < 0.0;
                     if (A.bits)
                         *reinterpret_cast<int2 *>(A.bits + (size_t)frame * 2 * N + 2 * j) = make_int2(bA, bB);
+                    if (A.app)
+                        *reinterpret_cast<float2 *>(A.app + (size_t)frame * 2 * N + 2 * j) =
+                            make_float2(__double2float_rn(LA), __double2float_rn(LB));
                     hb[f * N + j] = (unsigned char)(bA | (bB << 1));
                     if (A.ref_bits) {
                         const int errs = (bA != rb[u].x) + (bB != rb[u].y);

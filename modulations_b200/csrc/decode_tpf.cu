@@ -61,6 +61,7 @@ struct TpfArgs {
     unsigned long long *counters;
     unsigned char *ws;
     float llr_scale;                 // int8 element q is the LLR q * llr_scale (last: the other members keep their offsets)
+    float *app;                      // [B][2N] a-posteriori LLRs (float2 per couple) or NULL; last, for the same reason
 };
 
 struct Ctx {
@@ -790,6 +791,9 @@ tpf_kernel(const TpfArgs A)
                     word |= (unsigned)(bA | (bB << 1)) << (2 * (8 * (b & 1) + t));
                     if (live && A.bits)
                         *reinterpret_cast<int2 *>(A.bits + (size_t)frame * 2 * N + 2 * k) = make_int2(bA, bB);
+                    if (live && A.app)
+                        *reinterpret_cast<float2 *>(A.app + (size_t)frame * 2 * N + 2 * k) =
+                            make_float2(__double2float_rn(LA), __double2float_rn(LB));
                     if (cnt) {
                         const int errs = (bA != (rb[t] & 0xff)) + (bB != (rb[t] >> 8));
                         bit_err += errs;

@@ -197,21 +197,28 @@ class _CodecHandle:
         _lib.check(rc, "encode")
         return coded, circ
 
-    def decode(self, x, bits=None, packed=None, ref=None, counters=None, stream=None, ws=None, llr_scale=1.0):
+    def decode(self, x, bits=None, packed=None, ref=None, counters=None, stream=None, ws=None, llr_scale=1.0, app=None):
         """x float32, float16 or int8 CUDA [B, >= n_llr] (row stride in elements taken from the tensor).  float16 goes
         to b200dvb_decode_f16: the decode of its exact float32 widening, bit for bit.  int8 goes to b200dvb_decode_i8:
-        the decode of float32(q) * float32(llr_scale), bit for bit; ``llr_scale`` is not read for other dtypes."""
+        the decode of float32(q) * float32(llr_scale), bit for bit; ``llr_scale`` is not read for other dtypes.
+        ``app`` (float32 CUDA [B, 2N], contiguous): the call goes to b200dvb_decode_app, which also writes the
+        a-posteriori LLRs there; the other outputs are the same."""
         torch = _lib.torch_mod()
         B = x.shape[0]
         st = stream or self.stream()
-        entry, scaled = _LLR_FORMATS[_dtype_name(x.dtype)]
-        fn = getattr(_lib.load(), entry)
-        scale = (float(llr_scale),) if scaled else ()
+        entry, scaled, code = _LLR_FORMATS[_dtype_name(x.dtype)]
+        lib = _lib.load()
         with torch.cuda.device(self.device):
             buf, need = ws if ws is not None else self.workspace("decode", B, st)
             stride = x.stride(0) if B > 1 else x.shape[1]     # a length-1 axis may report stride 0
-            rc = fn(self.h, B, _lib.ptr(x), stride, *scale, _lib.ptr(bits), _lib.ptr(packed), _lib.ptr(ref),
-                    _lib.ptr(counters), _lib.ptr(buf), need, ctypes.c_void_p(st.cuda_stream))
+            outs = (_lib.ptr(bits), _lib.ptr(packed), _lib.ptr(ref), _lib.ptr(counters), _lib.ptr(buf), need,
+                    ctypes.c_void_p(st.cuda_stream))
+            if app is not None:
+                rc = lib.b200dvb_decode_app(self.h, B, _lib.ptr(x), code, float(llr_scale) if scaled else 1.0, stride,
+                                            _lib.ptr(app), *outs)
+            else:
+                scale = (float(llr_scale),) if scaled else ()
+                rc = getattr(lib, entry)(self.h, B, _lib.ptr(x), stride, *scale, *outs)
         _lib.check(rc, "decode")
 
     def siso(self, f4, d2, sf):
@@ -476,14 +483,17 @@ class DVBRCS2_Turbo:
         and is an error with any other dtype).  Any other dtype is converted to float32.
 
         out="bits": int32 [B, 2N] (reference layout); "packed": uint32 [B, ceil(2N/32)], bit i of a frame at
-        word i//32, bit i%32; "none": nothing (error counting only).  ``ref_bits`` (anything reshapeable to
-        uint8 [B, 2N]) and ``counters`` (CUDA int64/uint64 tensor, >= 4 elements) enable in-kernel error
-        counting: counters += {bit errors, frame errors, frames, info bits}.
+        word i//32, bit i%32; "app": float32 [B, 2N], the a-posteriori LLR of each info bit after the last
+        iteration in the layout of "bits", positive = bit 0 (b200dvb_decode_app: parity mode gives the float32 of
+        the reference's float64 sum, "nii" its float32 sum, "nii16" its 1/4-unit sum times 0.25); "none": nothing
+        (error counting only).  ``ref_bits`` (anything reshapeable to uint8 [B, 2N]) and ``counters`` (CUDA
+        int64/uint64 tensor, >= 4 elements) enable in-kernel error counting: counters += {bit errors, frame errors,
+        frames, info bits}.
         """
         torch = _lib.require_cuda()
         h = self.handle
-        if out not in ("bits", "packed", "none"):
-            raise ValueError('out must be "bits", "packed" or "none"')
+        if out not in ("bits", "packed", "app", "none"):
+            raise ValueError('out must be "bits", "packed", "app" or "none"')
         is_torch = isinstance(llr, torch.Tensor)
         if not is_torch:
             llr = np.asarray(llr)
@@ -496,11 +506,13 @@ class DVBRCS2_Turbo:
         if x.stride(1) != 1:
             x = x.contiguous()
         B = x.shape[0]
-        bits = packed = None
+        bits = packed = app = None
         if out == "bits":
             bits = torch.empty((B, self.k_info), dtype=torch.int32, device=h.device)
         elif out == "packed":
             packed = torch.empty((B, (self.k_info + 31) // 32), dtype=torch.int32, device=h.device)
+        elif out == "app":
+            app = kw["app"] = torch.empty((B, self.k_info), dtype=torch.float32, device=h.device)
         ref = None
         if ref_bits is not None:
             ref = _lib.to_device(ref_bits, torch.uint8, h.device)
@@ -513,7 +525,7 @@ class DVBRCS2_Turbo:
                                          and counters.device == h.device):
             raise ValueError("counters must be a contiguous CUDA int64/uint64 tensor with >= 4 elements on the codec's device")
         h.decode(x, bits=bits, packed=packed, ref=ref, counters=counters, **kw)
-        res = bits if out == "bits" else packed
+        res = {"bits": bits, "packed": packed, "app": app}.get(out)
         if res is not None and not is_torch:
             res = res.cpu().numpy()
         return res
@@ -529,7 +541,8 @@ class DVBRCS2_Turbo:
         out="bits": int32 [B, 2N], the reference's layout (1 696 B per N=212 frame over PCIe);
         out="packed": int32 words [B, ceil(2N/32)], bit i of a frame at word i//32, bit i%32 (56 B per frame:
         the kernel's packed output copied as it is — ``unpack_bits`` expands it lazily on the host);
-        out="uint8": uint8 [B, 2N], expanded from the packed words on the device (424 B per frame).
+        out="uint8": uint8 [B, 2N], expanded from the packed words on the device (424 B per frame);
+        out="app": float32 [B, 2N], the a-posteriori LLRs of ``decode_batch(out="app")`` (8 N bytes per frame).
 
         Chunks are pipelined over three CUDA streams so the host->device copy of chunk i+1, the decode of
         chunk i and the device->host copy of chunk i-1 overlap.  ``chunk`` defaults to one wave of the decode
@@ -537,8 +550,8 @@ class DVBRCS2_Turbo:
         returned CPU tensor can be read at once."""
         torch = _lib.require_cuda()
         h = self.handle
-        if out not in ("bits", "packed", "uint8"):
-            raise ValueError('out must be "bits", "packed" or "uint8"')
+        if out not in ("bits", "packed", "uint8", "app"):
+            raise ValueError('out must be "bits", "packed", "uint8" or "app"')
         if chunk is None:
             chunk = max(16, h.frames_per_wave)
         is_torch = isinstance(llr_host, torch.Tensor)
@@ -552,7 +565,7 @@ class DVBRCS2_Turbo:
         B, width = x.shape
         wpf = (self.k_info + 31) // 32
         oshape, odtype = {"bits": ((self.k_info,), torch.int32), "packed": ((wpf,), torch.int32),
-                          "uint8": ((self.k_info,), torch.uint8)}[out]
+                          "uint8": ((self.k_info,), torch.uint8), "app": ((self.k_info,), torch.float32)}[out]
         if out_host is None:
             out_host = torch.empty((B,) + oshape, dtype=odtype, pin_memory=True)
         elif tuple(out_host.shape) != (B,) + oshape or out_host.dtype != odtype:
@@ -582,6 +595,8 @@ class DVBRCS2_Turbo:
                     h.decode(din[j][:n], bits=dout[j], stream=streams[j], ws=wss[j], **kw)
                 elif out == "packed":
                     h.decode(din[j][:n], packed=dout[j], stream=streams[j], ws=wss[j], **kw)
+                elif out == "app":
+                    h.decode(din[j][:n], app=dout[j], stream=streams[j], ws=wss[j], **kw)
                 else:
                     h.decode(din[j][:n], packed=dpk[j], stream=streams[j], ws=wss[j], **kw)
                     _unpack_bits_device(dpk[j][:n], dout[j][:n], self.k_info)
@@ -625,10 +640,11 @@ class DVBRCS2_Turbo:
 
 
 # Channel LLR element formats the decoder takes, by dtype name (numpy's and torch's alike; the name is also the torch
-# dtype on the device): the C entry point, and whether it takes a scale (int8 q is the float32 LLR q * llr_scale).
-_LLR_FORMATS = {"float32": ("b200dvb_decode", False),
-                "float16": ("b200dvb_decode_f16", False),
-                "int8": ("b200dvb_decode_i8", True)}
+# dtype on the device): the C entry point, whether it takes a scale (int8 q is the float32 LLR q * llr_scale), and the
+# format code of b200dvb_decode_app.
+_LLR_FORMATS = {"float32": ("b200dvb_decode", False, _lib.LLR_F32),
+                "float16": ("b200dvb_decode_f16", False, _lib.LLR_F16),
+                "int8": ("b200dvb_decode_i8", True, _lib.LLR_I8)}
 
 
 def _dtype_name(dtype):
