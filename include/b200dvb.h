@@ -209,6 +209,15 @@ int b200dvb_demap(b200dvb_modem_t modem, size_t n_sym, const void *iq, float noi
  * (4 + 4 bps algorithmic bytes per symbol instead of 8 + 4 bps). */
 int b200dvb_demap_bf16(b200dvb_modem_t modem, size_t n_sym, const void *iq_bf16x2, float noise_var,
                        float scale, float *llr, void *stream);
+/* Max-log LLRs with perfect channel state: symbol i was received as y = h*c + noise with a known complex gain h.
+ *   llr[i*bps+b] = clip((min_{c: b=0} |y - h c|^2 - min_{c: b=1} |y - h c|^2) / max(noise_var, 0.005), +-30) * scale
+ * with the sign convention, floor, clip and scale of b200dvb_demap.  iq, gain float2[n_sym] and llr float32[n_sym*bps],
+ * all 16-byte aligned; gain is required (else B200DVB_EINVAL).  Computed as the arithmetic of b200dvb_demap on the
+ * equalised symbol z = y conj(h) / |h|^2 with 1/noise_var scaled by |h|^2, so a symbol with h = 1 gets exactly the
+ * LLRs b200dvb_demap gives it (z is formed in float64, then rounded to float32).  h = 0 gives 0, and every finite y
+ * and h give a finite LLR. */
+int b200dvb_demap_csi(b200dvb_modem_t modem, size_t n_sym, const void *iq, const void *gain, float noise_var,
+                      float scale, float *llr, void *stream);
 /* Hard decisions.  Replaces SDRModem.demodulate (sdr_modem.py:245-266) and
  * Modulator._demod_qam_generic (modulators.py:165-171): nearest constellation
  * point, evaluated in float64.  in_f64 selects float2 / double2 input. */
@@ -234,6 +243,13 @@ int b200dvb_mc_generate_bpsk(b200dvb_codec_t codec, int B, float noise_var,
  * (channel model of test.py:66-68).  iq float2[n_sym]; offset must be even. */
 int b200dvb_awgn_complex(size_t n_sym, float sigma, unsigned long long seed,
                          unsigned long long offset, void *iq, void *stream);
+/* Rayleigh block-fading channel with AWGN, in place: iq[i] = h[b]*iq[i] + sigma*(n_re + j*n_im), b = (offset + i) /
+ * block_len.  h[b] ~ CN(0, 1) (each component N(0, 1/2), E|h|^2 = 1) depends on (seed, b) only; block_len = 1 is fast
+ * fading, and a block may straddle calls and frames.  The noise is keyed exactly as in b200dvb_awgn_complex: with iq
+ * all zeros both write the same bits.  gain (nullable) float2[n_sym] receives the h applied to each symbol.
+ * B200DVB_EINVAL for a NULL iq, sigma < 0 or NaN, block_len < 1 or an odd offset. */
+int b200dvb_fading_complex(size_t n_sym, int block_len, float sigma, unsigned long long seed,
+                           unsigned long long offset, void *iq, void *gain, void *stream);
 
 /* Waveform stage next to the mapper / demapper (SURVEY 8(f) N4; float32 FMAs; taps_h = HOST float64[ntaps], the
  * reference's rrc_filter array, ntaps <= 448: they travel in the kernel's parameter space).

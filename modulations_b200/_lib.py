@@ -48,11 +48,14 @@ SIGNATURES = {
     "b200dvb_encode": (_c_int, [_c_void_p, _c_int, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
     "b200dvb_mc_generate_bpsk": (_c_int, [_c_void_p, _c_int, _c_float, _c_ull, _c_ull] + [_c_void_p] * 4),
     "b200dvb_awgn_complex": (_c_int, [_c_size_t, _c_float, _c_ull, _c_ull, _c_void_p, _c_void_p]),
+    "b200dvb_fading_complex": (_c_int, [_c_size_t, _c_int, _c_float, _c_ull, _c_ull, _c_void_p, _c_void_p, _c_void_p]),
     "b200dvb_modem_create": (_c_int, [_c_int, _c_void_p, _c_void_p]),
     "b200dvb_modem_destroy": (_c_int, [_c_void_p]),
     "b200dvb_map": (_c_int, [_c_void_p, _c_size_t, _c_void_p, _c_void_p, _c_int, _c_void_p]),
     "b200dvb_demap": (_c_int, [_c_void_p, _c_size_t, _c_void_p, _c_float, _c_float, _c_void_p, _c_void_p]),
     "b200dvb_demap_bf16": (_c_int, [_c_void_p, _c_size_t, _c_void_p, _c_float, _c_float, _c_void_p, _c_void_p]),
+    "b200dvb_demap_csi": (_c_int, [_c_void_p, _c_size_t, _c_void_p, _c_void_p, _c_float, _c_float, _c_void_p,
+                                   _c_void_p]),
     "b200dvb_hard_demod": (_c_int, [_c_void_p, _c_size_t, _c_void_p, _c_int, _c_void_p, _c_void_p]),
     "b200dvb_pulse_shape": (_c_int, [_c_size_t, _c_void_p, _c_void_p, _c_int, _c_int, _c_void_p, _c_void_p]),
     "b200dvb_matched_filter": (_c_int, [_c_size_t, _c_void_p, _c_void_p, _c_int, _c_int, _c_ll, _c_size_t, _c_void_p, _c_void_p]),

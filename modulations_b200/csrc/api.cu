@@ -407,6 +407,13 @@ int b200dvb_awgn_complex(size_t n_sym, float sigma, unsigned long long seed,
     return launch_awgn_complex(n_sym, sigma, seed, offset, iq, (cudaStream_t)stream);
 }
 
+int b200dvb_fading_complex(size_t n_sym, int block_len, float sigma, unsigned long long seed,
+                           unsigned long long offset, void *iq, void *gain, void *stream)
+{
+    if (!iq || !(sigma >= 0.f) || block_len < 1 || (offset & 1ull)) return B200DVB_EINVAL;
+    return launch_fading_complex(n_sym, block_len, sigma, seed, offset, iq, gain, (cudaStream_t)stream);
+}
+
 int b200dvb_pulse_shape(size_t n_sym, const void *sym, const double *taps_h, int ntaps, int sps, void *out, void *stream)
 {
     if (!sym || !taps_h || !out || ntaps < 1 || ntaps > kMaxFirTaps || sps < 1 || sps > 64) return B200DVB_EINVAL;
@@ -498,6 +505,13 @@ int b200dvb_demap_bf16(b200dvb_modem_t modem, size_t n_sym, const void *iq_bf16x
 {
     if (!modem || !iq_bf16x2 || !llr) return B200DVB_EINVAL;
     return launch_demap_bf16(modem->m, n_sym, iq_bf16x2, noise_var, scale, llr, (cudaStream_t)stream);
+}
+
+int b200dvb_demap_csi(b200dvb_modem_t modem, size_t n_sym, const void *iq, const void *gain, float noise_var,
+                      float scale, float *llr, void *stream)
+{
+    if (!modem || !iq || !gain || !llr) return B200DVB_EINVAL;
+    return launch_demap_csi(modem->m, n_sym, iq, gain, noise_var, scale, llr, (cudaStream_t)stream);
 }
 
 int b200dvb_hard_demod(b200dvb_modem_t modem, size_t n_sym, const void *iq, int in_f64,

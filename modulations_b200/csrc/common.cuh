@@ -255,12 +255,16 @@ int launch_mc_bpsk(const Codec &c, int B, float noise_var, unsigned long long se
 
 int launch_awgn_complex(size_t n, float sigma, unsigned long long seed, unsigned long long offset,
                         void *iq, cudaStream_t s);
+int launch_fading_complex(size_t n, int block_len, float sigma, unsigned long long seed, unsigned long long offset,
+                          void *iq, void *gain, cudaStream_t s);
 
 int launch_map(const Modem &m, size_t n, const uint8_t *bits, void *iq, int out_f64, cudaStream_t s);
 int launch_demap(const Modem &m, size_t n, const void *iq, float noise_var, float scale,
                  float *llr, cudaStream_t s);
 int launch_demap_bf16(const Modem &m, size_t n, const void *iq, float noise_var, float scale,
                       float *llr, cudaStream_t s);
+int launch_demap_csi(const Modem &m, size_t n, const void *iq, const void *gain, float noise_var, float scale,
+                     float *llr, cudaStream_t s);
 int launch_hard(const Modem &m, size_t n, const void *iq, int in_f64, uint8_t *bits, cudaStream_t s);
 
 constexpr int kMaxFirTaps = 448;    // FIR taps travel in the kernel parameter space (constant bank): 8 B per tap of 4 KB

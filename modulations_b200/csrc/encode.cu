@@ -224,6 +224,51 @@ __global__ void awgn_complex_kernel(size_t n2, size_t n, float sigma, unsigned l
     }
 }
 
+// Rayleigh block fading h[b] ~ CN(0, 1) of block b = (global symbol index) / block_len: one Philox draw of stream 4
+// serves blocks 2d and 2d+1 (a Box-Muller pair each, scaled by sqrt(1/2) so that E|h|^2 = 1).
+__device__ __forceinline__ float2 fading_gain(const Philox &r, unsigned long long b)
+{
+    const bool odd = b & 1ull;
+    const float u1 = ((float)(odd ? r.c[2] : r.c[0]) + 0.5f) * 2.3283064365386963e-10f;
+    const float u2 = ((float)(odd ? r.c[3] : r.c[1]) + 0.5f) * 2.3283064365386963e-10f;
+    float n0, n1;
+    box_muller(u1, u2, n0, n1);
+    return make_float2(0.70710678118654752f * n0, 0.70710678118654752f * n1);
+}
+
+// iq[i] = h[b] iq[i] + sigma (n_re + j n_im) in place, 2 symbols per thread; the noise is awgn_complex_kernel's,
+// draw for draw.  gain (nullable) receives the h of every symbol.
+__global__ void fading_complex_kernel(size_t n2, size_t n, unsigned long long block_len, float sigma,
+                                      unsigned long long seed, unsigned long long offset2, float2 *__restrict__ iq,
+                                      float2 *__restrict__ gain)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n2) return;
+    const Philox r = philox(offset2 + i, 3u, seed);
+    // blocks of the thread's two symbols: b1 is b0 or b0 + 1
+    const unsigned long long s0 = 2 * (offset2 + i);
+    const unsigned long long b0 = block_len == 1 ? s0 : s0 / block_len;
+    const unsigned long long b1 = block_len == 1 ? s0 + 1 : (s0 + 1) / block_len;
+    const Philox q0 = philox(b0 >> 1, 4u, seed);
+    const float2 h0 = fading_gain(q0, b0);
+    const float2 h1 = b1 == b0 ? h0 : fading_gain((b1 >> 1) == (b0 >> 1) ? q0 : philox(b1 >> 1, 4u, seed), b1);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const size_t e = 2 * i + h;
+        if (e >= n) break;
+        const float u1 = ((float)r.c[2 * h] + 0.5f) * 2.3283064365386963e-10f;
+        const float u2 = ((float)r.c[2 * h + 1] + 0.5f) * 2.3283064365386963e-10f;
+        float g0, g1;
+        box_muller(u1, u2, g0, g1);
+        const float2 hb = h ? h1 : h0, v = iq[e];
+        // + 0.f turns a faded -0 into +0: a zero input then gives awgn_complex_kernel's output bit for bit
+        float2 o = make_float2((hb.x * v.x - hb.y * v.y) + 0.f, (hb.x * v.y + hb.y * v.x) + 0.f);
+        o.x += sigma * g0; o.y += sigma * g1;
+        iq[e] = o;
+        if (gain) gain[e] = hb;
+    }
+}
+
 int odd_words(int bytes)
 {
     int w = (bytes + 3) / 4;
@@ -282,6 +327,18 @@ int launch_awgn_complex(size_t n, float sigma, unsigned long long seed, unsigned
     const size_t n2 = (n + 1) / 2;
     awgn_complex_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, s>>>(n2, n, sigma, seed, offset / 2,
                                                                     reinterpret_cast<float2 *>(iq));
+    B2_CUDA(cudaGetLastError());
+    return B200DVB_OK;
+}
+
+int launch_fading_complex(size_t n, int block_len, float sigma, unsigned long long seed, unsigned long long offset,
+                          void *iq, void *gain, cudaStream_t s)
+{
+    if (n == 0) return B200DVB_OK;
+    const size_t n2 = (n + 1) / 2;
+    fading_complex_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, s>>>(
+        n2, n, (unsigned long long)block_len, sigma, seed, offset / 2, reinterpret_cast<float2 *>(iq),
+        reinterpret_cast<float2 *>(gain));
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }

@@ -259,7 +259,9 @@ template <int BPS> struct PwlLlr {          // BPS = 2 * HALF
 
 // Symbol input formats of the demapper: complex64 (float2, the reference's dtype) or bf16x2 (4 bytes per symbol,
 // BASELINE north_star "bf16x2 loads of I/Q": widened exactly to float32, then the same arithmetic).
+// kCsi: the symbols come with a complex64 channel gain h each (InCsi below).
 struct InF32 {
+    static constexpr bool kCsi = false;
     typedef float2 sym_t;
     static __device__ __forceinline__ float2 one(const sym_t *p, size_t i) { return __ldcs(p + i); }
     static __device__ __forceinline__ void two(const sym_t *p, size_t i, float2 &a, float2 &b)
@@ -269,7 +271,8 @@ struct InF32 {
     }
 };
 struct InBf16 {
-    typedef unsigned sym_t;                                 // low half = I, high half = Q (a little-endian bf16 pair)
+    static constexpr bool kCsi = false;
+    typedef unsigned sym_t;                                // low half = I, high half = Q (a little-endian bf16 pair)
     static __device__ __forceinline__ float2 widen(unsigned w) { return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u)); }
     static __device__ __forceinline__ float2 one(const sym_t *p, size_t i) { return widen(__ldcs(p + i)); }
     static __device__ __forceinline__ void two(const sym_t *p, size_t i, float2 &a, float2 &b)
@@ -278,9 +281,29 @@ struct InBf16 {
         a = widen(t.x); b = widen(t.y);
     }
 };
+// complex64 symbols y with a complex64 gain h each (b200dvb_demap_csi): |y - hc|^2 = |h|^2 |z - c|^2 with
+// z = y conj(h) / |h|^2, so each symbol runs the arithmetic of InF32 on z with inv_nv scaled by |h|^2.
+struct InCsi : InF32 {
+    static constexpr bool kCsi = true;
+};
+
+// y <- z = y conj(h) / |h|^2 and inv_nv <- |h|^2 inv_nv.  z is formed in float64, where the products of float32
+// values are exact: in float32 the two terms of a component cancel, and the error of the sum is relative to |z|, not
+// to the component.  With h = 1 every step is exact, so the symbol's LLRs are those of b200dvb_demap.  Deep fades
+// produce no Inf * 0: the float64 z is finite for every finite y and h != 0, h = 0 gives z = 0 and LLR 0, and z's
+// components are clamped to +-1e18 (reached only where |y| > 1e18 |h|) so that |z - c|^2 stays finite in float32.
+__device__ __forceinline__ void equalise(float2 &y, const float2 h, float &inv_nv)
+{
+    const double hx = h.x, hy = h.y, h2 = hx * hx + hy * hy;
+    const double r = h2 > 0.0 ? 1.0 / h2 : 0.0;
+    const double zx = ((double)y.x * hx + (double)y.y * hy) * r, zy = ((double)y.y * hx - (double)y.x * hy) * r;
+    y = make_float2((float)fmin(fmax(zx, -1e18), 1e18), (float)fmin(fmax(zy, -1e18), 1e18));
+    inv_nv *= (float)h2;
+}
 
 template <int BPS, int SPT, class IN, class F>
-__device__ __forceinline__ void demap_body(size_t n, const typename IN::sym_t *__restrict__ iq, float *__restrict__ llr,
+__device__ __forceinline__ void demap_body(size_t n, const typename IN::sym_t *__restrict__ iq,
+                                           const float2 *__restrict__ gain, float *__restrict__ llr,
                                            const F &f, float *stage)
 {
     constexpr int CH = BPS * SPT;                       // floats per thread
@@ -289,17 +312,31 @@ __device__ __forceinline__ void demap_body(size_t n, const typename IN::sym_t *_
     for (size_t base = (size_t)blockIdx.x * tile; base < n; base += (size_t)gridDim.x * tile) {
         const size_t i0 = base + (size_t)threadIdx.x * SPT;
         const bool full = base + tile <= n;
-        float2 s[SPT];
+        float2 s[SPT], h[SPT];
         if (full && (SPT % 2) == 0) {
 #pragma unroll
-            for (int j = 0; j < SPT; j += 2) IN::two(iq, i0 + j, s[j], s[j + 1 < SPT ? j + 1 : j]);
+            for (int j = 0; j < SPT; j += 2) {
+                IN::two(iq, i0 + j, s[j], s[j + 1 < SPT ? j + 1 : j]);
+                if constexpr (IN::kCsi) InF32::two(gain, i0 + j, h[j], h[j + 1 < SPT ? j + 1 : j]);
+            }
         } else {
 #pragma unroll
-            for (int j = 0; j < SPT; ++j) s[j] = (i0 + j < n) ? IN::one(iq, i0 + j) : make_float2(0.f, 0.f);
+            for (int j = 0; j < SPT; ++j) {
+                s[j] = (i0 + j < n) ? IN::one(iq, i0 + j) : make_float2(0.f, 0.f);
+                if constexpr (IN::kCsi) h[j] = (i0 + j < n) ? InF32::one(gain, i0 + j) : make_float2(0.f, 0.f);
+            }
         }
         float v[SPT][BPS];
 #pragma unroll
-        for (int j = 0; j < SPT; ++j) f(s[j], v[j]);
+        for (int j = 0; j < SPT; ++j) {
+            if constexpr (IN::kCsi) {
+                F g = f;
+                equalise(s[j], h[j], g.inv_nv);
+                g(s[j], v[j]);
+            } else {
+                f(s[j], v[j]);
+            }
+        }
         if (!kStage) {
             if (full || i0 + SPT <= n) {
                 const float *p = &v[0][0];
@@ -332,7 +369,7 @@ __device__ __forceinline__ void demap_body(size_t n, const typename IN::sym_t *_
 template <int BPS, int SPT, class IN>
 __global__ void __launch_bounds__(kThreads)
 demap_generic(size_t n, const typename IN::sym_t *__restrict__ iq, const float *__restrict__ table,
-              float inv_nv, float scale, float *__restrict__ llr)
+              float inv_nv, float scale, float *__restrict__ llr, const float2 *__restrict__ gain)
 {
     constexpr int M = 1 << BPS;
     __shared__ float2 tab[M];
@@ -340,7 +377,7 @@ demap_generic(size_t n, const typename IN::sym_t *__restrict__ iq, const float *
     for (int i = threadIdx.x; i < M; i += blockDim.x) tab[i] = make_float2(table[2 * i], table[2 * i + 1]);
     __syncthreads();
     GenericLlr<BPS> f{tab, inv_nv, scale};
-    demap_body<BPS, SPT, IN>(n, iq, llr, f, stage);
+    demap_body<BPS, SPT, IN>(n, iq, gain, llr, f, stage);
 }
 
 // Per-axis piecewise-linear demapper.  coef: float2[2][HALF][nseg].
@@ -348,7 +385,7 @@ template <int HALF, int SPT, class IN>
 __global__ void __launch_bounds__(kThreads)
 demap_pwl(size_t n, const typename IN::sym_t *__restrict__ iq, const float2 *__restrict__ coef, int nseg,
           float x0a, float invda, float x0b, float invdb, int first_is_q, float inv_nv, float scale,
-          float *__restrict__ llr)
+          float *__restrict__ llr, const float2 *__restrict__ gain)
 {
     constexpr int BPS = 2 * HALF;
     __shared__ float2 sc[2 * 4 * 30];
@@ -356,23 +393,25 @@ demap_pwl(size_t n, const typename IN::sym_t *__restrict__ iq, const float2 *__r
     for (int i = threadIdx.x; i < 2 * HALF * nseg; i += blockDim.x) sc[i] = coef[i];
     __syncthreads();
     PwlLlr<BPS> f{sc, nseg, first_is_q, x0a, invda, x0b, invdb, inv_nv, scale};
-    demap_body<BPS, SPT, IN>(n, iq, llr, f, stage);
+    demap_body<BPS, SPT, IN>(n, iq, gain, llr, f, stage);
 }
 
 // 256QAM (4 bits per axis): one thread per (symbol, axis) writes one float4, so a warp's
 // stores are 512 contiguous bytes with no staging; both threads of a symbol read the same
-// 8 input bytes.
+// 8 input bytes (and the same gain, for InCsi).
 template <class IN>
 __global__ void __launch_bounds__(kThreads)
 demap_pwl_axis4(size_t n, const typename IN::sym_t *__restrict__ iq, const float2 *__restrict__ coef, int nseg,
-                float x0a, float invda, float x0b, float invdb, int first_is_q, float inv_nv, float scale,
-                float4 *__restrict__ llr4)
+                float x0a, float invda, float x0b, float invdb, int first_is_q, float inv_nv_, float scale,
+                float4 *__restrict__ llr4, const float2 *__restrict__ gain)
 {
     __shared__ float2 sc[2 * 4 * 30];
     for (int i = threadIdx.x; i < 2 * 4 * nseg; i += blockDim.x) sc[i] = coef[i];
     __syncthreads();
     for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < 2 * n; t += (size_t)gridDim.x * blockDim.x) {
-        const float2 s = IN::one(iq, t >> 1);
+        float2 s = IN::one(iq, t >> 1);
+        float inv_nv = inv_nv_;
+        if constexpr (IN::kCsi) equalise(s, InF32::one(gain, t >> 1), inv_nv);
         const int ax = (int)(t & 1);                    // 0: first half of the label, 1: second half
         const float x = (ax ^ first_is_q) ? s.y : s.x;
         const float x0 = ax ? x0b : x0a, invd = ax ? invdb : invda;
@@ -491,12 +530,13 @@ int launch_hard(const Modem &m, size_t n, const void *iq, int in_f64, uint8_t *b
 }
 
 template <class IN>
-static int launch_demap_t(const Modem &m, size_t n, const void *iq_, float noise_var, float scale, float *llr,
-                          cudaStream_t s)
+static int launch_demap_t(const Modem &m, size_t n, const void *iq_, const float2 *gain, float noise_var, float scale,
+                          float *llr, cudaStream_t s)
 {
     if (n == 0) return B200DVB_OK;
     const typename IN::sym_t *iq = (const typename IN::sym_t *)iq_;
-    if ((reinterpret_cast<uintptr_t>(iq_) & 15) || (reinterpret_cast<uintptr_t>(llr) & 15))
+    if ((reinterpret_cast<uintptr_t>(iq_) & 15) || (reinterpret_cast<uintptr_t>(gain) & 15) ||
+        (reinterpret_cast<uintptr_t>(llr) & 15))
         return B200DVB_EINVAL;                               // vector loads/stores need 16-byte alignment
     const float nv = noise_var > 0.005f ? noise_var : 0.005f;      // test_sdr_with_coding.py:202
     const float inv_nv = 1.0f / nv;
@@ -504,7 +544,7 @@ static int launch_demap_t(const Modem &m, size_t n, const void *iq_, float noise
         const float2 *coef = (const float2 *)m.d_pwl;
         const int fq = (m.separable == 2);
 #define PWL(H, S) demap_pwl<H, S, IN><<<grid_for(n, kThreads * S, 8), kThreads, 0, s>>>(                \
-        n, iq, coef, m.nseg, m.pwl_x0[0], m.pwl_invd[0], m.pwl_x0[1], m.pwl_invd[1], fq, inv_nv, scale, llr)
+        n, iq, coef, m.nseg, m.pwl_x0[0], m.pwl_invd[0], m.pwl_x0[1], m.pwl_invd[1], fq, inv_nv, scale, llr, gain)
         switch (m.half) {
         case 1: PWL(1, 2); break;
         case 2: PWL(2, 1); break;
@@ -512,14 +552,14 @@ static int launch_demap_t(const Modem &m, size_t n, const void *iq_, float noise
         case 4:
             demap_pwl_axis4<IN><<<grid_for(2 * n, kThreads, 8), kThreads, 0, s>>>(
                 n, iq, coef, m.nseg, m.pwl_x0[0], m.pwl_invd[0], m.pwl_x0[1], m.pwl_invd[1], fq, inv_nv, scale,
-                reinterpret_cast<float4 *>(llr));
+                reinterpret_cast<float4 *>(llr), gain);
             break;
         default: return B200DVB_ENOSPEC;
         }
 #undef PWL
     } else {
         switch (m.bps) {
-#define GEN(B, S) demap_generic<B, S, IN><<<grid_for(n, kThreads * S, 8), kThreads, 0, s>>>(n, iq, m.d_table32, inv_nv, scale, llr)
+#define GEN(B, S) demap_generic<B, S, IN><<<grid_for(n, kThreads * S, 8), kThreads, 0, s>>>(n, iq, m.d_table32, inv_nv, scale, llr, gain)
         case 1: GEN(1, 4); break;
         case 2: GEN(2, 2); break;
         case 3: GEN(3, 4); break;
@@ -536,11 +576,16 @@ static int launch_demap_t(const Modem &m, size_t n, const void *iq_, float noise
 
 int launch_demap(const Modem &m, size_t n, const void *iq, float noise_var, float scale, float *llr, cudaStream_t s)
 {
-    return launch_demap_t<InF32>(m, n, iq, noise_var, scale, llr, s);
+    return launch_demap_t<InF32>(m, n, iq, nullptr, noise_var, scale, llr, s);
 }
 int launch_demap_bf16(const Modem &m, size_t n, const void *iq, float noise_var, float scale, float *llr, cudaStream_t s)
 {
-    return launch_demap_t<InBf16>(m, n, iq, noise_var, scale, llr, s);
+    return launch_demap_t<InBf16>(m, n, iq, nullptr, noise_var, scale, llr, s);
+}
+int launch_demap_csi(const Modem &m, size_t n, const void *iq, const void *gain, float noise_var, float scale,
+                     float *llr, cudaStream_t s)
+{
+    return launch_demap_t<InCsi>(m, n, iq, (const float2 *)gain, noise_var, scale, llr, s);
 }
 
 }  // namespace b200dvb

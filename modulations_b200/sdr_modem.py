@@ -95,18 +95,29 @@ class ModemHandle:
         _lib.check(rc, "hard_demod")
         return out if is_torch else out.cpu().numpy()
 
-    def llr(self, symbols, noise_var, scale=1.0):
-        """float32 max-log LLRs [n*bps], clipped to +-30 then multiplied by `scale`."""
+    def llr(self, symbols, noise_var, scale=1.0, gain=None):
+        """float32 max-log LLRs [n*bps], clipped to +-30 then multiplied by `scale`.  With `gain` (complex64, numpy
+        or CUDA, one per symbol) the symbols were received as h*c + noise and the LLRs are over |y - h c|^2
+        (b200dvb_demap_csi, perfect channel state)."""
         torch = _lib.require_cuda()
         is_torch = isinstance(symbols, torch.Tensor)
         s = _lib.to_device(symbols if is_torch else np.asarray(symbols).astype(np.complex64),
                            torch.complex64, self.device).reshape(-1)
         n = s.numel()
+        if gain is not None:
+            g = _lib.to_device(gain if isinstance(gain, torch.Tensor) else np.asarray(gain).astype(np.complex64),
+                               torch.complex64, self.device).reshape(-1)
+            if g.numel() != n:
+                raise ValueError(f"gain has {g.numel()} elements for {n} symbols")
         out = torch.empty(n * self.bps, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            rc = _lib.load().b200dvb_demap(self.h, n, _lib.ptr(s), float(noise_var), float(scale),
-                                           _lib.ptr(out), _lib.stream_ptr(self.device))
-        _lib.check(rc, "demap")
+            if gain is None:
+                rc = _lib.load().b200dvb_demap(self.h, n, _lib.ptr(s), float(noise_var), float(scale),
+                                               _lib.ptr(out), _lib.stream_ptr(self.device))
+            else:
+                rc = _lib.load().b200dvb_demap_csi(self.h, n, _lib.ptr(s), _lib.ptr(g), float(noise_var),
+                                                   float(scale), _lib.ptr(out), _lib.stream_ptr(self.device))
+        _lib.check(rc, "demap" if gain is None else "demap_csi")
         return out if is_torch else out.cpu().numpy()
 
 

@@ -14,22 +14,23 @@ from . import _lib
 from .sdr_modem import gray_modem, ModemHandle
 
 
-def compute_llr(syms, mod_type, noise_var, constellation=None):
-    """-> float64[n*bps] (numpy in) or float32 CUDA tensor (torch in)."""
+def compute_llr(syms, mod_type, noise_var, constellation=None, gain=None):
+    """-> float64[n*bps] (numpy in) or float32 CUDA tensor (torch in).  `gain`: the complex channel gain of each
+    symbol (received as h*c + noise); the LLRs are then over |y - h c|^2 (``b200dvb_demap_csi``)."""
     if mod_type not in _lib.MOD_IDS:
         raise KeyError(mod_type)                         # reference: MODULATIONS[mod_type] KeyError
     modem = gray_modem(mod_type) if constellation is None else ModemHandle(mod_type, constellation)
     torch = _lib.torch_mod()
-    out = modem.llr(syms, noise_var)
+    out = modem.llr(syms, noise_var, gain=gain)
     if isinstance(out, torch.Tensor):
         return out
     return out.astype(np.float64)
 
 
-def decoder_llr(syms, mod_type, noise_var):
+def decoder_llr(syms, mod_type, noise_var, gain=None):
     """LLRs in the DECODER's convention (positive = bit 0): -compute_llr, fused in
     the kernel as scale = -1 (SURVEY §0 F4)."""
-    return gray_modem(mod_type).llr(syms, noise_var, scale=-1.0)
+    return gray_modem(mod_type).llr(syms, noise_var, scale=-1.0, gain=gain)
 
 
 def estimate_noise_var(rx_symbols, mod_type, floor=0.02, default=0.05, modem=None):

@@ -2,6 +2,7 @@
 """BER / FER sweep on the GPU path (BASELINE config 5 shape), one or more GPUs:
 
     python tools/ber_sweep.py [--N 212] [--rate 1/3] [--mod BPSK] [--ebn0 0 0.5 1 1.5 2] [--frames 1000000]
+                              [--channel awgn|rayleigh] [--coherence L]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/ber_sweep.py ...
 
 Two runs are reported (SURVEY 8d): the PARITY run with the reference's committed interleaver table
@@ -31,6 +32,9 @@ def main():
     ap.add_argument("--batch", type=int, default=1 << 17)
     ap.add_argument("--modes", nargs="+", default=["double-pass"], choices=["double-pass", "nii", "nii16"],
                     help="decoder modes for the bijective-interleaver runs (non-parity modes are labelled as such)")
+    ap.add_argument("--channel", default="awgn", choices=["awgn", "rayleigh"],
+                    help="rayleigh: block fading with perfect channel state at the demapper")
+    ap.add_argument("--coherence", type=int, default=1, help="rayleigh: symbols per fading block (1 = fast fading)")
     args = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -42,7 +46,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", torch.cuda.current_device()))
     cfg = mc.SweepConfig(N=args.N, rate=args.rate, iterations=args.iters, ebn0_db=args.ebn0,
                          frames_per_point=args.frames, batch=args.batch, modulation=args.mod,
-                         min_frame_errors=args.mfe)
+                         min_frame_errors=args.mfe, channel=args.channel, coherence=args.coherence)
     out = {}
     runs = [("parity (committed interleaver table)", None, "double-pass")]
     for mode in args.modes:
