@@ -26,8 +26,7 @@ namespace b200dvb {
 
 namespace {
 
-constexpr int kMfThreads = 256;
-constexpr int kMfTile = 512;        // outputs per block: two per thread (the constant reads and the loop are shared)
+constexpr int kMfThreads = 256;     // one or two outputs per thread (two share the constant reads and the loop)
 
 // Taps travel as a kernel argument: the parameter space is a constant bank, so a tap (and, for the matched filter,
 // the staged offset of the sample it multiplies) is a uniform constant-cache read, not a shared-memory wavefront.
@@ -57,16 +56,18 @@ pulse_shape_kernel(size_t n_sym, const float2 *__restrict__ sym, const __grid_co
 
 // Compile-time sps: a thread owns ALL sps output samples of one symbol period q — the Q = ceil(ntaps/sps) symbols
 // they depend on are loaded once (coalesced: consecutive threads, consecutive symbols) and the sps*Q complex MACs run
-// out of registers; the thread's sps samples are 8*sps contiguous bytes, stored 16 B at a time.  T.h is zero beyond ntaps.
+// out of registers; the thread's sps samples are 8*sps contiguous bytes, stored 16 B at a time.  Only taps below ntaps
+// take part: an FMA with a zero-padded tap would turn an Inf or NaN symbol into a NaN in outputs whose window (the real
+// taps) does not contain it.
 template <int SPS, int QT>
 __global__ void __launch_bounds__(256)
 pulse_shape_sps_kernel(size_t n_sym, const float2 *__restrict__ sym, const __grid_constant__ FirTaps T, int ntaps,
                        size_t n_out, float2 *__restrict__ out)
 {
-    // QT = compile-time bound of the symbols an output period depends on (ceil(ntaps / SPS) <= QT; T.h is zero beyond
-    // ntaps).  Interior periods (every one of the QT symbols exists) take a path without per-load bounds checks and
-    // 64-bit compares: the round-1 kernel spent 75 % of its issue slots on the ALU pipe doing exactly those
-    // (profiles/r02_waveform_ncu.txt) and was ALU-bound, not HBM-bound.
+    // QT = compile-time bound of the symbols an output period depends on (ceil(ntaps / SPS) <= QT).  Interior periods
+    // (every one of the QT symbols exists) take a path without per-load bounds checks and 64-bit compares: the round-1
+    // kernel spent 75 % of its issue slots on the ALU pipe doing exactly those (profiles/r02_waveform_ncu.txt) and was
+    // ALU-bound, not HBM-bound.
     const size_t nq = (n_out + SPS - 1) / SPS;                      // symbol periods that hold output samples
     for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += (size_t)gridDim.x * blockDim.x) {
         float2 s[QT];
@@ -84,11 +85,21 @@ pulse_shape_sps_kernel(size_t n_sym, const float2 *__restrict__ sym, const __gri
         for (int p = 0; p < SPS; ++p) acc[p] = make_float2(0.f, 0.f);
 #pragma unroll
         for (int j = 0; j < QT; ++j) {
+            const int real = ntaps - j * SPS;                       // taps j*SPS + p with p < real exist (uniform)
+            if (real >= SPS) {
 #pragma unroll
-            for (int p = 0; p < SPS; ++p) {
-                const float hh = T.h[j * SPS + p];
-                acc[p].x = fmaf(s[j].x, hh, acc[p].x);
-                acc[p].y = fmaf(s[j].y, hh, acc[p].y);
+                for (int p = 0; p < SPS; ++p) {
+                    acc[p].x = fmaf(s[j].x, T.h[j * SPS + p], acc[p].x);
+                    acc[p].y = fmaf(s[j].y, T.h[j * SPS + p], acc[p].y);
+                }
+            } else if (real > 0) {
+#pragma unroll
+                for (int p = 0; p < SPS; ++p) {
+                    if (p < real) {
+                        acc[p].x = fmaf(s[j].x, T.h[j * SPS + p], acc[p].x);
+                        acc[p].y = fmaf(s[j].y, T.h[j * SPS + p], acc[p].y);
+                    }
+                }
             }
         }
         float2 *o = out + q * SPS;
@@ -117,16 +128,20 @@ pulse_shape_sps_kernel(size_t n_sym, const float2 *__restrict__ sym, const __gri
 // consecutive 8-byte words.  The staged index of the sample that tap t multiplies for the tile's first output is
 // r0 - t with r0 = ntaps - 1 + ((start - ntaps + 1) mod sps) — the same for every tile — so its offset T.off[t] is a
 // per-launch constant the host tabulates.
+// NOUT outputs per thread: 2 (a 512-output tile) unless the tile's staging exceeds the shared memory a block may take
+// (sps >= 50, or sps 49 with more than 343 taps); then 1 (a 256-output tile, half the staging).
+template <int NOUT>
 __global__ void __launch_bounds__(kMfThreads, 4)
 matched_filter_kernel(size_t n, const float2 *__restrict__ x, const __grid_constant__ FirTaps T, int ntaps,
                       int sps, long long start, size_t n_out, float2 *__restrict__ out, int pitch, int r0)
 {
+    constexpr int kTile = NOUT * kMfThreads;
     extern __shared__ float2 xs[];                                  // [sps][pitch], phase-major
     const bool even = (kMfThreads % sps) == 0;                      // then a thread's phase never changes while staging
     const bool fast = even && (sps % 2) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0;
-    for (size_t m0 = (size_t)blockIdx.x * kMfTile; m0 < n_out; m0 += (size_t)gridDim.x * kMfTile) {
+    for (size_t m0 = (size_t)blockIdx.x * kTile; m0 < n_out; m0 += (size_t)gridDim.x * kTile) {
         const long long base = start + (long long)m0 * sps - r0;    // staged index 0 <-> sample `base` (a multiple of sps)
-        const int span = (kMfTile - 1) * sps + r0 + 1;
+        const int span = (kTile - 1) * sps + r0 + 1;
         __syncthreads();                                            // previous tile fully consumed
         if (fast && base >= 0 && (size_t)(base + span + 1) <= n) {
             // interior tile, even sps, 16-byte aligned input: 16-byte loads (two samples: phases ph, ph + 1 of the same
@@ -170,18 +185,21 @@ matched_filter_kernel(size_t n, const float2 *__restrict__ x, const __grid_const
             }
         }
         __syncthreads();
-        const float2 *xt = xs + threadIdx.x;                        // outputs m0 + tid and m0 + tid + 256
+        const float2 *xt = xs + threadIdx.x;                        // outputs m0 + tid (and m0 + tid + 256)
         float ar = 0.f, ai = 0.f, br = 0.f, bi = 0.f;
         for (int t = 0; t < ntaps; ++t) {
             const int o = T.off[t];
             const float hh = T.h[t];
-            const float2 v0 = xt[o], v1 = xt[o + kMfThreads];
+            const float2 v0 = xt[o];
             ar = fmaf(v0.x, hh, ar); ai = fmaf(v0.y, hh, ai);
-            br = fmaf(v1.x, hh, br); bi = fmaf(v1.y, hh, bi);
+            if (NOUT == 2) {
+                const float2 v1 = xt[o + kMfThreads];
+                br = fmaf(v1.x, hh, br); bi = fmaf(v1.y, hh, bi);
+            }
         }
         const size_t m = m0 + threadIdx.x;
         if (m < n_out) out[m] = make_float2(ar, ai);
-        if (m + kMfThreads < n_out) out[m + kMfThreads] = make_float2(br, bi);
+        if (NOUT == 2 && m + kMfThreads < n_out) out[m + kMfThreads] = make_float2(br, bi);
     }
 }
 
@@ -200,16 +218,32 @@ matched_filter_kernel(size_t n, const float2 *__restrict__ x, const __grid_const
 //  * Staging is asynchronous (cp.async, 16 bytes) into the other of two buffers while the current tile is computed:
 //    the load-then-compute phases of a block no longer alternate, HBM requests stay in flight all the time.
 // The host tabulates, per pair row, the first staged position its taps touch and both phases' taps in position order
-// (zero padded to QW).  Even sps only; odd sps takes matched_filter_kernel.
+// (zero padded to QW, with a mask of the real ones).  Even sps only; odd sps takes matched_filter_kernel.
 constexpr int kMf4Threads = 128;
 constexpr int kMf4Tile = 4 * kMf4Threads;
 constexpr int kMf4MaxPairs = 16;    // sps <= 32
 constexpr int kMf4MaxQ = 9;
 struct FirRows {
     float h[kMf4MaxPairs][2][kMf4MaxQ + 1];   // [pair row][phase in pair][position within the pair row's window]
+    unsigned real[kMf4MaxPairs][2];           // bit q set: h[..][..][q] is a tap, not padding
     int base[kMf4MaxPairs];
 };
 __device__ __forceinline__ int mf4_idx(int pos, int q4) { return (pos & 3) * q4 + (pos >> 2); }
+
+// acc[j] += (x_j, y_j) * h for the four outputs when `real`: predicated FMAs.  Written as a C++ branch, ptxas made
+// it one (with the tap's constant load moved inside it), which cost the matched filter 5 % of its bandwidth.
+__device__ __forceinline__ void fma4_if(unsigned real, float2 (&acc)[4], float x0, float y0, float x1, float y1,
+                                        float x2, float y2, float x3, float y3, float h)
+{
+    asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %17, 0;\n\t"
+        "@p fma.rn.f32 %0, %8, %16, %0;\n\t@p fma.rn.f32 %1, %9, %16, %1;\n\t"
+        "@p fma.rn.f32 %2, %10, %16, %2;\n\t@p fma.rn.f32 %3, %11, %16, %3;\n\t"
+        "@p fma.rn.f32 %4, %12, %16, %4;\n\t@p fma.rn.f32 %5, %13, %16, %5;\n\t"
+        "@p fma.rn.f32 %6, %14, %16, %6;\n\t@p fma.rn.f32 %7, %15, %16, %7;\n\t}"
+        : "+f"(acc[0].x), "+f"(acc[0].y), "+f"(acc[1].x), "+f"(acc[1].y),
+          "+f"(acc[2].x), "+f"(acc[2].y), "+f"(acc[3].x), "+f"(acc[3].y)
+        : "f"(x0), "f"(y0), "f"(x1), "f"(y1), "f"(x2), "f"(y2), "f"(x3), "f"(y3), "f"(h), "r"(real));
+}
 
 template <int QW, bool ASYNC>
 __global__ void __launch_bounds__(kMf4Threads, ASYNC ? 3 : 6)
@@ -291,20 +325,18 @@ matched_filter4_kernel(size_t n, const float2 *__restrict__ x, const __grid_cons
         const float4 *xt = buf + threadIdx.x;
         for (int pp = 0; pp < npair; ++pp) {
             const int b = T.base[pp];
+            const unsigned ra = T.real[pp][0], rb = T.real[pp][1];
             const float4 *row = xt + pp * pitch;
             float4 w[QW + 3];
 #pragma unroll
             for (int e = 0; e < QW + 3; ++e) w[e] = row[mf4_idx(b + e, q4)];
+            // padded taps take no part: 0 x (an Inf or NaN sample outside this output's window) would be NaN
 #pragma unroll
             for (int q = 0; q < QW; ++q) {
-                const float ha = T.h[pp][0][q], hb = T.h[pp][1][q];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    acc[j].x = fmaf(w[q + j].x, ha, acc[j].x);
-                    acc[j].y = fmaf(w[q + j].y, ha, acc[j].y);
-                    acc[j].x = fmaf(w[q + j].z, hb, acc[j].x);
-                    acc[j].y = fmaf(w[q + j].w, hb, acc[j].y);
-                }
+                fma4_if(ra & (1u << q), acc, w[q].x, w[q].y, w[q + 1].x, w[q + 1].y, w[q + 2].x, w[q + 2].y,
+                        w[q + 3].x, w[q + 3].y, T.h[pp][0][q]);
+                fma4_if(rb & (1u << q), acc, w[q].z, w[q].w, w[q + 1].z, w[q + 1].w, w[q + 2].z, w[q + 2].w,
+                        w[q + 3].z, w[q + 3].w, T.h[pp][1][q]);
             }
         }
         const size_t m = m0 + 4 * (size_t)threadIdx.x;
@@ -396,7 +428,11 @@ int launch_matched_filter(size_t n, const void *x, const double *taps_h, int nta
             if (bmax < 0) { bmin = 0; bmax = 0; }                   // a pair row without taps (ntaps < sps)
             R.base[pp] = bmin;
             for (int t = 0; t < ntaps; ++t)
-                if (((r04 - t) % sps) >> 1 == pp) R.h[pp][(r04 - t) % sps & 1][(r04 - t) / sps - bmin] = (float)taps_h[t];
+                if (((r04 - t) % sps) >> 1 == pp) {
+                    const int ph = (r04 - t) % sps & 1, q = (r04 - t) / sps - bmin;
+                    R.h[pp][ph][q] = (float)taps_h[t];
+                    R.real[pp][ph] |= 1u << q;
+                }
             if (bmin > omax) omax = bmin;
             if (bmax - bmin + 1 > qw) qw = bmax - bmin + 1;
         }
@@ -440,20 +476,28 @@ int launch_matched_filter(size_t n, const void *x, const double *taps_h, int nta
     }
     FirTaps T;
     if (int rc = fill_taps(T, taps_h, ntaps)) return rc;
-    // staged positions per phase: 256 outputs + the taps' reach + the rounding of the origin; odd pitch (in 8-byte
-    // words) spreads the sps rows of the staging pass over the banks
-    const int pitch = (kMfTile + (ntaps + sps - 1) / sps + 2) | 1;
+    // staged positions per phase: the tile's outputs + the taps' reach + the rounding of the origin; odd pitch (in
+    // 8-byte words) spreads the sps rows of the staging pass over the banks.  A 512-output tile fits for every
+    // sps <= 48; above that the 256-output tile keeps every (sps <= 64, ntaps <= 448) within 136 KB.
+    auto pitch_for = [&](int tile) { return (tile + (ntaps + sps - 1) / sps + 2) | 1; };
+    const int nout = (size_t)sps * pitch_for(2 * kMfThreads) * sizeof(float2) <= 200 * 1024 ? 2 : 1;
+    const int tile = nout * kMfThreads, pitch = pitch_for(tile);
     const long long lo = start - (ntaps - 1);                       // first sample of the first output
     const int r0 = ntaps - 1 + (int)(((lo % sps) + sps) % sps);     // its staged index with the origin on a multiple of sps
     for (int t = 0; t < ntaps; ++t) T.off[t] = ((r0 - t) % sps) * pitch + (r0 - t) / sps;
     const size_t smem = (size_t)sps * pitch * sizeof(float2);
-    if (smem > 200 * 1024) return B200DVB_EINVAL;
-    if (smem > 48 * 1024)
-        B2_CUDA(cudaFuncSetAttribute(matched_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    size_t blocks = (n_out + kMfTile - 1) / kMfTile;
+    size_t blocks = (n_out + tile - 1) / tile;
     if (blocks > (size_t)sms * 8) blocks = (size_t)sms * 8;
-    matched_filter_kernel<<<(unsigned)blocks, kMfThreads, smem, s>>>(
-        n, reinterpret_cast<const float2 *>(x), T, ntaps, sps, start, n_out, reinterpret_cast<float2 *>(out), pitch, r0);
+    const float2 *xi = reinterpret_cast<const float2 *>(x);
+    float2 *oo = reinterpret_cast<float2 *>(out);
+#define B2_MFK(K)                                                                                                      \
+    do {                                                                                                               \
+        if (smem > 48 * 1024)                                                                                          \
+            B2_CUDA(cudaFuncSetAttribute(matched_filter_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        matched_filter_kernel<K><<<(unsigned)blocks, kMfThreads, smem, s>>>(n, xi, T, ntaps, sps, start, n_out, oo, pitch, r0); \
+    } while (0)
+    if (nout == 2) B2_MFK(2); else B2_MFK(1);
+#undef B2_MFK
     B2_CUDA(cudaGetLastError());
     return B200DVB_OK;
 }
